@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
                     [--workload cfg4|cfg2|cfg3|cfg5|cfg1] [--math fp32|f16|bf16] [--batch B] [--no-secondary]
+                    [--dump-outputs DIR]
 
 One "step" is one pass of the hot path over one batch of synthetic input.  The DEFAULT workload, at every N, is
 BASELINE.json configs[3] -- the configuration the headline metric is quoted on:
@@ -35,6 +36,12 @@ Metric: pairs/s (image-caption pairs) for the DAMSM step, pixels/s for the atten
           which does not exist on the GPU box) on the host cores, on a bounded sample of the same workload;
 `torch_eager_gpu`: the same op-by-op port on cuda:0 (PyTorch ATen/cuBLAS eager), the second baseline of SURVEY 8d.
 Prints ONE JSON line on rank 0.
+
+`--dump-outputs DIR` writes what the last timed step of `value` handed back to its caller (losses, attention maps,
+gradients w.r.t. every input; for cfg4step the loss and the updated parameters), rank 0's shard, as DIR/<name>.npy
+in float32 (float64 stays float64).  The inputs are seeded, so two builds run with the same arguments can be compared
+array for array.  The files total at most 60 MiB: an output above its share of that is written as a fixed, seeded
+sample of its flattened elements (the same positions on every run with the same arguments).
 """
 from __future__ import annotations
 
@@ -52,6 +59,7 @@ sys.path.insert(0, ROOT)
 
 R_, T_, D_ = 289, 18, 256
 L2_FLUSH_BYTES = 256 << 20
+DUMP_BYTES = 60 << 20                   # --dump-outputs: under 64 MB with the .npy headers
 CFG_BATCH = {"cfg2": 48, "cfg4": 2048}
 METRIC_DAMSM = "damsm_words_sentence_loss_fwd_bwd_pairs_per_sec"
 METRIC_ATTN = "word_attention_fwd_bwd_pixels_per_sec"
@@ -212,6 +220,27 @@ def time_host(step, steps, warmup, sync=None):
     return (time.perf_counter() - t0) / steps
 
 
+def host_outputs(outputs):
+    """name -> device tensor  =>  name -> float32 / float64 numpy array, DUMP_BYTES in all.  Smallest first, each
+    output gets an equal share of what the smaller ones left; one above its share keeps a sorted sample of its
+    flattened elements drawn from a fixed seed"""
+    import torch
+    def elem_bytes(t):
+        return 8 if t.dtype == torch.float64 else 4
+    left, host = DUMP_BYTES, {}
+    order = sorted(outputs, key=lambda k: outputs[k].numel() * elem_bytes(outputs[k]))
+    for i, name in enumerate(order):
+        t = outputs[name].detach()
+        dt = torch.float64 if t.dtype == torch.float64 else torch.float32
+        keep = left // (len(order) - i) // elem_bytes(t)
+        if t.numel() > keep:
+            idx = torch.randint(t.numel(), (keep,), generator=torch.Generator().manual_seed(0)).unique()
+            t = t.reshape(-1)[idx.to(t.device)]
+        host[name] = t.to(dt).cpu().numpy()
+        left -= host[name].nbytes
+    return {k: host[k] for k in outputs}
+
+
 def run_reference(args):
     """reference arm: the reference's CPU implementation of the path (oracle port) on the host cores, rank 0 only"""
     import torch
@@ -312,8 +341,11 @@ class Env:
         self.lib.agb_prof_read(tag, ctypes.byref(ms), ctypes.byref(n))
         return ms.value, n.value
 
-    def measure(self, make_dev, step_dev, step_e2e, tags, steps, warmup, sample_clocks=False, e2e_pipe=None):
-        """the four timings of one workload + the per-kernel profile; all ranks call this together"""
+    def measure(self, make_dev, step_dev, step_e2e, tags, steps, warmup, sample_clocks=False, e2e_pipe=None,
+                keep_outputs=False):
+        """the four timings of one workload + the per-kernel profile; all ranks call this together.
+        step_dev returns its outputs as {name: tensor}; keep_outputs: host copies of those of the last timed step of
+        `value` under out["outputs"]"""
         lib = self.lib
         ts = make_dev()
         for _ in range(warmup):
@@ -337,13 +369,24 @@ class Env:
         if g is None and sampler:
             sampler.start()                       # no graph (torchrun / --no-graph): the eager timing IS the value
         step_dev(ts)                              # untimed: re-grows the allocator pool emptied above (cudaMalloc of the workspace)
-        out["eager"] = self.timed(lambda: step_dev(ts), steps)
+        run_eager, last = (lambda: step_dev(ts)), {}
+        if keep_outputs and g is None:            # the eager timing is `value`: hold on to its last step's outputs only
+            done = [0]
+
+            def run_eager():
+                outs = step_dev(ts)
+                done[0] += 1
+                if done[0] == steps:
+                    last["outputs"] = outs
+        out["eager"] = self.timed(run_eager, steps)
         if g is not None:
             if sampler:
                 sampler.start()
             out["value"] = self.timed(g.replay, steps)
         else:
             out["value"] = out["eager"]
+        if keep_outputs:                          # a graph's static outputs hold what its last replay wrote
+            out["outputs"] = host_outputs(g.outputs if g is not None else last.pop("outputs"))
         out["clocks"] = sampler.stop() if sampler else None
         out["graph"] = g is not None
         del g
@@ -381,7 +424,7 @@ class Env:
         return out
 
 
-def damsm_workload(env: Env, wl, Bg, math, steps, warmup, sample_clocks):
+def damsm_workload(env: Env, wl, Bg, math, steps, warmup, sample_clocks, keep_outputs=False):
     torch, pkg, dev, world, rank = env.torch, env.pkg, env.dev, env.world, env.rank
     assert Bg % world == 0
     Bl = Bg // world
@@ -408,9 +451,10 @@ def damsm_workload(env: Env, wl, Bg, math, steps, warmup, sample_clocks):
         im, wd, cn, rn, ln, cl = ts
         for t in (im, wd, cn, rn):
             t.grad = None
-        wl_, sl_, _ = loss_mod.get_losses(im, cn, wd.transpose(1, 2), rn, labels, ln, cl)
+        wl_, sl_, maps = loss_mod.get_losses(im, cn, wd.transpose(1, 2), rn, labels, ln, cl)
         (wl_ + sl_).backward()
-        return wl_, sl_
+        return {"words_loss": wl_, "sentence_loss": sl_, "att_maps": maps, "d_img_features": im.grad,
+                "d_words_emb": wd.grad, "d_cnn_code": cn.grad, "d_rnn_code": rn.grad}
 
     def step_e2e():
         im = img_h.to(dev, non_blocking=True).requires_grad_(True)
@@ -437,14 +481,14 @@ def damsm_workload(env: Env, wl, Bg, math, steps, warmup, sample_clocks):
     tc = math != "fp32"
     tags = list(DAMSM_KERNELS) if tc else [1]
     m = env.measure(make_dev, step_dev, step_e2e, tags, steps, warmup, sample_clocks,
-                    e2e_pipe=([img_h, wrd_h, cnn_h, rnn_h, lens_h, cls_h], run_on))
+                    e2e_pipe=([img_h, wrd_h, cnn_h, rnn_h, lens_h, cls_h], run_on), keep_outputs=keep_outputs)
     m.update(units=Bl * Bg, total_units=Bg * Bg, h2d=int(h2d), d2h=8, mean_len=mean_len, tc=tc,
              flop_unit=2.0 * R_ * mean_len * D_, metric=METRIC_DAMSM, unit="pairs/s",
              dtype={"fp32": "f32", "f16": "f16", "bf16": "bf16", "f16x2": "f16"}[math], math=math)
     return m
 
 
-def pretrain_workload(env: Env, Bg, math, steps, warmup, sample_clocks):
+def pretrain_workload(env: Env, Bg, math, steps, warmup, sample_clocks, keep_outputs=False):
     """the whole DAMSM pretraining step (SURVEY 8 f4) on synthetic bedroom captions + synthetic Inception features"""
     torch, dev, world, rank = env.torch, env.dev, env.world, env.rank
     from attention_gan_b200.pretrain import DamsmPretrainStep, SyntheticBedroomCaptions
@@ -463,11 +507,13 @@ def pretrain_workload(env: Env, Bg, math, steps, warmup, sample_clocks):
     out_h = torch.empty(1, dtype=torch.float32).pin_memory()
     h2d = sum(t.numel() * t.element_size() for t in (caps_h, lens_h, cls_h, m6e_h, pool_h))
 
+    params = {f"{k}.{n}": p for k, mod in st.modules().items() for n, p in mod.named_parameters() if p.requires_grad}
+
     def make_dev():
         return [caps_h.to(dev), lens_h.to(dev), cls_h.to(dev), m6e_h.to(dev), pool_h.to(dev)]
 
     def step_dev(ts):
-        return st.step(ts[0], ts[1], ts[2], ts[3], ts[4], labels)
+        return {"loss": st.step(ts[0], ts[1], ts[2], ts[3], ts[4], labels), **params}   # parameters: updated in place
 
     def step_e2e():
         ts = [t.to(dev, non_blocking=True) for t in (caps_h, lens_h, cls_h, m6e_h, pool_h)]
@@ -480,14 +526,14 @@ def pretrain_workload(env: Env, Bg, math, steps, warmup, sample_clocks):
 
     tc = math != "fp32"
     m = env.measure(make_dev, step_dev, step_e2e, list(DAMSM_KERNELS) if tc else [1], steps, warmup, sample_clocks,
-                    e2e_pipe=([caps_h, lens_h, cls_h, m6e_h, pool_h], run_on))
+                    e2e_pipe=([caps_h, lens_h, cls_h, m6e_h, pool_h], run_on), keep_outputs=keep_outputs)
     m.update(units=Bl * Bg, total_units=Bg * Bg, h2d=int(h2d), d2h=4, mean_len=7.0, tc=tc,
              flop_unit=2.0 * R_ * 7.0 * D_, metric="damsm_pretrain_step_pairs_per_sec", unit="pairs/s",
              dtype={"fp32": "f32", "f16": "f16", "bf16": "bf16", "f16x2": "f16"}[math], math=math)
     return m
 
 
-def attn_workload(env: Env, wl, batch, hw_only, steps, warmup, sample_clocks, local_share=False):
+def attn_workload(env: Env, wl, batch, hw_only, steps, warmup, sample_clocks, local_share=False, keep_outputs=False):
     torch, pkg, dev, world, rank = env.torch, env.pkg, env.dev, env.world, env.rank
     from oracle import ref_port as rp          # seeded input generators only (never inside a timed region)
     if wl == "cfg1":
@@ -534,13 +580,15 @@ def attn_workload(env: Env, wl, batch, hw_only, steps, warmup, sample_clocks, lo
     def step_dev(ts):
         ims, wd, dctxs = ts
         wd.grad = None
-        outs = []
-        for mod, im, dctx in zip(mods, ims, dctxs):
+        outs = {}
+        for hw, mod, im, dctx in zip(hws, mods, ims, dctxs):
             im.grad = None
             mod.conv1.weight.grad = None
             ctx, attn = mod(im, wd.transpose(1, 2))
             ctx.backward(dctx)
-            outs.append((ctx, attn))
+            outs.update({f"ctx_{hw}": ctx, f"attn_{hw}": attn, f"d_images_{hw}": im.grad,
+                         f"d_weight_{hw}": mod.conv1.weight.grad})
+        outs["d_words"] = wd.grad                 # summed over the stages
         return outs
 
     def step_e2e():
@@ -568,7 +616,7 @@ def attn_workload(env: Env, wl, batch, hw_only, steps, warmup, sample_clocks, lo
     npix = sum(hw * hw for hw in hws)
     es = 4 if tdt == torch.float32 else 2
     m = env.measure(make_dev, step_dev, step_e2e, [4, 5], steps, warmup, sample_clocks,
-                    e2e_pipe=([*img_h, *dctx_h, wrd_h], run_on))
+                    e2e_pipe=([*img_h, *dctx_h, wrd_h], run_on), keep_outputs=keep_outputs)
     m.update(units=Bl * npix, total_units=B * npix, h2d=int(h2d), d2h=int(d2h), metric=METRIC_ATTN, unit="pixels/s",
              bytes_fwd=es * (2 * C + T), bytes_bwd=es * 3 * C, dtype="f32" if es == 4 else "bf16",
              io="fp32" if es == 4 else "bf16", B=B, T=T, C=C, hws=hws)
@@ -646,21 +694,27 @@ def run_native(args):
     peaks = load_peaks()
     wl = args.workload
     damsm = wl in ("cfg2", "cfg4", "cfg4step")
+    keep = args.dump_outputs is not None
     if wl == "cfg4step":
         Bg = args.batch or 2048
-        m = pretrain_workload(env, Bg, args.math, args.steps, args.warmup, True)
+        m = pretrain_workload(env, Bg, args.math, args.steps, args.warmup, True, keep_outputs=keep)
         roof = damsm_roofline(m, peaks, long_step=m["value"] > 2e-3)
         name = (f"cfg4step: DAMSM pretraining step (text LSTM + CNN heads + WordsLoss + SentenceLoss + backward + clip + "
                 f"Adam), synthetic 7-token bedroom captions (k=7..500 hierarchy, <=990 words), global batch {Bg}")
     elif damsm:
         Bg = args.batch or CFG_BATCH[wl]
-        m = damsm_workload(env, wl, Bg, args.math, args.steps, args.warmup, True)
+        m = damsm_workload(env, wl, Bg, args.math, args.steps, args.warmup, True, keep_outputs=keep)
         roof = damsm_roofline(m, peaks, long_step=m["value"] > 2e-3)
         name = workload_name(wl, Bg)
     else:
-        m = attn_workload(env, wl, args.batch, args.hw, args.steps, args.warmup, True)
+        m = attn_workload(env, wl, args.batch, args.hw, args.steps, args.warmup, True, keep_outputs=keep)
         roof = attn_roofline(m, peaks)
         name = workload_name(wl)
+    if keep and env.rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for key, a in m.pop("outputs").items():
+            np.save(os.path.join(args.dump_outputs, key + ".npy"), a)
 
     secondary = {}
     if env.world == 1 and args.secondary and not (args.batch or args.hw):
@@ -769,7 +823,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="time eager launches only")
     ap.add_argument("--no-secondary", dest="secondary", action="store_false",
                     help="N=1: skip the cfg2 / cfg3 / cfg5 measurements reported under 'secondary'")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy; 60 MiB in all, an output "
+                         "above its share is written as a fixed, seeded sample of its elements")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "native":
+        ap.error("--dump-outputs writes the native arm's outputs; it needs --impl native")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)

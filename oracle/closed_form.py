@@ -204,3 +204,33 @@ def func_attention_fwd(query, context, gamma1=4.0, scaled=True):
     alpha = _softmax(s, axis=2)
     beta = _softmax(gamma1 * alpha, axis=1)
     return np.einsum("bdr,brt->bdt", c, beta), beta.transpose(0, 2, 1)
+
+
+def text_encoder_fwd(sd, captions, cap_lens):
+    """the reference's RNNEncoder in eval mode (rnn_encoder.py:69-96: embedding -> dropout (identity) -> packed
+    one-layer bidirectional LSTM -> zero-padded outputs), in fp64.  sd: its state dict (numpy arrays), captions
+    [B,T] word indices, cap_lens [B].  Returns words [B,2H,max(cap_lens)], sentence [B,2H] = (last forward state,
+    last backward state).  LSTM cell as torch.nn.LSTM: gates i, f, g, o stacked in the weight rows."""
+    def sig(x):
+        return 1.0 / (1.0 + np.exp(-x))
+
+    emb = np.asarray(sd["embedding.weight"], np.float64)[np.asarray(captions)]          # [B,T,E]
+    lens = [int(n) for n in cap_lens]
+    B, Tm = emb.shape[0], max(lens)
+    H = np.asarray(sd["rnn.weight_hh_l0"]).shape[1]
+    words = np.zeros((B, 2 * H, Tm))
+    sent = np.zeros((B, 2 * H))
+    for d, sfx in enumerate(("", "_reverse")):
+        wi, wh, bi, bh = (np.asarray(sd[f"rnn.{k}_l0{sfx}"], np.float64)
+                          for k in ("weight_ih", "weight_hh", "bias_ih", "bias_hh"))
+        for b in range(B):
+            h, c = np.zeros(H), np.zeros(H)
+            steps = range(lens[b]) if d == 0 else range(lens[b] - 1, -1, -1)
+            for t in steps:
+                z = wi @ emb[b, t] + bi + wh @ h + bh
+                i, f, g, o = sig(z[:H]), sig(z[H:2 * H]), np.tanh(z[2 * H:3 * H]), sig(z[3 * H:])
+                c = f * c + i * g
+                h = o * np.tanh(c)
+                words[b, d * H:(d + 1) * H, t] = h
+            sent[b, d * H:(d + 1) * H] = h
+    return words, sent

@@ -139,8 +139,31 @@ def golden_damsm(rwl, rsl, name, B, T, D, hw, seed, n_classes, full_len=False, t
         gammas=np.array(gammas), lambdas=np.array(lambdas), **out)
 
 
+def golden_text_encoder(name, seed):
+    """the text encoder's fixture.  The reference's RNNEncoder is stated in fp64 by oracle/closed_form.py
+    (text_encoder_fwd) on seeded weights (ref_port.synth_text_encoder); no reference import is needed, so
+    ``python oracle/make_golden.py text_encoder`` writes only this file.  tests/test_pretrain_cpu.py checks the
+    reference itself against it whenever AGB_REFERENCE_ROOT names a checkout."""
+    from attention_gan_b200.pretrain import SyntheticBedroomCaptions
+    from oracle import closed_form
+    d = SyntheticBedroomCaptions(64, seed=1)
+    caps, lens, _ = d.batch(0, 8)
+    ragged = torch.tensor([7, 3, 5, 2, 7, 6, 4, 2])
+    sd = ref_port.synth_text_encoder(d.vocab_size, seed=seed)
+    sd64 = {k: v.numpy() for k, v in sd.items()}
+    out = {}
+    for tag, ln in (("full", lens), ("ragged", ragged)):
+        out[f"words_{tag}"], out[f"sent_{tag}"] = closed_form.text_encoder_fwd(sd64, caps.numpy(), ln.numpy())
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), captions=caps.numpy(), cap_lens=lens.numpy(),
+                        cap_lens_ragged=ragged.numpy(), vocab=np.array(d.vocab_size), seed=np.array(seed),
+                        weight_abs_sums=np.array([float(v.double().abs().sum()) for v in sd.values()]), **out)
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
+    if sys.argv[1:] == ["text_encoder"]:
+        golden_text_encoder("text_encoder", seed=1)
+        return
     ratt, rwl, rsl = load_reference()
     # generator attention (a3/a4)
     golden_attention(ratt, "attn_small_scaled", B=3, C=8, E=16, T=5, hw=6, seed=1, scaled=True)
@@ -158,6 +181,7 @@ def main():
                  trained_like=0.12)
     golden_damsm(rwl, rsl, "damsm_gammas", B=5, T=6, D=64, hw=4, seed=11, n_classes=4,
                  gammas=(2.0, 3.0, 7.0), lambdas=(1.5, 0.5), full_len=True)
+    golden_text_encoder("text_encoder", seed=1)
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))
 

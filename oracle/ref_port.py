@@ -224,3 +224,16 @@ def synth_attention(B: int, C: int = 32, E: int = 256, T: int = 18, hw: int = 64
     lens[0] = T
     mask = (torch.arange(T)[None, :] < lens[:, None]).to(torch.int64)
     return images.to(dtype), words.to(dtype).transpose(1, 2), weight.to(dtype), mask, lens
+
+
+def synth_text_encoder(vocab: int, embdim: int = 300, nhidden: int = 256, seed: int = 0):
+    """seeded state dict of the reference's RNNEncoder (bidirectional, nhidden // 2 per direction): embedding
+    U(-0.1, 0.1) (rnn_encoder.py:48-50), LSTM tensors U(-1/sqrt(h), 1/sqrt(h)) (torch.nn.LSTM's default init)."""
+    g = torch.Generator().manual_seed(seed)
+    h = nhidden // 2
+    sd = {"embedding.weight": (torch.rand(vocab, embdim, generator=g) * 2 - 1) * 0.1}
+    for sfx in ("", "_reverse"):
+        for k, shape in (("weight_ih", (4 * h, embdim)), ("weight_hh", (4 * h, h)), ("bias_ih", (4 * h,)),
+                         ("bias_hh", (4 * h,))):
+            sd[f"rnn.{k}_l0{sfx}"] = (torch.rand(*shape, generator=g) * 2 - 1) / math.sqrt(h)
+    return sd

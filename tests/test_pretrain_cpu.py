@@ -9,8 +9,11 @@ import pytest
 import torch
 
 from attention_gan_b200.pretrain import RegionHeads, SyntheticBedroomCaptions, TextEncoder, hierarchical_k_values
+from conftest import load_golden
+from oracle import ref_port as rp
 
-REF = "/root/reference"
+# a checkout of the original project (as for oracle/make_golden.py); the live comparison with it skips without one
+REF = os.environ.get("AGB_REFERENCE_ROOT", "")
 
 
 def test_k_values_follow_the_reference_recipe():
@@ -65,7 +68,28 @@ def test_encoder_state_dicts_keep_the_reference_names():
     assert f.shape == (2, 256, 17, 17) and c.shape == (2, 256)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "networks")), reason="reference tree only in the build container")
+def test_text_encoder_matches_the_reference_fixture():
+    """TextEncoder == tests/golden/text_encoder.npz: the reference's RNNEncoder stated in fp64 on seeded weights
+    (oracle/closed_form.py text_encoder_fwd, written by oracle/make_golden.py); full-length captions through the
+    packed and the fixed-length path, ragged lengths through the packed path"""
+    g = load_golden("text_encoder")
+    sd = rp.synth_text_encoder(int(g["vocab"]), seed=int(g["seed"]))
+    np.testing.assert_allclose([float(v.double().abs().sum()) for v in sd.values()], g["weight_abs_sums"], rtol=1e-12)
+    mine = TextEncoder(vocabsize=int(g["vocab"]), nhidden=256).eval()
+    assert list(mine.state_dict().keys()) == list(sd.keys())
+    mine.load_state_dict(sd)
+    caps = torch.from_numpy(g["captions"])
+    cases = [("full", g["cap_lens"], False), ("full", g["cap_lens"], True), ("ragged", g["cap_lens_ragged"], False)]
+    with torch.no_grad():
+        for tag, lens, fixed in cases:
+            w, s = mine(caps, torch.from_numpy(lens), fixed_length=fixed)
+            assert w.shape == g[f"words_{tag}"].shape == (8, 256, 7)
+            np.testing.assert_allclose(w.numpy(), g[f"words_{tag}"], rtol=0, atol=1e-6)
+            np.testing.assert_allclose(s.numpy(), g[f"sent_{tag}"], rtol=0, atol=1e-6)
+
+
+@pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "networks")),
+                    reason="needs AGB_REFERENCE_ROOT: a checkout of the original project")
 def test_text_encoder_equals_the_reference_rnn_encoder():
     import subprocess
     code = r'''
@@ -88,8 +112,20 @@ for fixed in (False, True):
 lens2 = torch.tensor([7, 3, 5, 2, 7, 6, 4, 2])
 w0, s0 = ref(caps, lens2); w1, s1 = mine(caps, lens2)
 assert (w1 - w0).abs().max() < 1e-6 and (s1 - s0).abs().max() < 1e-6
+# the reference on the stored fixture's weights and captions reproduces it
+import numpy as np
+from oracle import ref_port as rp
+g = np.load(sys.argv[3])
+ref = RNNEncoder(vocabsize=int(g["vocab"]), nhidden=256).eval()
+ref.load_state_dict(rp.synth_text_encoder(int(g["vocab"]), seed=int(g["seed"])))
+for tag in ("full", "ragged"):
+    lens = g["cap_lens" if tag == "full" else "cap_lens_ragged"]
+    w0, s0 = ref(torch.from_numpy(g["captions"]), torch.from_numpy(lens))
+    assert np.abs(w0.detach().numpy() - g["words_" + tag]).max() < 1e-6
+    assert np.abs(s0.detach().numpy() - g["sent_" + tag]).max() < 1e-6
 print("encoder ok")
 '''
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-c", code, REF, root], capture_output=True, text=True, timeout=300)
+    fixture = os.path.join(root, "tests", "golden", "text_encoder.npz")
+    r = subprocess.run([sys.executable, "-c", code, REF, root, fixture], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "encoder ok" in r.stdout, r.stdout + r.stderr
