@@ -150,6 +150,51 @@ def damsm_bwd(img, words, cap_lens, gamma1, gamma2, eps, dm, gscale, need_dwords
     return dimg, dwords
 
 
+def damsm_cand_workspace_bytes(Bi: int, K: int, T: int, D: int, R: int, math: int) -> int:
+    """workspace of damsm_cand_fwd; 0 when the shapes are outside the candidate path's range"""
+    return int(N.lib().agb_damsm_cand_workspace_bytes(Bi, K, T, D, R, math))
+
+
+def damsm_cand_fwd(img: torch.Tensor, words: torch.Tensor, cap_lens: torch.Tensor, cand: torch.Tensor,
+                   gamma1: float, gamma2: float, math: int, ws: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """m of candidate pairs: img [Bi,D,R] fp32 contiguous, words [Bc,D,T] fp32 (any strides), cap_lens [Bc] int32,
+    cand [Bi,K] int32 contiguous.  Returns m [Bi,K] fp32, m[b,k] = damsm_fwd's m[b, cand[b,k]] bit for bit
+    (NaN where cand[b,k] is outside [0,Bc)).  Tensor-core math only.  ws: a uint8 workspace of at least
+    damsm_cand_workspace_bytes (allocated here when None)."""
+    require_cuda(img, words, cap_lens, cand)
+    Bi, D, R = img.shape
+    Bc, _, T = words.shape
+    K = cand.shape[1]
+    if cand.dtype != torch.int32 or not cand.is_contiguous() or cand.shape[0] != Bi:
+        raise RuntimeError("cand must be a contiguous int32 [Bi,K] tensor")
+    nbytes = damsm_cand_workspace_bytes(Bi, K, T, D, R, math)
+    if nbytes == 0:
+        raise N.NativeError(f"candidate DAMSM shape Bi={Bi} K={K} T={T} D={D} R={R} is unsupported for math mode {math}")
+    if ws is None:
+        ws = _ws(nbytes, img.device)
+    m = torch.empty((Bi, K), dtype=torch.float32, device=img.device)
+    rc = N.lib().agb_damsm_cand_fwd(_p(img), _p(words), words.stride(0), words.stride(1), words.stride(2),
+                                    _p(cap_lens), Bc, _p(cand), Bi, K, T, D, R, gamma1, gamma2, _p(m), _p(ws),
+                                    ws.numel(), math, _stream(img))
+    N.check(rc, "agb_damsm_cand_fwd")
+    return m
+
+
+def sent_cos_cand_fwd(cnn: torch.Tensor, rnn: torch.Tensor, cand: torch.Tensor, eps: float) -> torch.Tensor:
+    """cnn [Bi,D], rnn [Bc,D] fp32 contiguous, cand [Bi,K] int32 contiguous -> cosine [Bi,K] of the candidate
+    pairs (NaN where cand[b,k] is outside [0,Bc))"""
+    require_cuda(cnn, rnn, cand)
+    Bi, D = cnn.shape
+    Bc = rnn.shape[0]
+    if cand.dtype != torch.int32 or not cand.is_contiguous() or cand.shape[0] != Bi:
+        raise RuntimeError("cand must be a contiguous int32 [Bi,K] tensor")
+    K = cand.shape[1]
+    scos = torch.empty((Bi, K), dtype=torch.float32, device=cnn.device)
+    rc = N.lib().agb_sent_cos_cand_fwd(_p(cnn), _p(rnn), Bc, _p(cand), Bi, K, D, eps, _p(scos), _stream(cnn))
+    N.check(rc, "agb_sent_cos_cand_fwd")
+    return scos
+
+
 def contrastive(raw: torch.Tensor, class_ids: Optional[torch.Tensor], labels: torch.Tensor, gamma3: float,
                 lam: float, row_begin: int, row_count: int, want_grad: bool = True):
     """raw [B,B] fp32 (all rows), class_ids [B] int32 or None, labels [B] int64.

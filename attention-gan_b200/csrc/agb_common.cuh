@@ -18,7 +18,7 @@ int check_launch(const char* what);          // cudaGetLastError -> return code;
 
 // optional per-kernel timing for bench.py (agb_prof_enable / agb_prof_read); no-ops when disabled
 enum ProfTag { PROF_SGEMM = 1, PROF_DAMSM_TC_FWD = 2, PROF_DAMSM_TC_BWD = 3, PROF_ATTN_FWD = 4, PROF_ATTN_BWD = 5,
-               PROF_DAMSM_DIMG = 6, PROF_DAMSM_DWORDS = 7, PROF_DAMSM_PACK = 8, PROF_MAX = 16 };
+               PROF_DAMSM_DIMG = 6, PROF_DAMSM_DWORDS = 7, PROF_DAMSM_PACK = 8, PROF_DAMSM_CAND = 9, PROF_MAX = 16 };
 int prof_begin(int tag, cudaStream_t st);
 void prof_end(int slot, cudaStream_t st);
 

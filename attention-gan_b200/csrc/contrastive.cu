@@ -298,9 +298,45 @@ sent_grad_kernel(const float* __restrict__ x, const float* __restrict__ y, int n
   }
 }
 
+// sentence cosine of candidate pairs: one warp per entry v = b*K + k, caption j = cand[v];
+// out[v] = <c_b, r_j> / max(|c_b| |r_j|, eps), NaN when j is outside [0, Bc)
+__global__ void __launch_bounds__(256)
+sent_cos_cand_kernel(const float* __restrict__ cnn, const float* __restrict__ rnn, int Bc,
+                     const int32_t* __restrict__ cand, int K, int n, int D, float eps, float* __restrict__ out) {
+  const int v = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (v >= n) return;
+  const int b = v / K, j = cand[v];
+  if (j < 0 || j >= Bc) {
+    if (lane == 0) out[v] = __int_as_float(0x7fc00000);
+    return;
+  }
+  float num = 0.f, p2 = 0.f, q2 = 0.f;
+  for (int d = lane; d < D; d += 32) {
+    const float c = cnn[(size_t)b * D + d], r = rnn[(size_t)j * D + d];
+    num = fmaf(c, r, num);
+    p2 = fmaf(c, c, p2);
+    q2 = fmaf(r, r, q2);
+  }
+  num = warp_sum(num);
+  p2 = warp_sum(p2);
+  q2 = warp_sum(q2);
+  if (lane == 0) out[v] = num / fmaxf(sqrtf(p2) * sqrtf(q2), eps);
+}
+
 }  // namespace agb
 
 using namespace agb;
+
+extern "C" int agb_sent_cos_cand_fwd(const float* cnn, const float* rnn, int Bc, const int32_t* cand, int Bi, int K,
+                                     int D, float eps, float* scos_out, void* stream) {
+  if (Bi <= 0 || Bc <= 0 || K <= 0 || D <= 0) return fail_arg("non-positive size");
+  if (!cnn || !rnn || !cand || !scos_out) return fail_arg("null pointer");
+  const long long n = (long long)Bi * K;
+  if (n >= 0x7fffffffLL - 8) return fail_unsupported("Bi*K=%lld >= 2^31", n);
+  sent_cos_cand_kernel<<<(unsigned)((n + 7) / 8), 256, 0, (cudaStream_t)stream>>>(cnn, rnn, Bc, cand, K, (int)n, D, eps,
+                                                                               scos_out);
+  return check_launch("sent_cos_cand_kernel");
+}
 
 extern "C" size_t agb_contrastive_workspace_bytes(int B) { return B > 0 ? (size_t)4 * B * sizeof(float) : 0; }
 

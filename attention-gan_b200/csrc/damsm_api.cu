@@ -26,6 +26,10 @@ int damsm_tc_bwd(const float* img, const float* words, int64_t ws_b, int64_t ws_
                  const int32_t* cap_lens, int Bi, int Bc, int T, int D, int R, float gamma1,
                  float gamma2, float eps, const float* dm, const float* m_fwd, const float* gscale, float* dimg,
                  float* dwords, void* workspace, size_t workspace_bytes, int ws_from_fwd, int math, cudaStream_t st);
+size_t damsm_tc_cand_workspace_bytes(int Bi, int K, int T, int math);
+int damsm_tc_cand_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                      const int32_t* cap_lens, int Bc, const int32_t* cand, int Bi, int K, int T, int R, float gamma1,
+                      float gamma2, float* m_out, void* workspace, size_t workspace_bytes, int math, cudaStream_t st);
 #endif
 }  // namespace agb
 
@@ -100,6 +104,35 @@ extern "C" int agb_damsm_bwd(const float* img, const float* words, int64_t ws_b,
 #ifdef AGB_WITH_TC
   return damsm_tc_bwd(img, words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, T, D, R, gamma1, gamma2, eps, dm, m_fwd, gscale,
                       dimg, dwords, workspace, workspace_bytes, ws_from_fwd, math, st);
+#else
+  return fail_unsupported("library built without the tcgen05 kernels");
+#endif
+}
+
+// candidate pairs run only on the tensor-core kernels (no fp32 path, no training forward)
+static bool cand_math_ok(int math) {
+  return math == AGB_MATH_TC_F16 || math == AGB_MATH_TC_BF16 || math == AGB_MATH_TC_F16X2;
+}
+
+extern "C" size_t agb_damsm_cand_workspace_bytes(int Bi, int K, int T, int D, int R, int math) {
+  if (!cand_math_ok(math) || !agb_damsm_supported(T, D, R, math)) return 0;
+#ifdef AGB_WITH_TC
+  return damsm_tc_cand_workspace_bytes(Bi, K, T, math);
+#else
+  return 0;
+#endif
+}
+
+extern "C" int agb_damsm_cand_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                                  const int32_t* cap_lens, int Bc, const int32_t* cand, int Bi, int K, int T, int D,
+                                  int R, float gamma1, float gamma2, float* m_out, void* workspace,
+                                  size_t workspace_bytes, int math, void* stream) {
+  if (!img || !words || !cap_lens || !cand || !m_out || !workspace) return fail_arg("null pointer");
+  if (!cand_math_ok(math)) return fail_unsupported("math=%d: candidate scores need a tensor-core inference mode", math);
+  if (!agb_damsm_supported(T, D, R, math)) return fail_unsupported("T=%d D=%d R=%d math=%d is outside the compiled range", T, D, R, math);
+#ifdef AGB_WITH_TC
+  return damsm_tc_cand_fwd(img, words, ws_b, ws_d, ws_t, cap_lens, Bc, cand, Bi, K, T, R, gamma1, gamma2, m_out,
+                           workspace, workspace_bytes, math, (cudaStream_t)stream);
 #else
   return fail_unsupported("library built without the tcgen05 kernels");
 #endif

@@ -194,6 +194,171 @@ __global__ void pack_img_kernel_tc(const float* __restrict__ img, T16* __restric
 }
 
 // ---------------------------------------------------------------------------------------------
+// candidate packing (agb_damsm_cand_fwd): image b's K candidate captions become the virtual captions
+// v = b*K + k, packed by the rule of tile_pack_kernel into units of U rows (U = 64 in split precision) that
+// never mix two images; every image is padded to whole tiles.  An item of the pair kernels is one unit.
+// A candidate index outside [0, Bc) becomes an entry of length 0, whose m the pair kernel writes as NaN.
+// ---------------------------------------------------------------------------------------------
+// upper bound of one item's cost (kItemCost0 + per live caption its window and kItemCostCap, at most 128 captions
+// and 128 + 3 * 128 window rows): the host bounds the cost prefix of a call with it
+constexpr int kMaxItemCost = kItemCost0 + kTileN * (kItemCostCap + 4);
+
+// One warp per image, in lock-step (lane k % 32 loads entry k).  Pass 1 (!kWrite): the image's item count and
+// cost into img_items / img_cost.  Pass 2 (kWrite, after cand_scan_kernel turned them into exclusive prefixes):
+// cap_row, vlen of every entry, first entry / entry count / cost prefix of every item, image of every tile.
+template <bool kWrite>
+__global__ void __launch_bounds__(256)
+cand_pack_kernel(const int32_t* __restrict__ cap_lens, int Bc, int T, const int32_t* __restrict__ cand, int Bi, int K,
+                 int U, int32_t* __restrict__ img_items, int32_t* __restrict__ img_cost, int32_t* __restrict__ cap_row,
+                 int32_t* __restrict__ vlen, int32_t* __restrict__ item_first, int32_t* __restrict__ item_ncap,
+                 int32_t* __restrict__ cpre, int32_t* __restrict__ tile_img) {
+  const int b = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= Bi) return;
+  const int upt = kTileN / U;
+  const int v0 = b * K;
+  const int item0 = kWrite ? img_items[b] : 0, cost0 = kWrite ? img_cost[b] : 0;
+  int row = 0, unit = 0, first = 0, cost = kItemCost0, cacc = 0;
+  auto close_unit = [&](int next_first) {
+    if (kWrite && lane == 0) {
+      const int it = item0 + unit;
+      item_first[it] = v0 + first;
+      item_ncap[it] = next_first - first;
+      cpre[it] = cost0 + cacc;
+      if (it % upt == 0) tile_img[it / upt] = b;
+    }
+    cacc += cost;
+    cost = kItemCost0;
+    ++unit;
+    first = next_first;
+    row = 0;
+  };
+  for (int k0 = 0; k0 < K; k0 += 32) {
+    int myL = 0;
+    if (k0 + lane < K) {
+      const int j = cand[(size_t)v0 + k0 + lane];
+      myL = (j >= 0 && j < Bc) ? min(max(cap_lens[j], 0), T) : 0;
+    }
+    const int n = min(32, K - k0);
+    for (int i = 0; i < n; ++i) {
+      const int k = k0 + i, L = __shfl_sync(0xffffffffu, myL, i);
+      if (row + ((L + 3) & ~3) > U || k - first == U) close_unit(k);
+      if (kWrite && lane == i) {
+        cap_row[v0 + k] = (item0 + unit) * U + row;
+        vlen[v0 + k] = L;
+      }
+      row += L;
+      if (L > 0) cost += ((L + 3) & ~3) + kItemCostCap;
+    }
+  }
+  close_unit(K);
+  while (unit % upt != 0) close_unit(K);       // pad the image to whole tiles with empty units
+  if (!kWrite && lane == 0) {
+    img_items[b] = unit;
+    img_cost[b] = cacc;
+  }
+}
+
+// exclusive prefix over the images of their item counts and costs (one block); the totals give the number of
+// tiles / units and the end of the cost prefix
+__global__ void __launch_bounds__(1024)
+cand_scan_kernel(int32_t* __restrict__ img_items, int32_t* __restrict__ img_cost, int Bi, int upt,
+                 int32_t* __restrict__ cpre, int32_t* __restrict__ ntiles, int32_t* __restrict__ nunits) {
+  __shared__ int si[1024], sc[1024];
+  const int tid = threadIdx.x;
+  const int per = (Bi + 1023) / 1024;
+  const int lo = min(Bi, tid * per), hi = min(Bi, lo + per);
+  int a = 0, c = 0;
+  for (int b = lo; b < hi; ++b) {
+    a += img_items[b];
+    c += img_cost[b];
+  }
+  si[tid] = a;
+  sc[tid] = c;
+  __syncthreads();
+  for (int o = 1; o < 1024; o <<= 1) {
+    const int pa = tid >= o ? si[tid - o] : 0, pc = tid >= o ? sc[tid - o] : 0;
+    __syncthreads();
+    si[tid] += pa;
+    sc[tid] += pc;
+    __syncthreads();
+  }
+  int ra = si[tid] - a, rc = sc[tid] - c;
+  for (int b = lo; b < hi; ++b) {
+    const int x = img_items[b], y = img_cost[b];
+    img_items[b] = ra;
+    img_cost[b] = rc;
+    ra += x;
+    rc += y;
+  }
+  if (tid == 1023) {
+    cpre[si[tid]] = sc[tid];
+    ntiles[0] = si[tid] / upt;
+    if (nunits) nunits[0] = si[tid];
+  }
+}
+
+// One block per word tile: the 16-bit rows (hi, and lo in split precision) and norms of the tile's virtual
+// captions, straight from the caller's fp32 words; rows no caption uses are zero.  The arithmetic (conversion,
+// the norm's summation order) is that of pack_words_kernel_tc, so a candidate pair sees the same operands as the
+// same pair in agb_damsm_fwd.
+template <typename T16>
+__global__ void __launch_bounds__(512)
+cand_rows_kernel(const float* __restrict__ words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                 const int32_t* __restrict__ cand, const int32_t* __restrict__ vlen, const int32_t* __restrict__ cap_row,
+                 const int32_t* __restrict__ item_first, const int32_t* __restrict__ item_ncap, int U,
+                 const int32_t* __restrict__ ntiles, T16* __restrict__ Wh, T16* __restrict__ Wl, float* __restrict__ pn) {
+  __shared__ int src_j[kTileN];
+  __shared__ unsigned char src_t[kTileN];
+  __shared__ float red[kTileN][4];
+  const int tile = blockIdx.x;
+  if (tile >= ntiles[0]) return;
+  if (threadIdx.x < kTileN) src_j[threadIdx.x] = -1;
+  __syncthreads();
+  const int upt = kTileN / U;
+  for (int s = 0; s < upt; ++s) {
+    const int first = item_first[tile * upt + s], n = item_ncap[tile * upt + s];
+    for (int e = threadIdx.x; e < n; e += blockDim.x) {
+      const int v = first + e, L = vlen[v];
+      const int r0 = cap_row[v] - tile * kTileN, j = cand[v];
+      for (int t = 0; t < L; ++t) {
+        src_j[r0 + t] = j;
+        src_t[r0 + t] = (unsigned char)t;
+      }
+    }
+  }
+  __syncthreads();
+  const int x = threadIdx.x & 127, g = threadIdx.x >> 7;
+#pragma unroll 4
+  for (int r = g; r < kTileN; r += 4) {
+    const int j = src_j[r];
+    float v0 = 0.f, v1 = 0.f;
+    if (j >= 0) {
+      const float* src = words + (int64_t)j * ws_b + (int64_t)src_t[r] * ws_t;
+      v0 = src[(int64_t)x * ws_d];
+      v1 = src[(int64_t)(x + 128) * ws_d];
+    }
+    const size_t row = (size_t)tile * kTileN + r;
+    const T16 h0 = cvt16<T16>(v0), h1 = cvt16<T16>(v1);
+    Wh[row * kD + x] = h0;
+    Wh[row * kD + x + 128] = h1;
+    if (Wl) {
+      Wl[row * kD + x] = cvt16<T16>(v0 - to_f32(h0));
+      Wl[row * kD + x + 128] = cvt16<T16>(v1 - to_f32(h1));
+    }
+    float ss = fmaf(v0, v0, 0.f);
+    ss = fmaf(v1, v1, ss);
+    ss = warp_sum(ss);
+    if ((threadIdx.x & 31) == 0) red[r][x >> 5] = ss;
+  }
+  __syncthreads();
+  if (threadIdx.x < kTileN) {
+    float tot = 0.f;
+    for (int w = 0; w < 4; ++w) tot += red[threadIdx.x][w];
+    pn[(size_t)tile * kTileN + threadIdx.x] = sqrtf(tot);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
 // epilogue 1 for one caption and one region (thread): NL = caption length rounded up to 4.
 // Branch-free: slots t >= L are set to -inf (their exponentials are 0) and only their stores are
 // predicated; slots below NL-4 are always live, so they carry no predicate at all.
@@ -286,6 +451,18 @@ struct FwdParams {
   float4* rowst;         // [Bi, Ntot] {<w,v>, |v|, 1/Z, -}
   int Ntot;
 };
+
+// candidate mode (agb_damsm_cand_fwd): the captions are virtual (entry v = b*K + k is a copy of caption cand[b,k]),
+// every word tile belongs to one image, and a work item is one word tile.  tile_first / tile_ncap / cap_row /
+// cap_lens / tile_cpre describe the virtual captions, m_out is [Bi*K] indexed by v.
+struct FwdCandParams : FwdParams {
+  const int32_t* tile_img;   // [ntiles] image of every word tile
+  const void* wh;            // packed words (Wh): epilogue 2 reads <w, V> from here, not from the resident tile
+};
+
+// tile_img of candidate mode; the dense kernels never read it
+__device__ __forceinline__ const int32_t* cand_tile_img(const FwdParams&) { return nullptr; }
+__device__ __forceinline__ const int32_t* cand_tile_img(const FwdCandParams& p) { return p.tile_img; }
 
 #include "damsm_tc_fwd2.inc"
 #include "damsm_tc_fwd2x.inc"
@@ -477,6 +654,140 @@ static int launch_fwd(const Packed& pk, const int32_t* cap_lens, int Bi, int Bc,
   return check_launch("damsm_fwd_kernel");
 }
 
+// ---------------------------------------------------------------------------------------------
+// candidate mode: workspace plan from shapes only (the caption lengths stay on the device)
+// ---------------------------------------------------------------------------------------------
+struct CandPlan {
+  int split;
+  long long items_max, nt_max;   // items: word tiles, or 64-row units in split precision
+  size_t off_Wh, off_Wl, off_pn, off_caprow, off_vlen, off_ifirst, off_incap, off_cpre, off_timg, off_iitems, off_icost,
+      off_counts, off_Ct, off_Ck, off_Ctl, off_Ckl, total;
+};
+
+static CandPlan make_cand_plan(int Bi, int K, int T, bool split) {
+  CandPlan p;
+  p.split = split ? 1 : 0;
+  const int U = split ? 64 : kTileN;
+  const int window = (T + 3) & ~3;
+  const long long per_unit = U / window;       // captions that always fit in one unit
+  long long units = (K + per_unit - 1) / per_unit;
+  if (split) units += units & 1;               // whole tiles per image
+  p.items_max = (long long)Bi * units;
+  p.nt_max = split ? p.items_max / 2 : p.items_max;
+  size_t o = 0;
+  auto take = [&](size_t bytes) { const size_t at = o; o = align_up(o + bytes, 1024); return at; };
+  const size_t nv = (size_t)Bi * K;
+  p.off_Wh = take((size_t)p.nt_max * kTileN * kD * 2);
+  p.off_Wl = split ? take((size_t)p.nt_max * kTileN * kD * 2) : 0;
+  p.off_pn = take((size_t)p.nt_max * kTileN * 4);
+  p.off_caprow = take(nv * 4);
+  p.off_vlen = take(nv * 4);
+  p.off_ifirst = take((size_t)p.items_max * 4);
+  p.off_incap = take((size_t)p.items_max * 4);
+  p.off_cpre = take((size_t)(p.items_max + 1) * 4);
+  p.off_timg = take((size_t)p.nt_max * 4);
+  p.off_iitems = take((size_t)Bi * 4);
+  p.off_icost = take((size_t)Bi * 4);
+  p.off_counts = take(256);
+  p.off_Ct = take((size_t)Bi * kRRows * kD * 2);
+  p.off_Ck = take((size_t)Bi * kD * kRCols * 2);
+  p.off_Ctl = split ? take((size_t)Bi * kRRows * kD * 2) : 0;
+  p.off_Ckl = split ? take((size_t)Bi * kD * kRCols * 2) : 0;
+  p.total = o;
+  return p;
+}
+
+// the cost prefix and the packed row indices are int32
+static bool cand_plan_fits(const CandPlan& p) {
+  return p.items_max * kMaxItemCost < (long long)INT32_MAX && p.nt_max * kTileN < (long long)INT32_MAX;
+}
+
+template <typename T16>
+static int run_cand(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                    const int32_t* cap_lens, int Bc, const int32_t* cand, int Bi, int K, int T, int R, float gamma1,
+                    float gamma2, float* m_out, char* ws, const CandPlan& pl, cudaStream_t st) {
+  const bool bf = std::is_same<T16, __nv_bfloat16>::value;
+  const int U = pl.split ? 64 : kTileN;
+  T16* Wh = (T16*)(ws + pl.off_Wh);
+  T16* Wl = pl.split ? (T16*)(ws + pl.off_Wl) : nullptr;
+  float* pn = (float*)(ws + pl.off_pn);
+  int32_t* cap_row = (int32_t*)(ws + pl.off_caprow);
+  int32_t* vlen = (int32_t*)(ws + pl.off_vlen);
+  int32_t* ifirst = (int32_t*)(ws + pl.off_ifirst);
+  int32_t* incap = (int32_t*)(ws + pl.off_incap);
+  int32_t* cpre = (int32_t*)(ws + pl.off_cpre);
+  int32_t* timg = (int32_t*)(ws + pl.off_timg);
+  int32_t* iitems = (int32_t*)(ws + pl.off_iitems);
+  int32_t* icost = (int32_t*)(ws + pl.off_icost);
+  int32_t* ntiles = (int32_t*)(ws + pl.off_counts);
+  int32_t* nunits = pl.split ? ntiles + 1 : nullptr;
+  T16* Ct = (T16*)(ws + pl.off_Ct);
+  T16* Ck = (T16*)(ws + pl.off_Ck);
+  T16* Ctl = pl.split ? (T16*)(ws + pl.off_Ctl) : nullptr;
+  T16* Ckl = pl.split ? (T16*)(ws + pl.off_Ckl) : nullptr;
+
+  const int pack_blocks = cdiv(Bi, 8);
+  cand_pack_kernel<false><<<pack_blocks, 256, 0, st>>>(cap_lens, Bc, T, cand, Bi, K, U, iitems, icost, nullptr,
+                                                       nullptr, nullptr, nullptr, nullptr, nullptr);
+  if (int rc = check_launch("cand_pack_kernel<false>")) return rc;
+  cand_scan_kernel<<<1, 1024, 0, st>>>(iitems, icost, Bi, kTileN / U, cpre, ntiles, nunits);
+  if (int rc = check_launch("cand_scan_kernel")) return rc;
+  cand_pack_kernel<true><<<pack_blocks, 256, 0, st>>>(cap_lens, Bc, T, cand, Bi, K, U, iitems, icost, cap_row, vlen,
+                                                      ifirst, incap, cpre, timg);
+  if (int rc = check_launch("cand_pack_kernel<true>")) return rc;
+  cand_rows_kernel<T16><<<(unsigned)pl.nt_max, 512, 0, st>>>(words, ws_b, ws_d, ws_t, cand, vlen, cap_row, ifirst, incap,
+                                                             U, ntiles, Wh, Wl, pn);
+  if (int rc = check_launch("cand_rows_kernel")) return rc;
+  pack_img_kernel_tc<T16><<<dim3(kRRows / 32, kD / 32, Bi), dim3(32, 8), 0, st>>>(img, Ck, Ct, Ckl, Ctl, R);
+  if (int rc = check_launch("pack_img_kernel_tc")) return rc;
+
+  FwdCandParams p;
+  p.tile_first = ifirst; p.tile_ncap = incap; p.ntiles = ntiles; p.cap_row = cap_row; p.cap_lens = vlen;
+  p.tile_cpre = cpre;
+  p.uniform_split = 0;
+  p.img_block = 0;
+  p.dup_rem = R > 256 ? 1 : 0;
+  p.pn = pn; p.m_out = m_out; p.Bi = Bi; p.Bc = 0; p.T = T; p.R = R;
+  p.scale_log2 = kLog2e / sqrtf((float)kD);
+  p.g1_log2 = gamma1 * kLog2e;
+  p.gamma2 = gamma2;
+  p.v16 = nullptr; p.rowst = nullptr; p.Ntot = 0;
+  p.tile_img = timg;
+  p.wh = Wh;
+  const int grid = (int)std::min<long long>(num_sms(), pl.items_max);
+  CUtensorMap mapCt, mapCk;
+  if (int rc = make_tmap_2d(&mapCt, Ct, (uint64_t)Bi * kRRows, kD, 128, bf)) return rc;
+  if (int rc = make_tmap_2d(&mapCk, Ck, (uint64_t)Bi * kD, kRCols, 128, bf)) return rc;
+  if (pl.split) {
+    if constexpr (std::is_same<T16, __half>::value) {
+      CUtensorMap mapWh, mapWl, mapCtl, mapCkl;
+      if (int rc = make_tmap_2d(&mapWh, Wh, (uint64_t)pl.nt_max * kTileN, kD, 64, false)) return rc;
+      if (int rc = make_tmap_2d(&mapWl, Wl, (uint64_t)pl.nt_max * kTileN, kD, 64, false)) return rc;
+      if (int rc = make_tmap_2d(&mapCtl, Ctl, (uint64_t)Bi * kRRows, kD, 128, false)) return rc;
+      if (int rc = make_tmap_2d(&mapCkl, Ckl, (uint64_t)Bi * kD, kRCols, 128, false)) return rc;
+      FwdXCandParams xp;
+      xp.f = p; xp.unit_first = ifirst; xp.unit_ncap = incap; xp.nunits = nunits;
+      xp.tile_img = timg; xp.wh = Wh; xp.wl = Wl;
+      auto kx = damsm_fwd2x_kernel<false, true>;
+      AGB_CUDA(cudaFuncSetAttribute(kx, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes2));
+      const int slot = prof_begin(PROF_DAMSM_CAND, st);
+      kx<<<grid, kThreads, kSmemBytes2, st>>>(mapWh, mapWl, mapCt, mapCtl, mapCk, mapCkl, xp);
+      prof_end(slot, st);
+      return check_launch("damsm_fwd2x_kernel<cand>");
+    } else {
+      return fail_unsupported("split precision needs fp16 operands");
+    }
+  }
+  CUtensorMap mapW;
+  if (int rc = make_tmap_2d(&mapW, Wh, (uint64_t)pl.nt_max * kTileN, kD, 128, bf)) return rc;
+  auto kern = damsm_fwd2_kernel<T16, false, true>;
+  AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes2));
+  const int slot = prof_begin(PROF_DAMSM_CAND, st);
+  kern<<<grid, kThreads, kSmemBytes2, st>>>(mapW, mapCt, mapCk, p);
+  prof_end(slot, st);
+  return check_launch("damsm_fwd2_kernel<cand>");
+}
+
 #include "damsm_tc_bwd2.inc"
 #include "damsm_tc_bwd3.inc"
 #include "damsm_tc_bwd2_host.inc"
@@ -528,6 +839,33 @@ int damsm_tc_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_
   if (side)
     if (int rj = tc::side_join(side, st)) return rc ? rc : rj;
   return rc;
+}
+
+// 0 when the shapes are outside the candidate path's range (the caller has checked T, D, R and math)
+size_t damsm_tc_cand_workspace_bytes(int Bi, int K, int T, int math) {
+  if (Bi <= 0 || Bi > 65535 || K <= 0 || (long long)Bi * K >= (long long)INT32_MAX) return 0;
+  const tc::CandPlan pl = tc::make_cand_plan(Bi, K, T, math == AGB_MATH_TC_F16X2);
+  return tc::cand_plan_fits(pl) ? pl.total : 0;
+}
+
+int damsm_tc_cand_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                      const int32_t* cap_lens, int Bc, const int32_t* cand, int Bi, int K, int T, int R, float gamma1,
+                      float gamma2, float* m_out, void* workspace, size_t workspace_bytes, int math, cudaStream_t st) {
+  if (Bc <= 0 || Bi <= 0 || K <= 0) return fail_arg("non-positive size");
+  if (Bi > 65535) return fail_unsupported("Bi=%d > 65535", Bi);
+  if ((long long)Bi * K >= (long long)INT32_MAX) return fail_unsupported("Bi*K=%lld >= 2^31", (long long)Bi * K);
+  if (math != AGB_MATH_TC_BF16 && gamma1 > 11.f) return fail_unsupported("gamma1=%g overflows fp16 (use bf16 math)", gamma1);
+  const tc::CandPlan pl = tc::make_cand_plan(Bi, K, T, math == AGB_MATH_TC_F16X2);
+  if (!tc::cand_plan_fits(pl)) return fail_unsupported("Bi=%d K=%d: %lld word tiles exceed the int32 cost prefix", Bi, K, pl.nt_max);
+  if (workspace_bytes < pl.total) {
+    set_error("workspace too small: %zu < %zu", workspace_bytes, pl.total);
+    return AGB_E_WORKSPACE;
+  }
+  if (math == AGB_MATH_TC_BF16)
+    return tc::run_cand<__nv_bfloat16>(img, words, ws_b, ws_d, ws_t, cap_lens, Bc, cand, Bi, K, T, R, gamma1, gamma2,
+                                       m_out, (char*)workspace, pl, st);
+  return tc::run_cand<__half>(img, words, ws_b, ws_d, ws_t, cap_lens, Bc, cand, Bi, K, T, R, gamma1, gamma2, m_out,
+                              (char*)workspace, pl, st);
 }
 
 int damsm_tc_bwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,

@@ -1,0 +1,142 @@
+"""R-precision of a trained DAMSM, scored on the B200 kernels.
+
+The AttnGAN family evaluates text-to-image models by R-precision: every image is scored against 100 captions,
+its own and 99 drawn at random from other classes, and a hit is an image whose own caption scores highest.  Two
+scores are available:
+
+  ``DAMSMScorer.sentence``  cosine of the DAMSM global vectors (cnn_code, sent_emb): AttnGAN's published definition
+  ``DAMSMScorer.words``     DAMSM's word-level matching score m[b, i] (losses/words_loss.py:77-79), the score that
+                            WordsLoss is trained on
+
+Both evaluate only the listed pairs (agb_damsm_cand_fwd / agb_sent_cos_cand_fwd), not the dense N x N matrix.
+
+    scorer = DAMSMScorer(device, gamma1=4.0, gamma2=5.0, math="f16x2")
+    cands = mismatched_candidates(class_ids, n_mismatched=99, seed=0)       # [N, 100], column 0 = own caption
+    hits = r_precision(scorer.words(img_features, words_emb, cap_lens, cands), r=1)
+"""
+from __future__ import annotations
+
+from typing import Optional
+
+import numpy as np
+import torch
+
+from ..agb_native import native, ops
+from ..losses.damsm_core import as_device_i32
+
+_CAND_MATH = ("f16", "bf16", "f16x2")
+
+
+class DAMSMScorer:
+    """Scores images against per-image lists of candidate captions.  Inference only: the inputs are detached and
+    no autograd graph is recorded.  Every input must be on the scorer's CUDA device (there is no CPU fallback);
+    cap_lens and the candidate lists may also be host arrays.
+
+    math             "f16x2" (split precision: m as accurate as fp32 arithmetic), "f16" or "bf16"
+    workspace_bytes  bound on the workspace of one ``words`` launch; larger image sets are scored in chunks of
+                     images, with results identical to one launch
+    """
+
+    def __init__(self, device, gamma1: float = 4.0, gamma2: float = 5.0, math: str = "f16x2",
+                 workspace_bytes: int = 4 << 30, eps: float = 1e-8):
+        if math not in _CAND_MATH:
+            raise ValueError(f"math must be one of {_CAND_MATH} (candidate scores run on the tensor cores)")
+        self.device = torch.device(device)
+        self.gamma1 = float(gamma1)
+        self.gamma2 = float(gamma2)
+        self.math = native.MATH_NAMES[math]
+        self.workspace_bytes = int(workspace_bytes)
+        self.eps = float(eps)
+
+    def _chunk_images(self, N: int, K: int, T: int, D: int, R: int) -> int:
+        """the most images whose candidate workspace fits workspace_bytes (the size grows with the image count)"""
+        if ops.damsm_cand_workspace_bytes(1, K, T, D, R, self.math) == 0:
+            raise native.NativeError(f"candidate DAMSM shape K={K} T={T} D={D} R={R} is unsupported")
+        lo, hi = 0, min(N, 65535)
+        while lo < hi:
+            mid = (lo + hi + 1) // 2
+            nb = ops.damsm_cand_workspace_bytes(mid, K, T, D, R, self.math)
+            if 0 < nb <= self.workspace_bytes:
+                lo = mid
+            else:
+                hi = mid - 1
+        if lo == 0:
+            need = ops.damsm_cand_workspace_bytes(1, K, T, D, R, self.math)
+            raise native.NativeError(f"workspace_bytes={self.workspace_bytes} is below the {need} bytes one image needs")
+        return lo
+
+    def words(self, img_features: torch.Tensor, words_emb: torch.Tensor, cap_lens, candidates) -> torch.Tensor:
+        """img_features [N,D,h,w] or [N,D,R], words_emb [Nc,D,T] (any strides; the RNN's transposed view is read
+        coalesced), cap_lens [Nc], candidates [N,K] caption indices (numpy, int64 or int32).
+        Returns m [N,K] fp32: m[b,k] = the DAMSM word-level score of image b and caption candidates[b,k], bit for
+        bit what WordsLoss's similarity matrix holds for that pair in the same math mode; NaN for an index
+        outside [0, Nc)."""
+        ops.require_cuda(img_features, words_emb)
+        img = img_features.detach()
+        img = img.reshape(img.shape[0], img.shape[1], -1).float().contiguous()
+        words = words_emb.detach().float()
+        N, D, R = img.shape
+        T = words.shape[2]
+        lens = as_device_i32(cap_lens, img.device)
+        cand = as_device_i32(candidates, img.device)
+        if cand.dim() != 2 or cand.shape[0] != N:
+            raise ValueError(f"candidates must be [N={N}, K], got {tuple(cand.shape)}")
+        K = cand.shape[1]
+        per = self._chunk_images(N, K, T, D, R)
+        ws = ops._ws(ops.damsm_cand_workspace_bytes(per, K, T, D, R, self.math), img.device)
+        parts = [ops.damsm_cand_fwd(img[s:s + per], words, lens, cand[s:s + per], self.gamma1, self.gamma2, self.math,
+                                    ws=ws) for s in range(0, N, per)]
+        return parts[0] if len(parts) == 1 else torch.cat(parts)
+
+    def sentence(self, cnn_code: torch.Tensor, sent_emb: torch.Tensor, candidates) -> torch.Tensor:
+        """cnn_code [N,D], sent_emb [Nc,D], candidates [N,K] -> cosine [N,K] fp32 of every listed pair
+        (losses/sentence_loss.py:33-38 before gamma3); NaN for an index outside [0, Nc)."""
+        ops.require_cuda(cnn_code, sent_emb)
+        cnn = cnn_code.detach().float().contiguous()
+        rnn = sent_emb.detach().float().contiguous()
+        cand = as_device_i32(candidates, cnn.device)
+        if cand.dim() != 2 or cand.shape[0] != cnn.shape[0]:
+            raise ValueError(f"candidates must be [N={cnn.shape[0]}, K], got {tuple(cand.shape)}")
+        return ops.sent_cos_cand_fwd(cnn, rnn, cand, self.eps)
+
+
+def mismatched_candidates(class_ids, n_mismatched: int = 99, seed: int = 0, n: Optional[int] = None) -> np.ndarray:
+    """Candidate caption lists of the R-precision protocol: [N, 1 + n_mismatched] int64, column 0 = image i's own
+    caption i, the other columns drawn uniformly with replacement from the captions whose class differs from
+    class_ids[i].  class_ids=None treats every caption as its own class (then ``n`` gives N).  Seeded numpy
+    generator on the host.  Raises ValueError when an image has no caption of another class."""
+    rng = np.random.default_rng(seed)
+    if class_ids is None:
+        if n is None:
+            raise ValueError("class_ids=None needs the number of captions n")
+        N = int(n)
+        if N < 2:
+            raise ValueError("one caption has no mismatched caption to draw")
+        own = np.arange(N)
+        u = rng.integers(0, N - 1, size=(N, n_mismatched))
+        other = u + (u >= own[:, None])                      # skip caption i itself
+    else:
+        cls = class_ids.cpu().numpy() if torch.is_tensor(class_ids) else np.asarray(class_ids)
+        cls = cls.reshape(-1)
+        N = cls.shape[0]
+        order = np.argsort(cls, kind="stable")
+        uniq, start, count = np.unique(cls[order], return_index=True, return_counts=True)
+        ci = np.searchsorted(uniq, cls)
+        pool = N - count[ci]                                 # captions of another class
+        if (pool == 0).any():
+            i = int(np.flatnonzero(pool == 0)[0])
+            raise ValueError(f"image {i} has no caption of another class (class {cls[i]} covers every caption)")
+        u = rng.integers(0, pool[:, None], size=(N, n_mismatched))
+        # position u in the class-sorted order with image i's own class block cut out
+        u = u + (u >= start[ci][:, None]) * count[ci][:, None]
+        other = order[u]
+    return np.concatenate([np.arange(N, dtype=np.int64)[:, None], other.astype(np.int64)], axis=1)
+
+
+def r_precision(scores: torch.Tensor, r: int = 1) -> torch.Tensor:
+    """[N] bool: the own caption (column 0) ranks within the top r of its row.  A tie with a mismatched caption, or
+    a NaN on either side, counts against the own caption.  Plain torch ops on the scores' device (CPU too).
+    R-precision is hits.float().mean(); the protocol reports mean and std over 10 folds of the images."""
+    own = scores[:, :1]
+    ahead = (~(scores[:, 1:] < own)).sum(dim=1)              # mismatched captions scoring >= own, or NaN
+    return (ahead < r) & ~torch.isnan(own[:, 0])

@@ -1,7 +1,8 @@
 """Importable name of the ``attention-gan_b200/`` tree (a hyphen is not a legal module name).
 
 The sub-packages of ``attention-gan_b200/`` are served as ``attention_gan_b200.agb_native``,
-``attention_gan_b200.networks`` and ``attention_gan_b200.losses`` (this package's ``__path__`` points there).
+``attention_gan_b200.networks``, ``attention_gan_b200.losses`` and ``attention_gan_b200.evaluation`` (this package's
+``__path__`` points there).
 Nothing is put on ``sys.path``: the reference's own top-level ``networks`` / ``losses`` packages stay importable
 next to the drop-ins (its generator, discriminators, encoders, GAN losses are NOT replaced).
 
@@ -27,6 +28,7 @@ from .networks.region_head import RegionFeatureHead  # noqa: E402,F401
 from .losses.words_loss import WordsLoss  # noqa: E402,F401
 from .losses.sentence_loss import SentenceLoss  # noqa: E402,F401
 from .losses.damsm_loss import DAMSMLoss  # noqa: E402,F401
+from .evaluation import DAMSMScorer, mismatched_candidates, r_precision  # noqa: E402,F401
 
 # reference module -> (native module, names it provides)
 _REPLACED = {

@@ -91,7 +91,8 @@ int agb_tc_gemm_test(const void* A, const void* B, float* C, int M, int N, int K
  * per-kernel timing with CUDA events recorded on the launching stream around the dominant kernels.
  * tag: 1 = fp32 sgemm, 2 = tcgen05 DAMSM forward pair kernel, 3 = tcgen05 DAMSM backward pair kernel,
  *      4 = word-attention forward, 5 = word-attention backward (main kernel),
- *      6 = d img reduction GEMM (tcgen05), 7 = d words reduction GEMM (tcgen05).
+ *      6 = d img reduction GEMM (tcgen05), 7 = d words reduction GEMM (tcgen05),
+ *      9 = candidate pair kernel of agb_damsm_cand_fwd (tcgen05).
  * agb_prof_read synchronises the recorded events and returns the summed duration and the count. */
 long long agb_launch_count(void);
 void agb_prof_enable(int on);
@@ -183,6 +184,28 @@ int agb_damsm_bwd(const float* img, const float* words, int64_t ws_b, int64_t ws
 int agb_damsm_supported(int T, int D, int R, int math);
 
 /* ------------------------------------------------------------------------------------------------
+ * DAMSM word-region similarity of candidate pairs (evaluation: R-precision)
+ * every image b is scored against its own list of K captions, instead of all Bc of them
+ *   m_out[b,k] = m(image b, caption cand[b,k]), defined exactly as agb_damsm_fwd's m_out (words_loss.py:43-79)
+ *   img      [Bi,D,R] fp32 contiguous;  words [Bc,D,T] fp32, element strides (ws_b, ws_d, ws_t)
+ *   cap_lens [Bc]     int32, 1 <= L <= T
+ *   cand     [Bi,K]   int32 contiguous: an index outside [0,Bc) yields NaN for that entry (never a memory fault);
+ *                     so does a caption of length 0
+ *   m_out    [Bi,K]   fp32
+ *   math: AGB_MATH_TC_F16 | AGB_MATH_TC_BF16 | AGB_MATH_TC_F16X2 (inference only: AGB_MATH_SAVE is rejected).
+ *   A pair's m is bit for bit the m of the same pair from agb_damsm_fwd with the same math.
+ * Limits: the tensor-core range of agb_damsm_supported (D = 256, T <= 32, R <= 320), Bi <= 65535, Bi*K < 2^31,
+ * and at most 2^31 / 5508 word tiles in one call (the workspace query returns 0 beyond); otherwise
+ * AGB_E_UNSUPPORTED.  The workspace size depends on the shapes only.  No host synchronisation, nothing
+ * allocated: capturable in a CUDA graph.
+ * ---------------------------------------------------------------------------------------------- */
+size_t agb_damsm_cand_workspace_bytes(int Bi, int K, int T, int D, int R, int math);
+int agb_damsm_cand_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                       const int32_t* cap_lens, int Bc, const int32_t* cand, int Bi, int K, int T, int D, int R,
+                       float gamma1, float gamma2, float* m_out, void* workspace, size_t workspace_bytes,
+                       int math, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Sentence cosine matrix on its own (SentenceLoss called without WordsLoss)
  * replaces sentence_loss.py:33-38 and its autograd
  *   scos_out [Bi,Bc] raw cosine <c_b, r_i> / max(|c_b||r_i|, eps)
@@ -195,6 +218,10 @@ size_t agb_sent_cos_bwd_workspace_bytes(int Bi, int Bc);
 int agb_sent_cos_bwd(const float* cnn, const float* rnn, int Bi, int Bc, int D, float eps,
                      const float* dscos, const float* gscale, float* dcnn, float* drnn,
                      void* workspace, size_t workspace_bytes, void* stream);
+/* the same cosine for candidate pairs: cnn [Bi,D], rnn [Bc,D] fp32 contiguous, cand [Bi,K] int32 contiguous,
+ *   scos_out[b,k] = <cnn_b, rnn_j> / max(|cnn_b| |rnn_j|, eps), j = cand[b,k]; NaN if j is outside [0,Bc) */
+int agb_sent_cos_cand_fwd(const float* cnn, const float* rnn, int Bc, const int32_t* cand, int Bi, int K, int D,
+                          float eps, float* scos_out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Two-way contrastive cross-entropy over a B x B similarity matrix
