@@ -21,7 +21,7 @@ from typing import Optional
 import numpy as np
 import torch
 
-from ..agb_native import native, ops
+from ..agb_native import native, ops, torch_ops
 from ..losses.damsm_core import as_device_i32
 
 _CAND_MATH = ("f16", "bf16", "f16x2")
@@ -48,20 +48,20 @@ class DAMSMScorer:
         self.workspace_bytes = int(workspace_bytes)
         self.eps = float(eps)
 
-    def _chunk_images(self, N: int, K: int, T: int, D: int, R: int) -> int:
+    def _chunk_images(self, N: int, K: int, T: int, D: int, R: int, ws_bytes=ops.damsm_cand_workspace_bytes) -> int:
         """the most images whose candidate workspace fits workspace_bytes (the size grows with the image count)"""
-        if ops.damsm_cand_workspace_bytes(1, K, T, D, R, self.math) == 0:
+        if ws_bytes(1, K, T, D, R, self.math) == 0:
             raise native.NativeError(f"candidate DAMSM shape K={K} T={T} D={D} R={R} is unsupported")
         lo, hi = 0, min(N, 65535)
         while lo < hi:
             mid = (lo + hi + 1) // 2
-            nb = ops.damsm_cand_workspace_bytes(mid, K, T, D, R, self.math)
+            nb = ws_bytes(mid, K, T, D, R, self.math)
             if 0 < nb <= self.workspace_bytes:
                 lo = mid
             else:
                 hi = mid - 1
         if lo == 0:
-            need = ops.damsm_cand_workspace_bytes(1, K, T, D, R, self.math)
+            need = ws_bytes(1, K, T, D, R, self.math)
             raise native.NativeError(f"workspace_bytes={self.workspace_bytes} is below the {need} bytes one image needs")
         return lo
 
@@ -82,6 +82,12 @@ class DAMSMScorer:
         if cand.dim() != 2 or cand.shape[0] != N:
             raise ValueError(f"candidates must be [N={N}, K], got {tuple(cand.shape)}")
         K = cand.shape[1]
+        if torch.compiler.is_compiling():
+            # traced: the same chunks as agb::damsm_cand_fwd calls, each with a workspace of its own
+            per = self._chunk_images(N, K, T, D, R, _traced_cand_workspace_bytes)
+            parts = [torch.ops.agb.damsm_cand_fwd(img[s:s + per], words, lens, cand[s:s + per], self.gamma1,
+                                                  self.gamma2, self.math) for s in range(0, N, per)]
+            return parts[0] if len(parts) == 1 else torch.cat(parts)
         per = self._chunk_images(N, K, T, D, R)
         ws = ops._ws(ops.damsm_cand_workspace_bytes(per, K, T, D, R, self.math), img.device)
         parts = [ops.damsm_cand_fwd(img[s:s + per], words, lens, cand[s:s + per], self.gamma1, self.gamma2, self.math,
@@ -97,7 +103,13 @@ class DAMSMScorer:
         cand = as_device_i32(candidates, cnn.device)
         if cand.dim() != 2 or cand.shape[0] != cnn.shape[0]:
             raise ValueError(f"candidates must be [N={cnn.shape[0]}, K], got {tuple(cand.shape)}")
+        if torch.compiler.is_compiling():
+            return torch.ops.agb.sent_cos_cand_fwd(cnn, rnn, cand, self.eps)
         return ops.sent_cos_cand_fwd(cnn, rnn, cand, self.eps)
+
+
+def _traced_cand_workspace_bytes(*args) -> int:
+    return torch_ops.host_query("agb_damsm_cand_workspace_bytes", *args)
 
 
 def mismatched_candidates(class_ids, n_mismatched: int = 99, seed: int = 0, n: Optional[int] = None) -> np.ndarray:

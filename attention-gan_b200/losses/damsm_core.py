@@ -27,6 +27,7 @@ import torch.distributed as dist
 
 from ..agb_native import native
 from ..agb_native import ops as native_ops
+from ..agb_native import torch_ops
 
 
 @dataclass
@@ -52,12 +53,17 @@ def resolve_math(math, img_features=None, words_emb=None, gamma1: float = 4.0) -
     kernels of this library; the choice is a host-side query (agb_damsm_supported), no data is touched."""
     if math != "auto":
         return native.MATH_NAMES[math]
-    if img_features is None or words_emb is None or not native.lib().agb_has_tcgen05() or gamma1 > 11.0:
+    query = torch_ops.host_query if torch.compiler.is_compiling() else _host_query
+    if img_features is None or words_emb is None or not query("agb_has_tcgen05") or gamma1 > 11.0:
         return native.AGB_MATH_FP32
     D, T = int(words_emb.shape[1]), int(words_emb.shape[2])
     R = int(img_features.shape[2]) * int(img_features.shape[3]) if img_features.dim() == 4 else int(img_features.shape[2])
-    ok = native.lib().agb_damsm_supported(T, D, R, native.AGB_MATH_TC_F16X2)
+    ok = query("agb_damsm_supported", T, D, R, native.AGB_MATH_TC_F16X2)
     return native.AGB_MATH_TC_F16X2 if ok else native.AGB_MATH_FP32
+
+
+def _host_query(name: str, *args):
+    return getattr(native.lib(), name)(*args)
 
 
 def _world(group) -> int:
@@ -237,6 +243,41 @@ class _SentLossFn(torch.autograd.Function):
         return dcnn, drnn, None, None, None
 
 
+# ------------------------------------------------------------------------------------------------
+# the same losses while torch.compile traces: the agb:: ops (agb_native/torch_ops.py), single process only
+# ------------------------------------------------------------------------------------------------
+def _op_path(*cfgs: DamsmConfig) -> bool:
+    """trace the agb:: ops: compiling, the native kernels (not an injected backend) and no process group (the
+    NCCL exchange of a sharded loss stays eager, behind a graph break)"""
+    return torch.compiler.is_compiling() and all(c.ops is native_ops and c.group is None for c in cfgs)
+
+
+def _words_loss_op(img, words, cfg: DamsmConfig, ex: _Exchange):
+    """_WordsLossFn of a single process as agb:: ops: (loss, packed att [Bl,T,R] or empty)"""
+    Bl, D = img.shape[0], img.shape[1]
+    img3 = img.float().reshape(Bl, D, -1).contiguous()
+    w32 = words.float()
+    math = cfg.math
+    if math != native.AGB_MATH_FP32 and \
+            not torch_ops.host_query("agb_damsm_supported", int(w32.shape[2]), D, int(img3.shape[2]), math):
+        math = native.AGB_MATH_FP32
+    save = math != native.AGB_MATH_FP32 and torch.is_grad_enabled() and (img.requires_grad or words.requires_grad)
+    m, att, _, _ = torch.ops.agb.damsm_fwd(img3, w32, ex.lens, None, None, cfg.gamma1, cfg.gamma2, cfg.eps, 0,
+                                           cfg.want_att, math, save)
+    loss, _ = torch.ops.agb.contrastive(m, ex.cls, ex.labels, cfg.gamma3, cfg.lam, 0, Bl, True)
+    return loss.reshape(()), att
+
+
+def _sentence_loss_op(cnn, rnn, cfg: DamsmConfig, ex: _Exchange):
+    """_SentLossFn of a single process as agb:: ops"""
+    D = cnn.shape[-1]
+    cnn32 = cnn.float().reshape(-1, D).contiguous()
+    rnn32 = rnn.float().reshape(-1, D).contiguous()
+    scos = torch.ops.agb.sent_cos_fwd(cnn32, rnn32, cfg.eps)
+    loss, _ = torch.ops.agb.contrastive(scos, ex.cls, ex.labels, cfg.gamma3, cfg.lam, 0, cnn32.shape[0], True)
+    return loss.reshape(())
+
+
 def split_att_maps(att: torch.Tensor, cap_lens, ih: int, iw: int, row0: int = 0) -> List[torch.Tensor]:
     """packed beta [Bl,T,R] of the matched pairs -> the reference's list of [1, L_i, ih, iw]
     (words_loss.py:63).  Needs the caption lengths on the host, like the reference (:41)."""
@@ -248,7 +289,10 @@ def words_loss(img_features, words_emb, labels, cap_lens, class_ids, cfg: DamsmC
     """(wloss, packed att [Bl,T,R] or None)"""
     cfg.ops.require_cuda(img_features, words_emb) if hasattr(cfg.ops, "require_cuda") else None
     ex = _Exchange(cfg, img_features.shape[0], labels, cap_lens, class_ids, img_features.device)
-    loss, att = _WordsLossFn.apply(img_features, words_emb, cfg, ex, None, None)
+    if _op_path(cfg):
+        loss, att = _words_loss_op(img_features, words_emb, cfg, ex)
+    else:
+        loss, att = _WordsLossFn.apply(img_features, words_emb, cfg, ex, None, None)
     return loss, (att if cfg.want_att else None)
 
 
@@ -256,6 +300,8 @@ def sentence_loss(cnn_code, rnn_code, labels, class_ids, cfg: DamsmConfig):
     cfg.ops.require_cuda(cnn_code, rnn_code) if hasattr(cfg.ops, "require_cuda") else None
     n_local = cnn_code.shape[-2]
     ex = _Exchange(cfg, n_local, labels, None, class_ids, cnn_code.device)
+    if _op_path(cfg):
+        return _sentence_loss_op(cnn_code, rnn_code, cfg, ex)
     return _SentLossFn.apply(cnn_code, rnn_code, cfg, ex, None)
 
 
@@ -266,6 +312,12 @@ def damsm_losses(img_features, cnn_code, words_emb, rnn_code, labels, cap_lens, 
     Returns (wloss, sloss, packed att or None)."""
     wcfg.ops.require_cuda(img_features, words_emb, cnn_code, rnn_code) if hasattr(wcfg.ops, "require_cuda") else None
     ex = _Exchange(wcfg, img_features.shape[0], labels, cap_lens, class_ids, img_features.device)
+    if _op_path(wcfg, scfg):
+        # traced: the two losses one after the other on the current stream (the kernels are deterministic, so the
+        # results are those of the forked-stream eager path)
+        sloss = _sentence_loss_op(cnn_code, rnn_code, scfg, ex)
+        wloss, att = _words_loss_op(img_features, words_emb, wcfg, ex)
+        return wloss, sloss, (att if wcfg.want_att else None)
     if ex.W == 1 and img_features.is_cuda:
         # Single process: the sentence loss (cosine matrix, its contrastive CE and, in backward, its two
         # gradient kernels) is independent of the word-region kernels, so it runs on a forked stream beside

@@ -18,6 +18,7 @@ import torch
 from torch import nn
 
 from ..agb_native import ops
+from ..agb_native import torch_ops  # noqa: F401  (registers torch.ops.agb, used while compiling)
 
 GlobalAttention = None  # set below (BASELINE.json's name for AttentionModule)
 
@@ -107,6 +108,15 @@ class _WordAttentionInto(torch.autograd.Function):
         return (dimages if need_img else None), dwords, dweight, None, None, None, None
 
 
+def _word_attn_operands(images, words, weight, mask):
+    """the operands the kernels take, built like _WordAttention.forward does (traced by torch.compile)"""
+    w32 = words if words.dtype == torch.float32 else words.float()
+    wt = weight.reshape(weight.shape[0], -1)
+    wt32 = (wt if wt.dtype == torch.float32 else wt.float()).contiguous()
+    m64 = (mask if mask.dtype == torch.int64 else mask.to(torch.int64)).to(images.device).contiguous()
+    return w32, wt32, m64
+
+
 class AttentionModule(nn.Module):
     """Word-context attention of the generator's refinement stages
     (reference networks/attention.py:15-79; called from generator_submodules.py:113-114)."""
@@ -127,8 +137,11 @@ class AttentionModule(nn.Module):
             # the reference dereferences self.mask unconditionally (attention.py:47,65)
             raise AttributeError("AttentionModule.forward called before apply_mask(mask)")
         ops.require_cuda(images, words, self.conv1.weight)
+        if torch.compiler.is_compiling():
+            w32, wt32, m64 = _word_attn_operands(images, words, self.conv1.weight, self.mask)
+            ctx, attn, _ = torch.ops.agb.word_attn_fwd(images, w32, wt32, m64, bool(scaled), True)
+            return ctx, attn
         return _WordAttention.apply(images, words, self.conv1.weight, self.mask, bool(scaled))
-
 
     def forward_into(self, images, words, out, scaled=True, want_attn=True):
         """images [B, C, H, W], words [B, E, T], out [B, 2C, H, W] (pre-allocated, contiguous) ->
@@ -137,9 +150,31 @@ class AttentionModule(nn.Module):
         if self.mask is None:
             raise AttributeError("AttentionModule.forward_into called before apply_mask(mask)")
         ops.require_cuda(images, words, self.conv1.weight, out)
+        if torch.compiler.is_compiling():
+            # the op returns a fresh buffer (custom ops do not write into their inputs' storage): one extra copy
+            B, C, H, W = images.shape
+            if out.shape != (B, 2 * C, H, W) or out.dtype != images.dtype or not out.is_contiguous():
+                raise RuntimeError("forward_into: `out` must be a contiguous [B, 2*C, H, W] tensor of the images' dtype")
+            res, attn = self.forward_cat(images, words, scaled, want_attn)
+            return out.copy_(res), attn
         res, attn = _WordAttentionInto.apply(images, words, self.conv1.weight, self.mask, bool(scaled), out,
                                              bool(want_attn))
         return res, (attn if want_attn else None)
+
+    def forward_cat(self, images, words, scaled=True, want_attn=True):
+        """images [B, C, H, W], words [B, E, T] -> (torch.cat((images, context), 1) [B, 2C, H, W], attn [B, T, H, W]
+        or None): forward_into with a buffer of its own.  The spelling for code compiled with torch.compile, where
+        the kernel writes the context straight into the fresh buffer.  Not part of the reference API."""
+        if self.mask is None:
+            raise AttributeError("AttentionModule.forward_cat called before apply_mask(mask)")
+        ops.require_cuda(images, words, self.conv1.weight)
+        if torch.compiler.is_compiling():
+            w32, wt32, m64 = _word_attn_operands(images, words, self.conv1.weight, self.mask)
+            out, attn, _ = torch.ops.agb.word_attn_cat(images, w32, wt32, m64, bool(scaled), bool(want_attn))
+            return out, (attn if want_attn else None)
+        B, C, H, W = images.shape
+        out = torch.empty((B, 2 * C, H, W), dtype=images.dtype, device=images.device)
+        return self.forward_into(images, words, out, scaled, want_attn)
 
 
 GlobalAttention = AttentionModule
@@ -180,4 +215,11 @@ def func_attention(query, context, gamma1=4.0, scaled=True):
     """query [B, D, L] (words), context [B, D, ih, iw] (regions) ->
     (weightedContext [B, D, L], attn [B, L, ih, iw])        reference networks/attention.py:82-121"""
     ops.require_cuda(query, context)
+    if torch.compiler.is_compiling():
+        B, D, L = query.shape
+        ih, iw = context.shape[2], context.shape[3]
+        q32 = query if query.dtype == torch.float32 else query.float()
+        c32 = (context if context.dtype == torch.float32 else context.float()).reshape(B, D, ih * iw).contiguous()
+        wc, attn = torch.ops.agb.func_attention_fwd(q32, c32, float(gamma1), bool(scaled))
+        return wc.to(query.dtype), attn.reshape(B, L, ih, iw).to(query.dtype)
     return _FuncAttention.apply(query, context, float(gamma1), bool(scaled))

@@ -13,6 +13,7 @@ import torch
 from torch import nn
 
 from ..agb_native import ops
+from ..agb_native import torch_ops  # noqa: F401  (registers torch.ops.agb, used while compiling)
 
 
 class _RegionHead(torch.autograd.Function):
@@ -42,6 +43,19 @@ class _RegionHead(torch.autograd.Function):
         return dx, dw
 
 
+def region_head(x: torch.Tensor, weight: torch.Tensor) -> torch.Tensor:
+    """x [B, Cin, H, W], weight [Cout, Cin, 1, 1] -> [B, Cout, H, W]: _RegionHead, or agb::region_head_fwd while
+    torch.compile traces (same kernels, same operands)"""
+    if torch.compiler.is_compiling():
+        B, Cin, H, W = x.shape
+        x3 = (x if x.dtype == torch.float32 else x.float()).reshape(B, Cin, H * W).contiguous()
+        w2 = weight.reshape(weight.shape[0], Cin)
+        w2 = (w2 if w2.dtype == torch.float32 else w2.float()).contiguous()
+        feat, _ = torch.ops.agb.region_head_fwd(x3, w2)
+        return feat.reshape(B, weight.shape[0], H, W).to(x.dtype)
+    return _RegionHead.apply(x, weight)
+
+
 class RegionFeatureHead(nn.Module):
     def __init__(self, out_dim: int = 256, in_dim: int = 768):
         super().__init__()
@@ -51,4 +65,4 @@ class RegionFeatureHead(nn.Module):
     def forward(self, mixed_6e: torch.Tensor) -> torch.Tensor:
         """mixed_6e [B, 768, 17, 17] -> region features [B, out_dim, 17, 17]"""
         ops.require_cuda(mixed_6e, self.emb_features.weight)
-        return _RegionHead.apply(mixed_6e, self.emb_features.weight)
+        return region_head(mixed_6e, self.emb_features.weight)

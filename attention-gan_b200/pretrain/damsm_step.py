@@ -28,7 +28,7 @@ from torch.nn.utils import clip_grad_norm_
 from torch.nn.utils.rnn import pack_padded_sequence, pad_packed_sequence
 
 from ..losses.damsm_loss import DAMSMLoss
-from ..networks.region_head import _RegionHead
+from ..networks.region_head import region_head
 
 
 class TextEncoder(nn.Module):
@@ -83,7 +83,7 @@ class RegionHeads(nn.Module):
     def forward(self, mixed_6e: torch.Tensor, pooled: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
         """mixed_6e [B,768,17,17], pooled [B,2048] -> (region features [B,256,17,17], cnn_code [B,256])"""
         if self.native and mixed_6e.is_cuda:
-            return _RegionHead.apply(mixed_6e, self.emb_features.weight), self.emb_cnn_code(pooled)
+            return region_head(mixed_6e, self.emb_features.weight), self.emb_cnn_code(pooled)
         return self.emb_features(mixed_6e), self.emb_cnn_code(pooled)
 
 
