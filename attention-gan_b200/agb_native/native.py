@@ -50,7 +50,13 @@ SIGNATURES = {
     "agb_damsm_cand_fwd": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p, c_int,
                                    c_int, c_int, c_int, c_int, c_float, c_float, c_void_p, c_void_p, c_size_t, c_int,
                                    c_void_p]),
+    "agb_damsm_pairs_workspace_bytes": (c_size_t, [c_int, c_int, ctypes.c_longlong, c_int, c_int, c_int, c_int]),
+    "agb_damsm_pairs_fwd": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int, c_void_p,
+                                    c_void_p, ctypes.c_longlong, c_int, c_int, c_int, c_float, c_float, c_void_p,
+                                    c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
     "agb_sent_cos_fwd": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p]),
+    "agb_sent_cos_pairs_fwd": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, ctypes.c_longlong, c_int,
+                                       c_float, c_void_p, c_void_p]),
     "agb_sent_cos_cand_fwd": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_float, c_void_p,
                                       c_void_p]),
     "agb_sent_cos_bwd_workspace_bytes": (c_size_t, [c_int, c_int]),

@@ -195,6 +195,65 @@ def sent_cos_cand_fwd(cnn: torch.Tensor, rnn: torch.Tensor, cand: torch.Tensor, 
     return scos
 
 
+def damsm_pairs_workspace_bytes(Bi: int, Bc: int, P: int, T: int, D: int, R: int, math: int) -> int:
+    """workspace of damsm_pairs_fwd; 0 when the shapes are outside the pair path's range"""
+    return int(N.lib().agb_damsm_pairs_workspace_bytes(Bi, Bc, P, T, D, R, math))
+
+
+def _pair_index(t: torch.Tensor, name: str) -> None:
+    if t.dtype != torch.int32 or t.dim() != 1 or not t.is_contiguous():
+        raise RuntimeError(f"{name} must be a contiguous int32 [P] tensor")
+
+
+def damsm_pairs_fwd(img: torch.Tensor, words: torch.Tensor, cap_lens: torch.Tensor, pair_img: torch.Tensor,
+                    pair_cap: torch.Tensor, gamma1: float, gamma2: float, math: int, want_att: bool = False,
+                    ws: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+    """m of a pair list: img [Bi,D,R] fp32 contiguous, words [Bc,D,T] fp32 (any strides), cap_lens [Bc] int32,
+    pair_img / pair_cap [P] int32 contiguous.  Returns (m [P] fp32, att [P,T,R] fp32 or None): m[p] = damsm_fwd's
+    m[pair_img[p], pair_cap[p]] bit for bit, att[p] the pair's beta maps; NaN for an index out of range or a caption
+    of length 0.  Tensor-core math only.  ws: a uint8 workspace of at least damsm_pairs_workspace_bytes."""
+    require_cuda(img, words, cap_lens, pair_img, pair_cap)
+    Bi, D, R = img.shape
+    Bc, _, T = words.shape
+    _pair_index(pair_img, "pair_img")
+    _pair_index(pair_cap, "pair_cap")
+    P = pair_img.shape[0]
+    if pair_cap.shape[0] != P:
+        raise RuntimeError(f"pair_img has {P} entries, pair_cap {pair_cap.shape[0]}")
+    nbytes = damsm_pairs_workspace_bytes(Bi, Bc, P, T, D, R, math)
+    if nbytes == 0:
+        raise N.NativeError(f"pair DAMSM shape Bi={Bi} Bc={Bc} P={P} T={T} D={D} R={R} is unsupported for math mode {math}")
+    m = torch.empty((P,), dtype=torch.float32, device=img.device)
+    att = torch.empty((P, T, R), dtype=torch.float32, device=img.device) if want_att else None
+    if P == 0:
+        return m, att
+    if ws is None:
+        ws = _ws(nbytes, img.device)
+    rc = N.lib().agb_damsm_pairs_fwd(_p(img), _p(words), words.stride(0), words.stride(1), words.stride(2),
+                                     _p(cap_lens), Bi, Bc, _p(pair_img), _p(pair_cap), P, T, D, R, gamma1, gamma2,
+                                     _p(m), _p(att), _p(ws), ws.numel(), math, _stream(img))
+    N.check(rc, "agb_damsm_pairs_fwd")
+    return m, att
+
+
+def sent_cos_pairs_fwd(cnn: torch.Tensor, rnn: torch.Tensor, pair_img: torch.Tensor, pair_cap: torch.Tensor,
+                       eps: float) -> torch.Tensor:
+    """cnn [Bi,D], rnn [Bc,D] fp32 contiguous, pair_img / pair_cap [P] int32 contiguous -> cosine [P] of the pairs
+    (NaN where an index is out of range)"""
+    require_cuda(cnn, rnn, pair_img, pair_cap)
+    Bi, D = cnn.shape
+    _pair_index(pair_img, "pair_img")
+    _pair_index(pair_cap, "pair_cap")
+    P = pair_img.shape[0]
+    if pair_cap.shape[0] != P:
+        raise RuntimeError(f"pair_img has {P} entries, pair_cap {pair_cap.shape[0]}")
+    scos = torch.empty((P,), dtype=torch.float32, device=cnn.device)
+    rc = N.lib().agb_sent_cos_pairs_fwd(_p(cnn), _p(rnn), Bi, rnn.shape[0], _p(pair_img), _p(pair_cap), P, D, eps,
+                                        _p(scos), _stream(cnn))
+    N.check(rc, "agb_sent_cos_pairs_fwd")
+    return scos
+
+
 def contrastive(raw: torch.Tensor, class_ids: Optional[torch.Tensor], labels: torch.Tensor, gamma3: float,
                 lam: float, row_begin: int, row_count: int, want_grad: bool = True):
     """raw [B,B] fp32 (all rows), class_ids [B] int32 or None, labels [B] int64.

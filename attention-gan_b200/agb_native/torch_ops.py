@@ -332,6 +332,41 @@ def _(cnn, rnn, cand, eps):
     return cnn.new_empty((cnn.shape[0], cand.shape[1]), dtype=torch.float32)
 
 
+@_op("damsm_pairs_fwd")
+def damsm_pairs_fwd(img: Tensor, words: Tensor, cap_lens: Tensor, pair_img: Tensor, pair_cap: Tensor, gamma1: float,
+                    gamma2: float, want_att: bool, math: int) -> Tuple[Tensor, Tensor]:
+    """(m [P], att [P,T,R] or empty) of the pair list pair_img / pair_cap [P] int32 (ops.damsm_pairs_fwd; the
+    workspace is allocated here)"""
+    m, att = ops.damsm_pairs_fwd(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math, want_att)
+    return m, _none(att, img.device)
+
+
+@damsm_pairs_fwd.register_fake
+def _(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, want_att, math):
+    Bi, D, R = img.shape
+    Bc, _, T = words.shape
+    P = pair_img.shape[0]
+    if pair_cap.shape[0] != P:
+        raise RuntimeError(f"pair_img has {P} entries, pair_cap {pair_cap.shape[0]}")
+    if int(N.lib().agb_damsm_pairs_workspace_bytes(Bi, Bc, P, T, D, R, math)) == 0:
+        raise N.NativeError(f"pair DAMSM shape Bi={Bi} Bc={Bc} P={P} T={T} D={D} R={R} is unsupported for math mode {math}")
+    f32 = dict(dtype=torch.float32)
+    return img.new_empty((P,), **f32), img.new_empty((P, T, R) if want_att else (0,), **f32)
+
+
+@_op("sent_cos_pairs_fwd")
+def sent_cos_pairs_fwd(cnn: Tensor, rnn: Tensor, pair_img: Tensor, pair_cap: Tensor, eps: float) -> Tensor:
+    """cosine [P] of the pair list"""
+    return ops.sent_cos_pairs_fwd(cnn, rnn, pair_img, pair_cap, eps)
+
+
+@sent_cos_pairs_fwd.register_fake
+def _(cnn, rnn, pair_img, pair_cap, eps):
+    if pair_cap.shape[0] != pair_img.shape[0]:
+        raise RuntimeError(f"pair_img has {pair_img.shape[0]} entries, pair_cap {pair_cap.shape[0]}")
+    return cnn.new_empty((pair_img.shape[0],), dtype=torch.float32)
+
+
 # ------------------------------------------------------------------------------------------------
 # functional region-word attention
 # ------------------------------------------------------------------------------------------------
@@ -442,3 +477,5 @@ region_head_fwd.register_autograd(_region_head_backward, setup_context=_region_h
 OPS = ("word_attn_fwd", "word_attn_cat", "word_attn_bwd", "damsm_fwd", "damsm_bwd", "contrastive", "sent_cos_fwd",
        "sent_cos_bwd", "func_attention_fwd", "func_attention_bwd", "region_head_fwd", "region_head_bwd",
        "damsm_cand_fwd", "sent_cos_cand_fwd")
+# the pair-list scorers of the evaluation path (DAMSMScorer.words_pairs / sentence_pairs)
+PAIR_OPS = ("damsm_pairs_fwd", "sent_cos_pairs_fwd")

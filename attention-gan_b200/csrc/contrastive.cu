@@ -323,9 +323,48 @@ sent_cos_cand_kernel(const float* __restrict__ cnn, const float* __restrict__ rn
   if (lane == 0) out[v] = num / fmaxf(sqrtf(p2) * sqrtf(q2), eps);
 }
 
+// sentence cosine of listed pairs: one warp per pair p, image b = pair_img[p], caption j = pair_cap[p], with the
+// summation order of sent_cos_cand_kernel; NaN when b or j is out of range
+__global__ void __launch_bounds__(256)
+sent_cos_pairs_kernel(const float* __restrict__ cnn, const float* __restrict__ rnn, int Bi, int Bc,
+                      const int32_t* __restrict__ pair_img, const int32_t* __restrict__ pair_cap, int n, int D,
+                      float eps, float* __restrict__ out) {
+  const long long v = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (v >= n) return;
+  const int b = pair_img[v], j = pair_cap[v];
+  if (b < 0 || b >= Bi || j < 0 || j >= Bc) {
+    if (lane == 0) out[v] = __int_as_float(0x7fc00000);
+    return;
+  }
+  float num = 0.f, p2 = 0.f, q2 = 0.f;
+  for (int d = lane; d < D; d += 32) {
+    const float c = cnn[(size_t)b * D + d], r = rnn[(size_t)j * D + d];
+    num = fmaf(c, r, num);
+    p2 = fmaf(c, c, p2);
+    q2 = fmaf(r, r, q2);
+  }
+  num = warp_sum(num);
+  p2 = warp_sum(p2);
+  q2 = warp_sum(q2);
+  if (lane == 0) out[v] = num / fmaxf(sqrtf(p2) * sqrtf(q2), eps);
+}
+
 }  // namespace agb
 
 using namespace agb;
+
+extern "C" int agb_sent_cos_pairs_fwd(const float* cnn, const float* rnn, int Bi, int Bc, const int32_t* pair_img,
+                                      const int32_t* pair_cap, long long P, int D, float eps, float* scos_out,
+                                      void* stream) {
+  if (Bi <= 0 || Bc <= 0 || D <= 0 || P < 0) return fail_arg("non-positive size");
+  if (P >= 0x7fffffffLL) return fail_unsupported("P=%lld >= 2^31", P);
+  if (P == 0) return 0;
+  if (!cnn || !rnn || !pair_img || !pair_cap || !scos_out) return fail_arg("null pointer");
+  sent_cos_pairs_kernel<<<(unsigned)((P + 7) / 8), 256, 0, (cudaStream_t)stream>>>(cnn, rnn, Bi, Bc, pair_img, pair_cap,
+                                                                                 (int)P, D, eps, scos_out);
+  return check_launch("sent_cos_pairs_kernel");
+}
 
 extern "C" int agb_sent_cos_cand_fwd(const float* cnn, const float* rnn, int Bc, const int32_t* cand, int Bi, int K,
                                      int D, float eps, float* scos_out, void* stream) {

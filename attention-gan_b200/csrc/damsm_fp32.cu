@@ -551,11 +551,15 @@ static int func_scores(const float* query, int64_t qs_b, int64_t qs_d, int64_t q
 // The feature dimension is split over the CTAs of a thread-block cluster (blockIdx.y = slice): every CTA
 // accumulates the raw scores of its slice, the partial sums meet in the leader through distributed
 // shared memory in a fixed order, and the leader finishes the two softmaxes.
-template <int TMAX>
-__global__ void __launch_bounds__(1024)
-diag_att_kernel(const float* __restrict__ img, const float* __restrict__ words, int64_t ws_b, int64_t ws_d,
-                int64_t ws_t, const int32_t* __restrict__ cap_lens, int T, int D, int R, float inv_sqrt_d,
-                float gamma1, int row_offset, float* __restrict__ att_out) {
+// Body of one block.  pick(b, i, o) chooses image b, caption i and the att_out slot o of the block; when it returns
+// false the block writes NaN maps instead (pick is the same for every CTA of a cluster, so the cluster returns as
+// one).
+template <int TMAX, class Pick>
+__device__ __forceinline__ void att_maps_block(const float* __restrict__ img, const float* __restrict__ words,
+                                               int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                                               const int32_t* __restrict__ cap_lens, int T, int D, int R,
+                                               float inv_sqrt_d, float gamma1, Pick pick,
+                                               float* __restrict__ att_out) {
   namespace cg = cooperative_groups;
   cg::cluster_group cluster = cg::this_cluster();
   extern __shared__ float w_s[];                  // [slice of D][TMAX] words, then [TMAX][blockDim.x] partial scores
@@ -564,7 +568,13 @@ diag_att_kernel(const float* __restrict__ img, const float* __restrict__ words, 
   float* acc_s = w_s + (size_t)((D + parts - 1) / parts + 1) * TMAX;
   __shared__ float red_s[32 * TMAX];
   __shared__ float z_s[TMAX];
-  const int b = blockIdx.x, r = threadIdx.x, i = row_offset + b;
+  int b, i, o;
+  if (!pick(b, i, o)) {
+    if (part == 0 && (int)threadIdx.x < R)
+      for (int t = 0; t < T; ++t) att_out[((size_t)o * T + t) * R + threadIdx.x] = __int_as_float(0x7fc00000);
+    return;
+  }
+  const int r = threadIdx.x;
   const int L = min(max(cap_lens[i], 0), T);
   for (int k = threadIdx.x; k < (d1 - d0) * TMAX; k += blockDim.x) {
     const int d = k / TMAX, t = k - d * TMAX;
@@ -626,7 +636,39 @@ diag_att_kernel(const float* __restrict__ img, const float* __restrict__ words, 
   if (!live) return;
 #pragma unroll
   for (int t = 0; t < TMAX; ++t)
-    if (t < T) att_out[((size_t)b * T + t) * R + r] = (t < L) ? e[t] / z_s[t] : 0.f;
+    if (t < T) att_out[((size_t)o * T + t) * R + r] = (t < L) ? e[t] / z_s[t] : 0.f;
+}
+
+template <int TMAX>
+__global__ void __launch_bounds__(1024)
+diag_att_kernel(const float* __restrict__ img, const float* __restrict__ words, int64_t ws_b, int64_t ws_d,
+                int64_t ws_t, const int32_t* __restrict__ cap_lens, int T, int D, int R, float inv_sqrt_d,
+                float gamma1, int row_offset, float* __restrict__ att_out) {
+  auto pick = [&](int& b, int& i, int& o) {
+    b = blockIdx.x;
+    i = row_offset + b;
+    o = b;
+    return true;
+  };
+  att_maps_block<TMAX>(img, words, ws_b, ws_d, ws_t, cap_lens, T, D, R, inv_sqrt_d, gamma1, pick, att_out);
+}
+
+// beta of listed pairs (agb_damsm_pairs_fwd): block p = image pair_img[p], caption pair_cap[p], with the arithmetic
+// of diag_att_kernel.  A pair whose image or caption index is out of range, or whose caption has length 0, gets NaN
+// maps.
+template <int TMAX>
+__global__ void __launch_bounds__(1024)
+pair_att_kernel(const float* __restrict__ img, const float* __restrict__ words, int64_t ws_b, int64_t ws_d,
+                int64_t ws_t, const int32_t* __restrict__ cap_lens, int Bi, int Bc, const int32_t* __restrict__ pair_img,
+                const int32_t* __restrict__ pair_cap, int T, int D, int R, float inv_sqrt_d, float gamma1,
+                float* __restrict__ att_out) {
+  auto pick = [&](int& b, int& i, int& o) {
+    o = blockIdx.x;
+    b = pair_img[o];
+    i = pair_cap[o];
+    return b >= 0 && b < Bi && i >= 0 && i < Bc && cap_lens[i] > 0;
+  };
+  att_maps_block<TMAX>(img, words, ws_b, ws_d, ws_t, cap_lens, T, D, R, inv_sqrt_d, gamma1, pick, att_out);
 }
 
 int damsm_diag_att_maps(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
@@ -659,6 +701,36 @@ int damsm_diag_att_maps(const float* img, const float* words, int64_t ws_b, int6
                                 att_out));
   });
   return check_launch("diag_att_kernel");
+}
+
+int damsm_pair_att_maps(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                        const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap,
+                        int P, int T, int D, int R, float gamma1, float* att_out, cudaStream_t st) {
+  const int tpr = (R + 31) / 32 * 32;
+  if (tpr > 1024) return fail_unsupported("R=%d regions > 1024", R);
+  const int parts = D >= 64 ? 4 : 1;              // the cluster split of damsm_diag_att_maps
+  const float isd = 1.f / sqrtf((float)D);
+  const int tm = pick_tmax(T);
+  const size_t smem = ((size_t)((D + parts - 1) / parts + 1) * tm + (size_t)tm * tpr) * sizeof(float);
+  AGB_TMAX_SWITCH(tm, {
+    auto kern = pair_att_kernel<TMAX>;
+    if (smem > 48 * 1024) AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(P, parts);
+    cfg.blockDim = dim3(tpr);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 1;
+    attr[0].val.clusterDim.y = parts;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    AGB_CUDA(cudaLaunchKernelEx(&cfg, kern, img, words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, pair_img, pair_cap, T, D, R,
+                                isd, gamma1, att_out));
+  });
+  return check_launch("pair_att_kernel");
 }
 
 }  // namespace agb

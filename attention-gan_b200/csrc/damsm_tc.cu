@@ -35,6 +35,9 @@ int sent_cos_fwd_launch(const float* cnn, const float* rnn, int Bi, int Bc, int 
 int damsm_diag_att_maps(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
                         const int32_t* cap_lens, int Bi, int T, int D, int R, float gamma1, int row_offset,
                         float* att_out, float* S, float* Bt, cudaStream_t st);
+int damsm_pair_att_maps(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                        const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap,
+                        int P, int T, int D, int R, float gamma1, float* att_out, cudaStream_t st);
 size_t damsm_fp32_workspace_bytes(int Bi, int Bc, int T, int D, int R);
 int damsm_fp32_bwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
                    const int32_t* cap_lens, int Bi, int Bc, int T, int D, int R, float gamma1, float gamma2,
@@ -194,83 +197,114 @@ __global__ void pack_img_kernel_tc(const float* __restrict__ img, T16* __restric
 }
 
 // ---------------------------------------------------------------------------------------------
-// candidate packing (agb_damsm_cand_fwd): image b's K candidate captions become the virtual captions
-// v = b*K + k, packed by the rule of tile_pack_kernel into units of U rows (U = 64 in split precision) that
-// never mix two images; every image is padded to whole tiles.  An item of the pair kernels is one unit.
-// A candidate index outside [0, Bc) becomes an entry of length 0, whose m the pair kernel writes as NaN.
+// candidate packing (agb_damsm_cand_fwd, agb_damsm_pairs_fwd): every image owns a range of entries (virtual
+// captions), [b*K, (b+1)*K) for K candidates per image or CSR offsets eoff[b] .. eoff[b+1] for a pair list grouped
+// by image.  The entries are packed by the rule of tile_pack_kernel into units of U rows (U = 64 in split
+// precision) that never mix two images.  An image's range is cut into segments of S entries counted from its first
+// entry (S = 64 units of the widest captions, see make_plan), and every segment is padded to whole tiles.  An item
+// of the pair kernels is one unit.  An entry whose caption index is outside [0, Bc) becomes an entry of length 0,
+// whose m the pair kernel writes as NaN.
 // ---------------------------------------------------------------------------------------------
 // upper bound of one item's cost (kItemCost0 + per live caption its window and kItemCostCap, at most 128 captions
 // and 128 + 3 * 128 window rows): the host bounds the cost prefix of a call with it
 constexpr int kMaxItemCost = kItemCost0 + kTileN * (kItemCostCap + 4);
 
-// One warp per image, in lock-step (lane k % 32 loads entry k).  Pass 1 (!kWrite): the image's item count and
-// cost into img_items / img_cost.  Pass 2 (kWrite, after cand_scan_kernel turned them into exclusive prefixes):
-// cap_row, vlen of every entry, first entry / entry count / cost prefix of every item, image of every tile.
+__device__ __forceinline__ int ent_off(const int32_t* eoff, int K, int b) { return eoff ? eoff[b] : b * K; }
+
+// the image whose (non-empty) entry range holds entry g < number of entries
+__device__ __forceinline__ int ent_img(const int32_t* eoff, int K, int Bi, int g) {
+  if (!eoff) return g / K;
+  int lo = 0, hi = Bi - 1;                     // the last b with eoff[b] <= g
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (eoff[mid] <= g) lo = mid;
+    else hi = mid - 1;
+  }
+  return lo;
+}
+
+// One warp per window of S consecutive entries: it packs, in image order, every segment that starts inside the
+// window, in lock-step (lane k % 32 loads entry k of the segment).  A segment holds at most S entries, so no warp
+// walks more than 2 S entries however skewed the ranges are.  Pass 1 (!kWrite): the window's item count and cost
+// into win_items / win_cost.  Pass 2 (kWrite, after cand_scan_kernel turned them into exclusive prefixes): cap_row,
+// vlen of every entry, first entry / entry count / cost prefix of every item, image of every tile.  With K <= S
+// every image is one segment, and the layout is that of one warp per image.
 template <bool kWrite>
 __global__ void __launch_bounds__(256)
-cand_pack_kernel(const int32_t* __restrict__ cap_lens, int Bc, int T, const int32_t* __restrict__ cand, int Bi, int K,
-                 int U, int32_t* __restrict__ img_items, int32_t* __restrict__ img_cost, int32_t* __restrict__ cap_row,
+cand_pack_kernel(const int32_t* __restrict__ cap_lens, int Bc, int T, const int32_t* __restrict__ cand,
+                 const int32_t* __restrict__ eoff, int Bi, int K, int nwin, int S, int U,
+                 int32_t* __restrict__ win_items, int32_t* __restrict__ win_cost, int32_t* __restrict__ cap_row,
                  int32_t* __restrict__ vlen, int32_t* __restrict__ item_first, int32_t* __restrict__ item_ncap,
                  int32_t* __restrict__ cpre, int32_t* __restrict__ tile_img) {
-  const int b = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-  if (b >= Bi) return;
+  const int w = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (w >= nwin) return;
+  const int nent = ent_off(eoff, K, Bi);
+  const long long g0 = (long long)w * S, g1 = min((long long)nent, g0 + S);
   const int upt = kTileN / U;
-  const int v0 = b * K;
-  const int item0 = kWrite ? img_items[b] : 0, cost0 = kWrite ? img_cost[b] : 0;
-  int row = 0, unit = 0, first = 0, cost = kItemCost0, cacc = 0;
-  auto close_unit = [&](int next_first) {
-    if (kWrite && lane == 0) {
-      const int it = item0 + unit;
-      item_first[it] = v0 + first;
-      item_ncap[it] = next_first - first;
-      cpre[it] = cost0 + cacc;
-      if (it % upt == 0) tile_img[it / upt] = b;
-    }
-    cacc += cost;
-    cost = kItemCost0;
-    ++unit;
-    first = next_first;
-    row = 0;
-  };
-  for (int k0 = 0; k0 < K; k0 += 32) {
-    int myL = 0;
-    if (k0 + lane < K) {
-      const int j = cand[(size_t)v0 + k0 + lane];
-      myL = (j >= 0 && j < Bc) ? min(max(cap_lens[j], 0), T) : 0;
-    }
-    const int n = min(32, K - k0);
-    for (int i = 0; i < n; ++i) {
-      const int k = k0 + i, L = __shfl_sync(0xffffffffu, myL, i);
-      if (row + ((L + 3) & ~3) > U || k - first == U) close_unit(k);
-      if (kWrite && lane == i) {
-        cap_row[v0 + k] = (item0 + unit) * U + row;
-        vlen[v0 + k] = L;
+  const int item0 = kWrite ? win_items[w] : 0, cost0 = kWrite ? win_cost[w] : 0;
+  int unit = 0, cacc = 0;
+  for (long long g = g0; g < g1;) {
+    const int b = ent_img(eoff, K, Bi, (int)g);
+    const int e0 = ent_off(eoff, K, b), e1 = ent_off(eoff, K, b + 1);
+    const long long s0 = e0 + (g - e0 + S - 1) / S * S;   // image b's first segment start at or after g
+    g = e1;
+    if (s0 >= g1 || s0 >= e1) continue;          // no segment of image b starts in this window
+    const int v0 = (int)s0, cnt = (int)(min((long long)e1, s0 + S) - s0);
+    int row = 0, first = 0, cost = kItemCost0;
+    auto close_unit = [&](int next_first) {
+      if (kWrite && lane == 0) {
+        const int it = item0 + unit;
+        item_first[it] = v0 + first;
+        item_ncap[it] = next_first - first;
+        cpre[it] = cost0 + cacc;
+        if (it % upt == 0) tile_img[it / upt] = b;
       }
-      row += L;
-      if (L > 0) cost += ((L + 3) & ~3) + kItemCostCap;
+      cacc += cost;
+      cost = kItemCost0;
+      ++unit;
+      first = next_first;
+      row = 0;
+    };
+    for (int k0 = 0; k0 < cnt; k0 += 32) {
+      int myL = 0;
+      if (k0 + lane < cnt) {
+        const int j = cand[(size_t)v0 + k0 + lane];
+        myL = (j >= 0 && j < Bc) ? min(max(cap_lens[j], 0), T) : 0;
+      }
+      const int n = min(32, cnt - k0);
+      for (int i = 0; i < n; ++i) {
+        const int k = k0 + i, L = __shfl_sync(0xffffffffu, myL, i);
+        if (row + ((L + 3) & ~3) > U || k - first == U) close_unit(k);
+        if (kWrite && lane == i) {
+          cap_row[v0 + k] = (item0 + unit) * U + row;
+          vlen[v0 + k] = L;
+        }
+        row += L;
+        if (L > 0) cost += ((L + 3) & ~3) + kItemCostCap;
+      }
     }
+    close_unit(cnt);
+    while (unit % upt != 0) close_unit(cnt);   // pad the segment to whole tiles with empty units
   }
-  close_unit(K);
-  while (unit % upt != 0) close_unit(K);       // pad the image to whole tiles with empty units
   if (!kWrite && lane == 0) {
-    img_items[b] = unit;
-    img_cost[b] = cacc;
+    win_items[w] = unit;
+    win_cost[w] = cacc;
   }
 }
 
-// exclusive prefix over the images of their item counts and costs (one block); the totals give the number of
+// exclusive prefix over the windows of their item counts and costs (one block); the totals give the number of
 // tiles / units and the end of the cost prefix
 __global__ void __launch_bounds__(1024)
-cand_scan_kernel(int32_t* __restrict__ img_items, int32_t* __restrict__ img_cost, int Bi, int upt,
+cand_scan_kernel(int32_t* __restrict__ win_items, int32_t* __restrict__ win_cost, int n, int upt,
                  int32_t* __restrict__ cpre, int32_t* __restrict__ ntiles, int32_t* __restrict__ nunits) {
   __shared__ int si[1024], sc[1024];
   const int tid = threadIdx.x;
-  const int per = (Bi + 1023) / 1024;
-  const int lo = min(Bi, tid * per), hi = min(Bi, lo + per);
+  const int per = (n + 1023) / 1024;
+  const int lo = min(n, tid * per), hi = min(n, lo + per);
   int a = 0, c = 0;
   for (int b = lo; b < hi; ++b) {
-    a += img_items[b];
-    c += img_cost[b];
+    a += win_items[b];
+    c += win_cost[b];
   }
   si[tid] = a;
   sc[tid] = c;
@@ -284,9 +318,9 @@ cand_scan_kernel(int32_t* __restrict__ img_items, int32_t* __restrict__ img_cost
   }
   int ra = si[tid] - a, rc = sc[tid] - c;
   for (int b = lo; b < hi; ++b) {
-    const int x = img_items[b], y = img_cost[b];
-    img_items[b] = ra;
-    img_cost[b] = rc;
+    const int x = win_items[b], y = win_cost[b];
+    win_items[b] = ra;
+    win_cost[b] = rc;
     ra += x;
     rc += y;
   }
@@ -356,6 +390,130 @@ cand_rows_kernel(const float* __restrict__ words, int64_t ws_b, int64_t ws_d, in
     for (int w = 0; w < 4; ++w) tot += red[threadIdx.x][w];
     pn[(size_t)tile * kTileN + threadIdx.x] = sqrtf(tot);
   }
+}
+
+// ---------------------------------------------------------------------------------------------
+// pair lists (agb_damsm_pairs_fwd): the pairs are grouped by image with a stable counting sort on the image index,
+// as a least-significant-digit radix sort over two 8-bit digits.  Each pass is a per-block digit histogram, one
+// exclusive scan over (digit, block), and a stable scatter.  A pair whose image is outside [0, Bi) gets key 0xffff
+// (Bi <= 65535 keeps it free), which sorts after every image and is not packed.  Integer counts only: the order is
+// deterministic, and inside an image the pairs keep their list order.
+// ---------------------------------------------------------------------------------------------
+constexpr int kSortTile = 2048;                // pairs per block of a sort pass (8 per thread)
+
+__device__ __forceinline__ int pair_key(const int32_t* __restrict__ pair_img, int Bi, long long p) {
+  const int b = pair_img[p];
+  return (b >= 0 && b < Bi) ? b : 0xffff;
+}
+
+// digit counts of one block's pairs: hist[digit * gridDim.x + block].  kin == nullptr: keys from pair_img
+__global__ void __launch_bounds__(256)
+pair_hist_kernel(const int32_t* __restrict__ pair_img, int Bi, const int32_t* __restrict__ kin, long long P, int shift,
+                 int32_t* __restrict__ hist) {
+  __shared__ int cnt[256];
+  cnt[threadIdx.x] = 0;
+  __syncthreads();
+  for (int i = threadIdx.x; i < kSortTile; i += 256) {
+    const long long p = (long long)blockIdx.x * kSortTile + i;
+    if (p < P) atomicAdd(&cnt[((kin ? kin[p] : pair_key(pair_img, Bi, p)) >> shift) & 255], 1);
+  }
+  __syncthreads();
+  hist[threadIdx.x * gridDim.x + blockIdx.x] = cnt[threadIdx.x];
+}
+
+// in-place exclusive prefix of n ints (one block)
+__global__ void __launch_bounds__(1024) excl_scan_kernel(int32_t* __restrict__ a, int n) {
+  __shared__ int s[1024];
+  const int tid = threadIdx.x;
+  const int per = (n + 1023) / 1024;
+  const int lo = min(n, tid * per), hi = min(n, lo + per);
+  int acc = 0;
+  for (int i = lo; i < hi; ++i) acc += a[i];
+  s[tid] = acc;
+  __syncthreads();
+  for (int o = 1; o < 1024; o <<= 1) {
+    const int pv = tid >= o ? s[tid - o] : 0;
+    __syncthreads();
+    s[tid] += pv;
+    __syncthreads();
+  }
+  int r = s[tid] - acc;
+  for (int i = lo; i < hi; ++i) {
+    const int x = a[i];
+    a[i] = r;
+    r += x;
+  }
+}
+
+// stable scatter of one block's pairs to their digit's slots: rounds of 256 pairs in list order; inside a round the
+// rank of a pair is its lane rank among the warp's pairs of the same digit plus the counts of the earlier warps.
+// kin == nullptr: keys from pair_img, values = pair indices
+__global__ void __launch_bounds__(256)
+pair_scatter_kernel(const int32_t* __restrict__ pair_img, int Bi, const int32_t* __restrict__ kin,
+                    const int32_t* __restrict__ vin, long long P, int shift, const int32_t* __restrict__ hist,
+                    int32_t* __restrict__ kout, int32_t* __restrict__ vout) {
+  __shared__ int base[256];
+  __shared__ int wcnt[8][256];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  base[threadIdx.x] = hist[threadIdx.x * gridDim.x + blockIdx.x];
+  for (int w = 0; w < 8; ++w) wcnt[w][threadIdx.x] = 0;
+  __syncthreads();
+  for (int r0 = 0; r0 < kSortTile; r0 += 256) {
+    const long long p = (long long)blockIdx.x * kSortTile + r0 + threadIdx.x;
+    const bool live = p < P;
+    int key = 0, val = 0, d = 256;
+    if (live) {
+      key = kin ? kin[p] : pair_key(pair_img, Bi, p);
+      val = kin ? vin[p] : (int)p;
+      d = (key >> shift) & 255;
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, d);
+    const int rank = __popc(peers & ((1u << lane) - 1u));
+    if (live && rank == 0) wcnt[warp][d] = __popc(peers);
+    __syncthreads();
+    if (live) {
+      int pos = base[d] + rank;
+      for (int w = 0; w < warp; ++w) pos += wcnt[w][d];
+      kout[pos] = key;
+      vout[pos] = val;
+    }
+    __syncthreads();
+    int tot = 0;
+    for (int w = 0; w < 8; ++w) {
+      tot += wcnt[w][threadIdx.x];
+      wcnt[w][threadIdx.x] = 0;
+    }
+    base[threadIdx.x] += tot;
+    __syncthreads();
+  }
+}
+
+// thread t <= Bi: eoff[t] = the first sorted pair of image t (eoff[Bi] = number of pairs with a valid image);
+// thread t < P: the caption index of sorted pair t
+__global__ void __launch_bounds__(256)
+pair_offsets_kernel(const int32_t* __restrict__ key, const int32_t* __restrict__ val,
+                    const int32_t* __restrict__ pair_cap, int P, int Bi, int32_t* __restrict__ eoff,
+                    int32_t* __restrict__ cap_sorted) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t <= Bi) {
+    int lo = 0, hi = P;                        // the first sorted position with key >= t
+    while (lo < hi) {
+      const int mid = (int)(((long long)lo + hi) >> 1);
+      if (key[mid] < t) lo = mid + 1;
+      else hi = mid;
+    }
+    eoff[t] = lo;
+  }
+  if (t < P) cap_sorted[t] = pair_cap[val[t]];
+}
+
+// m from packed (sorted) order back to list order; pairs with an invalid image get NaN
+__global__ void __launch_bounds__(256)
+pair_scatter_m_kernel(const float* __restrict__ m_sorted, const int32_t* __restrict__ val,
+                      const int32_t* __restrict__ eoff, int Bi, int P, float* __restrict__ m_out) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P) return;
+  m_out[val[i]] = i < eoff[Bi] ? m_sorted[i] : __int_as_float(0x7fc00000);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -658,25 +816,32 @@ static int launch_fwd(const Packed& pk, const int32_t* cap_lens, int Bi, int Bc,
 // candidate mode: workspace plan from shapes only (the caption lengths stay on the device)
 // ---------------------------------------------------------------------------------------------
 struct CandPlan {
-  int split;
-  long long items_max, nt_max;   // items: word tiles, or 64-row units in split precision
+  int split, S;                  // S: entries per packing segment (see cand_pack_kernel)
+  long long nent, nwin, items_max, nt_max, sort_blocks;   // items: word tiles, or 64-row units in split precision
   size_t off_Wh, off_Wl, off_pn, off_caprow, off_vlen, off_ifirst, off_incap, off_cpre, off_timg, off_iitems, off_icost,
       off_counts, off_Ct, off_Ck, off_Ctl, off_Ckl, total;
+  // pair lists only: sort buffers (keys, values: pass 1 -> A, pass 2 -> B), digit histogram, CSR offsets, the
+  // caption index of every sorted pair and m in sorted order
+  size_t off_keyA, off_valA, off_keyB, off_valB, off_hist, off_eoff, off_capS, off_mS;
 };
 
-static CandPlan make_cand_plan(int Bi, int K, int T, bool split) {
+// nent entries over Bi images, at most items_max items (units).  S = 64 units of the widest captions: an even
+// number of units, so that cutting a range into segments never needs more units than packing it whole (every
+// closed unit holds at least per_unit captions).
+static CandPlan make_plan(int Bi, long long nent, long long items_max, int T, bool split, bool pairs) {
   CandPlan p;
   p.split = split ? 1 : 0;
   const int U = split ? 64 : kTileN;
   const int window = (T + 3) & ~3;
-  const long long per_unit = U / window;       // captions that always fit in one unit
-  long long units = (K + per_unit - 1) / per_unit;
-  if (split) units += units & 1;               // whole tiles per image
-  p.items_max = (long long)Bi * units;
-  p.nt_max = split ? p.items_max / 2 : p.items_max;
+  p.S = 64 * (U / window);
+  p.nent = nent;
+  p.nwin = (nent + p.S - 1) / p.S;
+  p.items_max = items_max;
+  p.nt_max = split ? (p.items_max + 1) / 2 : p.items_max;
+  p.sort_blocks = pairs ? (nent + kSortTile - 1) / kSortTile : 0;
   size_t o = 0;
   auto take = [&](size_t bytes) { const size_t at = o; o = align_up(o + bytes, 1024); return at; };
-  const size_t nv = (size_t)Bi * K;
+  const size_t nv = (size_t)nent;
   p.off_Wh = take((size_t)p.nt_max * kTileN * kD * 2);
   p.off_Wl = split ? take((size_t)p.nt_max * kTileN * kD * 2) : 0;
   p.off_pn = take((size_t)p.nt_max * kTileN * 4);
@@ -686,15 +851,44 @@ static CandPlan make_cand_plan(int Bi, int K, int T, bool split) {
   p.off_incap = take((size_t)p.items_max * 4);
   p.off_cpre = take((size_t)(p.items_max + 1) * 4);
   p.off_timg = take((size_t)p.nt_max * 4);
-  p.off_iitems = take((size_t)Bi * 4);
-  p.off_icost = take((size_t)Bi * 4);
+  p.off_iitems = take((size_t)p.nwin * 4);
+  p.off_icost = take((size_t)p.nwin * 4);
   p.off_counts = take(256);
   p.off_Ct = take((size_t)Bi * kRRows * kD * 2);
   p.off_Ck = take((size_t)Bi * kD * kRCols * 2);
   p.off_Ctl = split ? take((size_t)Bi * kRRows * kD * 2) : 0;
   p.off_Ckl = split ? take((size_t)Bi * kD * kRCols * 2) : 0;
+  p.off_keyA = p.off_valA = p.off_keyB = p.off_valB = p.off_hist = p.off_eoff = p.off_capS = p.off_mS = 0;
+  if (pairs) {
+    p.off_keyA = take(nv * 4);
+    p.off_valA = take(nv * 4);
+    p.off_keyB = take(nv * 4);
+    p.off_valB = take(nv * 4);
+    p.off_hist = take((size_t)p.sort_blocks * 256 * 4);
+    p.off_eoff = take((size_t)(Bi + 1) * 4);
+    p.off_capS = take(nv * 4);
+    p.off_mS = take(nv * 4);
+  }
   p.total = o;
   return p;
+}
+
+// K candidates per image: at most ceil(K / per_unit) units per image (even in split precision)
+static CandPlan make_cand_plan(int Bi, int K, int T, bool split) {
+  const int U = split ? 64 : kTileN;
+  const long long per_unit = U / ((T + 3) & ~3);   // captions that always fit in one unit
+  long long units = (K + per_unit - 1) / per_unit;
+  if (split) units += units & 1;                   // whole tiles per image
+  return make_plan(Bi, (long long)Bi * K, (long long)Bi * units, T, split, false);
+}
+
+// P pairs: image b with n_b > 0 pairs takes at most ceil(n_b / per_unit) units plus one of tile padding in split
+// precision, so all of them at most ceil(P / per_unit) + (1 + split) * min(Bi, P)
+static CandPlan make_pairs_plan(int Bi, long long P, int T, bool split) {
+  const int U = split ? 64 : kTileN;
+  const long long per_unit = U / ((T + 3) & ~3);
+  const long long items = (P + per_unit - 1) / per_unit + (split ? 2 : 1) * std::min<long long>(Bi, P);
+  return make_plan(Bi, P, items, T, split, true);
 }
 
 // the cost prefix and the packed row indices are int32
@@ -702,10 +896,12 @@ static bool cand_plan_fits(const CandPlan& p) {
   return p.items_max * kMaxItemCost < (long long)INT32_MAX && p.nt_max * kTileN < (long long)INT32_MAX;
 }
 
+// cand: the caption index of every entry; eoff: CSR entry offsets of the images, or nullptr for K entries per image.
+// m_out[v] is written for every entry v.
 template <typename T16>
 static int run_cand(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
-                    const int32_t* cap_lens, int Bc, const int32_t* cand, int Bi, int K, int T, int R, float gamma1,
-                    float gamma2, float* m_out, char* ws, const CandPlan& pl, cudaStream_t st) {
+                    const int32_t* cap_lens, int Bc, const int32_t* cand, const int32_t* eoff, int Bi, int K, int T,
+                    int R, float gamma1, float gamma2, float* m_out, char* ws, const CandPlan& pl, cudaStream_t st) {
   const bool bf = std::is_same<T16, __nv_bfloat16>::value;
   const int U = pl.split ? 64 : kTileN;
   T16* Wh = (T16*)(ws + pl.off_Wh);
@@ -726,14 +922,15 @@ static int run_cand(const float* img, const float* words, int64_t ws_b, int64_t 
   T16* Ctl = pl.split ? (T16*)(ws + pl.off_Ctl) : nullptr;
   T16* Ckl = pl.split ? (T16*)(ws + pl.off_Ckl) : nullptr;
 
-  const int pack_blocks = cdiv(Bi, 8);
-  cand_pack_kernel<false><<<pack_blocks, 256, 0, st>>>(cap_lens, Bc, T, cand, Bi, K, U, iitems, icost, nullptr,
-                                                       nullptr, nullptr, nullptr, nullptr, nullptr);
+  const int nwin = (int)pl.nwin;
+  const int pack_blocks = cdiv(nwin, 8);
+  cand_pack_kernel<false><<<pack_blocks, 256, 0, st>>>(cap_lens, Bc, T, cand, eoff, Bi, K, nwin, pl.S, U, iitems,
+                                                       icost, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
   if (int rc = check_launch("cand_pack_kernel<false>")) return rc;
-  cand_scan_kernel<<<1, 1024, 0, st>>>(iitems, icost, Bi, kTileN / U, cpre, ntiles, nunits);
+  cand_scan_kernel<<<1, 1024, 0, st>>>(iitems, icost, nwin, kTileN / U, cpre, ntiles, nunits);
   if (int rc = check_launch("cand_scan_kernel")) return rc;
-  cand_pack_kernel<true><<<pack_blocks, 256, 0, st>>>(cap_lens, Bc, T, cand, Bi, K, U, iitems, icost, cap_row, vlen,
-                                                      ifirst, incap, cpre, timg);
+  cand_pack_kernel<true><<<pack_blocks, 256, 0, st>>>(cap_lens, Bc, T, cand, eoff, Bi, K, nwin, pl.S, U, iitems, icost,
+                                                      cap_row, vlen, ifirst, incap, cpre, timg);
   if (int rc = check_launch("cand_pack_kernel<true>")) return rc;
   cand_rows_kernel<T16><<<(unsigned)pl.nt_max, 512, 0, st>>>(words, ws_b, ws_d, ws_t, cand, vlen, cap_row, ifirst, incap,
                                                              U, ntiles, Wh, Wl, pn);
@@ -786,6 +983,43 @@ static int run_cand(const float* img, const float* words, int64_t ws_b, int64_t 
   kern<<<grid, kThreads, kSmemBytes2, st>>>(mapW, mapCt, mapCk, p);
   prof_end(slot, st);
   return check_launch("damsm_fwd2_kernel<cand>");
+}
+
+// pair lists: group the pairs by image (two radix passes), CSR offsets, then the candidate pipeline over the
+// sorted pairs and a scatter of m back to list order
+template <typename T16>
+static int run_pairs(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                     const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap, int P,
+                     int T, int R, float gamma1, float gamma2, float* m_out, char* ws, const CandPlan& pl,
+                     cudaStream_t st) {
+  int32_t* keyA = (int32_t*)(ws + pl.off_keyA);
+  int32_t* valA = (int32_t*)(ws + pl.off_valA);
+  int32_t* keyB = (int32_t*)(ws + pl.off_keyB);
+  int32_t* valB = (int32_t*)(ws + pl.off_valB);
+  int32_t* hist = (int32_t*)(ws + pl.off_hist);
+  int32_t* eoff = (int32_t*)(ws + pl.off_eoff);
+  int32_t* capS = (int32_t*)(ws + pl.off_capS);
+  float* mS = (float*)(ws + pl.off_mS);
+  const unsigned G = (unsigned)pl.sort_blocks;
+  for (int pass = 0; pass < 2; ++pass) {
+    const int32_t* kin = pass ? keyA : nullptr;
+    const int32_t* vin = pass ? valA : nullptr;
+    int32_t* kout = pass ? keyB : keyA;
+    int32_t* vout = pass ? valB : valA;
+    pair_hist_kernel<<<G, 256, 0, st>>>(pair_img, Bi, kin, P, 8 * pass, hist);
+    if (int rc = check_launch("pair_hist_kernel")) return rc;
+    excl_scan_kernel<<<1, 1024, 0, st>>>(hist, (int)(256 * G));
+    if (int rc = check_launch("excl_scan_kernel")) return rc;
+    pair_scatter_kernel<<<G, 256, 0, st>>>(pair_img, Bi, kin, vin, P, 8 * pass, hist, kout, vout);
+    if (int rc = check_launch("pair_scatter_kernel")) return rc;
+  }
+  pair_offsets_kernel<<<(unsigned)((std::max(P, Bi + 1) + 255LL) / 256), 256, 0, st>>>(keyB, valB, pair_cap, P, Bi, eoff, capS);
+  if (int rc = check_launch("pair_offsets_kernel")) return rc;
+  if (int rc = run_cand<T16>(img, words, ws_b, ws_d, ws_t, cap_lens, Bc, capS, eoff, Bi, 0, T, R, gamma1, gamma2, mS,
+                             ws, pl, st))
+    return rc;
+  pair_scatter_m_kernel<<<(unsigned)((P + 255LL) / 256), 256, 0, st>>>(mS, valB, eoff, Bi, P, m_out);
+  return check_launch("pair_scatter_m_kernel");
 }
 
 #include "damsm_tc_bwd2.inc"
@@ -862,10 +1096,59 @@ int damsm_tc_cand_fwd(const float* img, const float* words, int64_t ws_b, int64_
     return AGB_E_WORKSPACE;
   }
   if (math == AGB_MATH_TC_BF16)
-    return tc::run_cand<__nv_bfloat16>(img, words, ws_b, ws_d, ws_t, cap_lens, Bc, cand, Bi, K, T, R, gamma1, gamma2,
-                                       m_out, (char*)workspace, pl, st);
-  return tc::run_cand<__half>(img, words, ws_b, ws_d, ws_t, cap_lens, Bc, cand, Bi, K, T, R, gamma1, gamma2, m_out,
-                              (char*)workspace, pl, st);
+    return tc::run_cand<__nv_bfloat16>(img, words, ws_b, ws_d, ws_t, cap_lens, Bc, cand, nullptr, Bi, K, T, R, gamma1,
+                                       gamma2, m_out, (char*)workspace, pl, st);
+  return tc::run_cand<__half>(img, words, ws_b, ws_d, ws_t, cap_lens, Bc, cand, nullptr, Bi, K, T, R, gamma1, gamma2,
+                              m_out, (char*)workspace, pl, st);
+}
+
+// 0 when the shapes are outside the pair path's range (the caller has checked T, D, R and math)
+size_t damsm_tc_pairs_workspace_bytes(int Bi, int Bc, long long P, int T, int math) {
+  if (Bi <= 0 || Bi > 65535 || Bc <= 0 || P < 0 || P >= (long long)INT32_MAX) return 0;
+  const tc::CandPlan pl = tc::make_pairs_plan(Bi, P, T, math == AGB_MATH_TC_F16X2);
+  return tc::cand_plan_fits(pl) ? pl.total : 0;
+}
+
+int damsm_tc_pairs_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                       const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap,
+                       long long P, int T, int D, int R, float gamma1, float gamma2, float* m_out, float* att_out,
+                       void* workspace, size_t workspace_bytes, int math, cudaStream_t st) {
+  if (Bc <= 0 || Bi <= 0 || P < 0) return fail_arg("non-positive size");
+  if (Bi > 65535) return fail_unsupported("Bi=%d > 65535", Bi);
+  if (P >= (long long)INT32_MAX) return fail_unsupported("P=%lld >= 2^31", P);
+  if (math != AGB_MATH_TC_BF16 && gamma1 > 11.f) return fail_unsupported("gamma1=%g overflows fp16 (use bf16 math)", gamma1);
+  const tc::CandPlan pl = tc::make_pairs_plan(Bi, P, T, math == AGB_MATH_TC_F16X2);
+  if (!tc::cand_plan_fits(pl)) return fail_unsupported("Bi=%d P=%lld: %lld word tiles exceed the int32 cost prefix", Bi, P, pl.nt_max);
+  if (P == 0) return 0;
+  if (workspace_bytes < pl.total) {
+    set_error("workspace too small: %zu < %zu", workspace_bytes, pl.total);
+    return AGB_E_WORKSPACE;
+  }
+  int rc;
+  // the pair maps only read the caller's inputs: they run on a forked stream beside the grouping, the pack
+  // kernels and the pair kernel, as agb_damsm_fwd runs its matched maps
+  tc::SideStream* side = nullptr;
+  int rc_side = 0;
+  if (att_out) {
+    if ((rc = tc::side_stream(&side))) return rc;
+    if ((rc = tc::side_fork(side, st))) return rc;
+    rc_side = damsm_pair_att_maps(img, words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, pair_img, pair_cap, (int)P, T, D, R,
+                                  gamma1, att_out, side->stream);
+  }
+  if (rc_side == 0) {
+    if (math == AGB_MATH_TC_BF16)
+      rc = tc::run_pairs<__nv_bfloat16>(img, words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, pair_img, pair_cap, (int)P, T,
+                                        R, gamma1, gamma2, m_out, (char*)workspace, pl, st);
+    else
+      rc = tc::run_pairs<__half>(img, words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, pair_img, pair_cap, (int)P, T, R,
+                                 gamma1, gamma2, m_out, (char*)workspace, pl, st);
+  } else {
+    rc = rc_side;
+  }
+  // joined on every path after the fork (an enclosing graph capture must not be left forked)
+  if (side)
+    if (int rj = tc::side_join(side, st)) return rc ? rc : rj;
+  return rc;
 }
 
 int damsm_tc_bwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,

@@ -92,7 +92,7 @@ int agb_tc_gemm_test(const void* A, const void* B, float* C, int M, int N, int K
  * tag: 1 = fp32 sgemm, 2 = tcgen05 DAMSM forward pair kernel, 3 = tcgen05 DAMSM backward pair kernel,
  *      4 = word-attention forward, 5 = word-attention backward (main kernel),
  *      6 = d img reduction GEMM (tcgen05), 7 = d words reduction GEMM (tcgen05),
- *      9 = candidate pair kernel of agb_damsm_cand_fwd (tcgen05).
+ *      9 = candidate pair kernel of agb_damsm_cand_fwd and agb_damsm_pairs_fwd (tcgen05).
  * agb_prof_read synchronises the recorded events and returns the summed duration and the count. */
 long long agb_launch_count(void);
 void agb_prof_enable(int on);
@@ -276,6 +276,35 @@ int agb_func_attention_bwd(const float* query, int64_t qs_b, int64_t qs_d, int64
                            const float* context, int B, int D, int L, int R, float gamma1,
                            int scaled, const float* dwc, const float* dattn, float* dquery,
                            float* dcontext, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * DAMSM word-region similarity of an arbitrary list of (image, caption) pairs (evaluation: text-to-image
+ * R-precision, hard-negative inspection, attention maps of chosen pairs)
+ *   m_out[p] = m(image pair_img[p], caption pair_cap[p]), bit for bit agb_damsm_fwd's m of that pair in the same math
+ *   img, words, cap_lens as in agb_damsm_cand_fwd
+ *   pair_img, pair_cap [P] int32: any order, duplicates allowed.  A pair whose image is outside [0,Bi), whose caption
+ *                      is outside [0,Bc) or whose caption has length 0 yields NaN (never a memory fault)
+ *   m_out    [P]       fp32
+ *   att_out  [P,T,R]   fp32 or NULL: beta of every pair (words_loss.py:63), the arithmetic of agb_damsm_fwd's matched
+ *                      att_out; rows t >= L are 0, every row of an invalid pair is NaN
+ *   The pairs are grouped by image on the device (stable counting sort: inside an image the list order is kept)
+ *   and scored by the kernels of agb_damsm_cand_fwd.  P = 0 is a successful no-op.
+ *   math: AGB_MATH_TC_F16 | AGB_MATH_TC_BF16 | AGB_MATH_TC_F16X2 (inference only: AGB_MATH_SAVE is rejected).
+ * Limits: the tensor-core range of agb_damsm_supported (D = 256, T <= 32, R <= 320), Bi <= 65535, P < 2^31 and at
+ * most 2^31 / 5508 work items; otherwise the workspace query returns 0 and the call AGB_E_UNSUPPORTED.  The
+ * workspace size depends on (Bi, Bc, P, T, math) only.  No host synchronisation, nothing allocated: capturable in
+ * a CUDA graph.
+ * ---------------------------------------------------------------------------------------------- */
+size_t agb_damsm_pairs_workspace_bytes(int Bi, int Bc, long long P, int T, int D, int R, int math);
+int agb_damsm_pairs_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                        const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap,
+                        long long P, int T, int D, int R, float gamma1, float gamma2, float* m_out, float* att_out,
+                        void* workspace, size_t workspace_bytes, int math, void* stream);
+
+/* sentence cosine of a pair list: scos_out[p] = the cosine (agb_sent_cos_fwd) of image pair_img[p] and caption pair_cap[p], bit for bit
+ *   agb_sent_cos_cand_fwd's value for that pair; NaN if either index is out of range.  P = 0 is a no-op, P < 2^31 */
+int agb_sent_cos_pairs_fwd(const float* cnn, const float* rnn, int Bi, int Bc, const int32_t* pair_img,
+                           const int32_t* pair_cap, long long P, int D, float eps, float* scos_out, void* stream);
 
 #ifdef __cplusplus
 }
