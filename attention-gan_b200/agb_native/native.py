@@ -54,6 +54,17 @@ SIGNATURES = {
     "agb_damsm_pairs_fwd": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int, c_void_p,
                                     c_void_p, ctypes.c_longlong, c_int, c_int, c_int, c_float, c_float, c_void_p,
                                     c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
+    "agb_damsm_pairs_train_workspace_bytes": (c_size_t, [c_int, c_int, ctypes.c_longlong, c_int, c_int, c_int,
+                                                         c_int]),
+    "agb_damsm_pairs_train_fwd": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int,
+                                          c_void_p, c_void_p, ctypes.c_longlong, c_int, c_int, c_int, c_float, c_float,
+                                          c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
+    "agb_damsm_pairs_bwd": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int, c_void_p,
+                                    c_void_p, ctypes.c_longlong, c_int, c_int, c_int, c_float, c_float, c_void_p,
+                                    c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
+    "agb_sent_cos_pairs_bwd_workspace_bytes": (c_size_t, [c_int, c_int, ctypes.c_longlong, c_int]),
+    "agb_sent_cos_pairs_bwd": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, ctypes.c_longlong, c_int,
+                                       c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "agb_sent_cos_fwd": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p]),
     "agb_sent_cos_pairs_fwd": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, ctypes.c_longlong, c_int,
                                        c_float, c_void_p, c_void_p]),

@@ -254,6 +254,99 @@ def sent_cos_pairs_fwd(cnn: torch.Tensor, rnn: torch.Tensor, pair_img: torch.Ten
     return scos
 
 
+def damsm_pairs_train_workspace_bytes(Bi: int, Bc: int, P: int, T: int, D: int, R: int, math: int) -> int:
+    """workspace of damsm_pairs_train_fwd / damsm_pairs_bwd; 0 when the shapes are outside the pair path's range"""
+    return int(N.lib().agb_damsm_pairs_train_workspace_bytes(Bi, Bc, P, T, D, R, math))
+
+
+def _pair_list(pair_img: torch.Tensor, pair_cap: torch.Tensor) -> int:
+    _pair_index(pair_img, "pair_img")
+    _pair_index(pair_cap, "pair_cap")
+    P = pair_img.shape[0]
+    if pair_cap.shape[0] != P:
+        raise RuntimeError(f"pair_img has {P} entries, pair_cap {pair_cap.shape[0]}")
+    return P
+
+
+def _pairs_train_ws(img, words, P: int, math: int, ws: Optional[torch.Tensor]) -> torch.Tensor:
+    Bi, D, R = img.shape
+    Bc, _, T = words.shape
+    nbytes = damsm_pairs_train_workspace_bytes(Bi, Bc, P, T, D, R, math)
+    if nbytes == 0:
+        raise N.NativeError(f"pair DAMSM shape Bi={Bi} Bc={Bc} P={P} T={T} D={D} R={R} is unsupported for math mode {math}")
+    if ws is None:
+        return _ws(nbytes, img.device)
+    if ws.numel() < nbytes:
+        raise RuntimeError(f"workspace of {ws.numel()} bytes is below the {nbytes} the pair list needs")
+    return ws
+
+
+def damsm_pairs_train_fwd(img: torch.Tensor, words: torch.Tensor, cap_lens: torch.Tensor, pair_img: torch.Tensor,
+                          pair_cap: torch.Tensor, gamma1: float, gamma2: float, math: int,
+                          ws: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The training forward of a pair list: the arguments of damsm_pairs_fwd without the maps.  Returns (m [P], ws):
+    m bit for bit damsm_pairs_fwd's, ws the workspace (of at least damsm_pairs_train_workspace_bytes, allocated here
+    when None) that damsm_pairs_bwd reads."""
+    require_cuda(img, words, cap_lens, pair_img, pair_cap)
+    Bi, D, R = img.shape
+    Bc, _, T = words.shape
+    P = _pair_list(pair_img, pair_cap)
+    ws = _pairs_train_ws(img, words, P, math, ws)
+    m = torch.empty((P,), dtype=torch.float32, device=img.device)
+    rc = N.lib().agb_damsm_pairs_train_fwd(_p(img), _p(words), words.stride(0), words.stride(1), words.stride(2),
+                                           _p(cap_lens), Bi, Bc, _p(pair_img), _p(pair_cap), P, T, D, R, gamma1,
+                                           gamma2, _p(m), _p(ws), ws.numel(), math, _stream(img))
+    N.check(rc, "agb_damsm_pairs_train_fwd")
+    return m, ws
+
+
+def damsm_pairs_bwd(img: torch.Tensor, words: torch.Tensor, cap_lens: torch.Tensor, pair_img: torch.Tensor,
+                    pair_cap: torch.Tensor, gamma1: float, gamma2: float, math: int, dm: torch.Tensor,
+                    ws: torch.Tensor, need_dwords: bool = True, need_dimg: bool = True
+                    ) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """dm [P] fp32 contiguous = dLoss/dm in list order, ws: the workspace of the matching damsm_pairs_train_fwd.
+    Returns (dimg [Bi,D,R] or None, dwords [Bc,T,D] word-major or None)."""
+    require_cuda(img, words, cap_lens, pair_img, pair_cap, dm, ws)
+    Bi, D, R = img.shape
+    Bc, _, T = words.shape
+    P = _pair_list(pair_img, pair_cap)
+    if dm.dtype != torch.float32 or dm.shape != (P,) or not dm.is_contiguous():
+        raise RuntimeError(f"dm must be a contiguous fp32 [{P}] tensor")
+    ws = _pairs_train_ws(img, words, P, math, ws)
+    dimg = torch.empty((Bi, D, R), dtype=torch.float32, device=img.device) if need_dimg else None
+    dwords = torch.empty((Bc, T, D), dtype=torch.float32, device=img.device) if need_dwords else None
+    rc = N.lib().agb_damsm_pairs_bwd(_p(img), _p(words), words.stride(0), words.stride(1), words.stride(2),
+                                     _p(cap_lens), Bi, Bc, _p(pair_img), _p(pair_cap), P, T, D, R, gamma1, gamma2,
+                                     _p(dm), _p(dimg), _p(dwords), _p(ws), ws.numel(), math, _stream(img))
+    N.check(rc, "agb_damsm_pairs_bwd")
+    return dimg, dwords
+
+
+def sent_cos_pairs_bwd_workspace_bytes(Bi: int, Bc: int, P: int, D: int) -> int:
+    return int(N.lib().agb_sent_cos_pairs_bwd_workspace_bytes(Bi, Bc, P, D))
+
+
+def sent_cos_pairs_bwd(cnn: torch.Tensor, rnn: torch.Tensor, pair_img: torch.Tensor, pair_cap: torch.Tensor,
+                       eps: float, dscos: torch.Tensor, need_dcnn: bool = True, need_drnn: bool = True):
+    """dscos [P] fp32 contiguous = dLoss/dcos in list order -> (dcnn [Bi,D] or None, drnn [Bc,D] or None)"""
+    require_cuda(cnn, rnn, pair_img, pair_cap, dscos)
+    Bi, D = cnn.shape
+    Bc = rnn.shape[0]
+    P = _pair_list(pair_img, pair_cap)
+    if dscos.dtype != torch.float32 or dscos.shape != (P,) or not dscos.is_contiguous():
+        raise RuntimeError(f"dscos must be a contiguous fp32 [{P}] tensor")
+    dcnn = torch.empty_like(cnn) if need_dcnn else None
+    drnn = torch.empty_like(rnn) if need_drnn else None
+    nbytes = sent_cos_pairs_bwd_workspace_bytes(Bi, Bc, P, D)
+    if nbytes == 0:
+        raise N.NativeError(f"sentence pair shape Bi={Bi} Bc={Bc} P={P} D={D} is unsupported")
+    ws = _ws(nbytes, cnn.device)
+    rc = N.lib().agb_sent_cos_pairs_bwd(_p(cnn), _p(rnn), Bi, Bc, _p(pair_img), _p(pair_cap), P, D, eps, _p(dscos),
+                                        _p(dcnn), _p(drnn), _p(ws), ws.numel(), _stream(cnn))
+    N.check(rc, "agb_sent_cos_pairs_bwd")
+    return dcnn, drnn
+
+
 def contrastive(raw: torch.Tensor, class_ids: Optional[torch.Tensor], labels: torch.Tensor, gamma3: float,
                 lam: float, row_begin: int, row_count: int, want_grad: bool = True):
     """raw [B,B] fp32 (all rows), class_ids [B] int32 or None, labels [B] int64.

@@ -367,6 +367,119 @@ def _(cnn, rnn, pair_img, pair_cap, eps):
     return cnn.new_empty((pair_img.shape[0],), dtype=torch.float32)
 
 
+# the differentiable pair scores (losses/pair_scores.py): the training forward returns its workspace, which the
+# backward reads and overwrites with its staging
+@_op("damsm_pairs_train_fwd")
+def damsm_pairs_train_fwd(img: Tensor, words: Tensor, cap_lens: Tensor, pair_img: Tensor, pair_cap: Tensor,
+                          gamma1: float, gamma2: float, math: int) -> Tuple[Tensor, Tensor]:
+    """(m [P], ws uint8) of the pair list (ops.damsm_pairs_train_fwd)"""
+    return ops.damsm_pairs_train_fwd(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math)
+
+
+@damsm_pairs_train_fwd.register_fake
+def _(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math):
+    Bi, D, R = img.shape
+    Bc, _, T = words.shape
+    P = pair_img.shape[0]
+    if pair_cap.shape[0] != P:
+        raise RuntimeError(f"pair_img has {P} entries, pair_cap {pair_cap.shape[0]}")
+    nbytes = int(N.lib().agb_damsm_pairs_train_workspace_bytes(Bi, Bc, P, T, D, R, math))
+    if nbytes == 0:
+        raise N.NativeError(f"pair DAMSM shape Bi={Bi} Bc={Bc} P={P} T={T} D={D} R={R} is unsupported for math mode {math}")
+    return img.new_empty((P,), dtype=torch.float32), _ws_like(nbytes, img)
+
+
+@_op("damsm_pairs_bwd", mutates_args=("ws",))
+def damsm_pairs_bwd(img: Tensor, words: Tensor, cap_lens: Tensor, pair_img: Tensor, pair_cap: Tensor, gamma1: float,
+                    gamma2: float, math: int, dm: Tensor, ws: Tensor, need_dimg: bool,
+                    need_dwords: bool) -> Tuple[Tensor, Tensor]:
+    """(dimg [Bi,D,R] or empty, dwords [Bc,T,D] word-major or empty) from the workspace damsm_pairs_train_fwd
+    returned"""
+    dimg, dwords = ops.damsm_pairs_bwd(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math, dm, ws,
+                                       need_dwords, need_dimg)
+    return _none(dimg, img.device), _none(dwords, img.device)
+
+
+@damsm_pairs_bwd.register_fake
+def _(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math, dm, ws, need_dimg, need_dwords):
+    Bc, D, T = words.shape
+    e = img.new_empty((0,), dtype=torch.float32)
+    return (torch.empty_like(img) if need_dimg else e), (img.new_empty((Bc, T, D)) if need_dwords else e.clone())
+
+
+def _damsm_pairs_setup(ctx, inputs, output):
+    img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math = inputs
+    ctx.save_for_backward(img, words, cap_lens, pair_img, pair_cap)
+    ctx.ws = output[1]
+    ctx.cfg = (gamma1, gamma2, math)
+    ctx.mark_non_differentiable(output[1])
+    ctx.set_materialize_grads(False)
+
+
+def _damsm_pairs_backward(ctx, dm, _dws):
+    img, words, cap_lens, pair_img, pair_cap = ctx.saved_tensors
+    gamma1, gamma2, math = ctx.cfg
+    need_img, need_words = ctx.needs_input_grad[:2]
+    dimg = dwords = None
+    if dm is not None and (need_img or need_words):
+        if ctx.ws is None:
+            raise RuntimeError("agb::damsm_pairs_train_fwd: a second backward is not supported (the first one "
+                               "released the training workspace)")
+        di, dw = torch.ops.agb.damsm_pairs_bwd(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math,
+                                               dm.contiguous(), ctx.ws, need_img, need_words)
+        dimg = di if need_img else None
+        dwords = dw.transpose(1, 2) if need_words else None           # [Bc,D,T] view like words
+    ctx.ws = None
+    return dimg, dwords, None, None, None, None, None, None
+
+
+damsm_pairs_train_fwd.register_autograd(_damsm_pairs_backward, setup_context=_damsm_pairs_setup)
+
+
+@_op("sent_cos_pairs_train_fwd")
+def sent_cos_pairs_train_fwd(cnn: Tensor, rnn: Tensor, pair_img: Tensor, pair_cap: Tensor, eps: float) -> Tensor:
+    """cosine [P] of the pair list, the values of sent_cos_pairs_fwd, with a registered backward"""
+    return ops.sent_cos_pairs_fwd(cnn, rnn, pair_img, pair_cap, eps)
+
+
+@sent_cos_pairs_train_fwd.register_fake
+def _(cnn, rnn, pair_img, pair_cap, eps):
+    if pair_cap.shape[0] != pair_img.shape[0]:
+        raise RuntimeError(f"pair_img has {pair_img.shape[0]} entries, pair_cap {pair_cap.shape[0]}")
+    return cnn.new_empty((pair_img.shape[0],), dtype=torch.float32)
+
+
+@_op("sent_cos_pairs_bwd")
+def sent_cos_pairs_bwd(cnn: Tensor, rnn: Tensor, pair_img: Tensor, pair_cap: Tensor, eps: float, dscos: Tensor,
+                       need_dcnn: bool, need_drnn: bool) -> Tuple[Tensor, Tensor]:
+    """(dcnn or empty, drnn or empty)"""
+    dcnn, drnn = ops.sent_cos_pairs_bwd(cnn, rnn, pair_img, pair_cap, eps, dscos, need_dcnn, need_drnn)
+    return _none(dcnn, cnn.device), _none(drnn, cnn.device)
+
+
+@sent_cos_pairs_bwd.register_fake
+def _(cnn, rnn, pair_img, pair_cap, eps, dscos, need_dcnn, need_drnn):
+    e = cnn.new_empty((0,), dtype=torch.float32)
+    return (torch.empty_like(cnn) if need_dcnn else e), (torch.empty_like(rnn) if need_drnn else e.clone())
+
+
+def _sent_cos_pairs_setup(ctx, inputs, output):
+    cnn, rnn, pair_img, pair_cap, eps = inputs
+    ctx.save_for_backward(cnn, rnn, pair_img, pair_cap)
+    ctx.eps = eps
+
+
+def _sent_cos_pairs_backward(ctx, dscos):
+    cnn, rnn, pair_img, pair_cap = ctx.saved_tensors
+    need_c, need_r = ctx.needs_input_grad[:2]
+    dc, dr = torch.ops.agb.sent_cos_pairs_bwd(cnn, rnn, pair_img, pair_cap, ctx.eps, dscos.contiguous(), need_c,
+                                              need_r)
+    return (dc if need_c else None), (dr if need_r else None), None, None, None
+
+
+sent_cos_pairs_train_fwd.register_autograd(_sent_cos_pairs_backward, setup_context=_sent_cos_pairs_setup)
+
+
 # ------------------------------------------------------------------------------------------------
 # functional region-word attention
 # ------------------------------------------------------------------------------------------------
@@ -479,3 +592,5 @@ OPS = ("word_attn_fwd", "word_attn_cat", "word_attn_bwd", "damsm_fwd", "damsm_bw
        "damsm_cand_fwd", "sent_cos_cand_fwd")
 # the pair-list scorers of the evaluation path (DAMSMScorer.words_pairs / sentence_pairs)
 PAIR_OPS = ("damsm_pairs_fwd", "sent_cos_pairs_fwd")
+# the differentiable pair scores (losses/pair_scores.py)
+PAIR_TRAIN_OPS = ("damsm_pairs_train_fwd", "damsm_pairs_bwd", "sent_cos_pairs_train_fwd", "sent_cos_pairs_bwd")

@@ -31,6 +31,18 @@ int damsm_tc_cand_fwd(const float* img, const float* words, int64_t ws_b, int64_
                       const int32_t* cap_lens, int Bc, const int32_t* cand, int Bi, int K, int T, int R, float gamma1,
                       float gamma2, float* m_out, void* workspace, size_t workspace_bytes, int math, cudaStream_t st);
 size_t damsm_tc_pairs_workspace_bytes(int Bi, int Bc, long long P, int T, int math);
+size_t damsm_tc_pairs_train_workspace_bytes(int Bi, int Bc, long long P, int T, int math);
+int damsm_tc_pairs_train_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                             const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap,
+                             long long P, int T, int R, float gamma1, float gamma2, float* m_out, void* workspace,
+                             size_t workspace_bytes, int math, cudaStream_t st);
+int damsm_tc_pairs_bwd(const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t, const int32_t* cap_lens, int Bi,
+                       int Bc, long long P, int T, int R, float gamma1, float gamma2, const float* dm, float* dimg,
+                       float* dwords, void* workspace, size_t workspace_bytes, int math, cudaStream_t st);
+size_t sent_cos_pairs_bwd_workspace_bytes(int Bi, int Bc, long long P);
+int sent_cos_pairs_bwd(const float* cnn, const float* rnn, int Bi, int Bc, const int32_t* pair_img,
+                       const int32_t* pair_cap, long long P, int D, float eps, const float* dscos, float* dcnn,
+                       float* drnn, void* workspace, size_t workspace_bytes, cudaStream_t st);
 int damsm_tc_pairs_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
                        const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap,
                        long long P, int T, int D, int R, float gamma1, float gamma2, float* m_out, float* att_out,
@@ -164,6 +176,70 @@ extern "C" int agb_damsm_pairs_fwd(const float* img, const float* words, int64_t
 #ifdef AGB_WITH_TC
   return damsm_tc_pairs_fwd(img, words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, pair_img, pair_cap, P, T, D, R, gamma1,
                             gamma2, m_out, att_out, workspace, workspace_bytes, math, (cudaStream_t)stream);
+#else
+  return fail_unsupported("library built without the tcgen05 kernels");
+#endif
+}
+
+extern "C" size_t agb_damsm_pairs_train_workspace_bytes(int Bi, int Bc, long long P, int T, int D, int R, int math) {
+  if (!cand_math_ok(math) || !agb_damsm_supported(T, D, R, math)) return 0;
+#ifdef AGB_WITH_TC
+  return damsm_tc_pairs_train_workspace_bytes(Bi, Bc, P, T, math);
+#else
+  return 0;
+#endif
+}
+
+extern "C" int agb_damsm_pairs_train_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                                         const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img,
+                                         const int32_t* pair_cap, long long P, int T, int D, int R, float gamma1,
+                                         float gamma2, float* m_out, void* workspace, size_t workspace_bytes, int math,
+                                         void* stream) {
+  if (!cand_math_ok(math)) return fail_unsupported("math=%d: pair training needs a tensor-core mode", math);
+  if (!agb_damsm_supported(T, D, R, math)) return fail_unsupported("T=%d D=%d R=%d math=%d is outside the compiled range", T, D, R, math);
+  if (P > 0 && (!img || !words || !cap_lens || !pair_img || !pair_cap || !m_out || !workspace))
+    return fail_arg("null pointer");
+#ifdef AGB_WITH_TC
+  return damsm_tc_pairs_train_fwd(img, words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, pair_img, pair_cap, P, T, R, gamma1,
+                                  gamma2, m_out, workspace, workspace_bytes, math, (cudaStream_t)stream);
+#else
+  return fail_unsupported("library built without the tcgen05 kernels");
+#endif
+}
+
+extern "C" int agb_damsm_pairs_bwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                                   const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img,
+                                   const int32_t* pair_cap, long long P, int T, int D, int R, float gamma1, float gamma2,
+                                   const float* dm, float* dimg, float* dwords, void* workspace,
+                                   size_t workspace_bytes, int math, void* stream) {
+  if (!cand_math_ok(math)) return fail_unsupported("math=%d: pair training needs a tensor-core mode", math);
+  if (!agb_damsm_supported(T, D, R, math)) return fail_unsupported("T=%d D=%d R=%d math=%d is outside the compiled range", T, D, R, math);
+  if (P > 0 && (!img || !words || !cap_lens || !pair_img || !pair_cap || !dm || !workspace))
+    return fail_arg("null pointer");
+#ifdef AGB_WITH_TC
+  return damsm_tc_pairs_bwd(words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, P, T, R, gamma1, gamma2, dm, dimg, dwords,
+                            workspace, workspace_bytes, math, (cudaStream_t)stream);
+#else
+  return fail_unsupported("library built without the tcgen05 kernels");
+#endif
+}
+
+extern "C" size_t agb_sent_cos_pairs_bwd_workspace_bytes(int Bi, int Bc, long long P, int D) {
+  if (D <= 0) return 0;
+#ifdef AGB_WITH_TC
+  return sent_cos_pairs_bwd_workspace_bytes(Bi, Bc, P);
+#else
+  return 0;
+#endif
+}
+
+extern "C" int agb_sent_cos_pairs_bwd(const float* cnn, const float* rnn, int Bi, int Bc, const int32_t* pair_img,
+                                      const int32_t* pair_cap, long long P, int D, float eps, const float* dscos,
+                                      float* dcnn, float* drnn, void* workspace, size_t workspace_bytes, void* stream) {
+  if (P > 0 && (!cnn || !rnn || !pair_img || !pair_cap || !dscos || !workspace)) return fail_arg("null pointer");
+#ifdef AGB_WITH_TC
+  return sent_cos_pairs_bwd(cnn, rnn, Bi, Bc, pair_img, pair_cap, P, D, eps, dscos, dcnn, drnn, workspace,
+                            workspace_bytes, (cudaStream_t)stream);
 #else
   return fail_unsupported("library built without the tcgen05 kernels");
 #endif

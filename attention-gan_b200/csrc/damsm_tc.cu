@@ -26,7 +26,7 @@
 #include <algorithm>
 #include <type_traits>
 
-#include "tc_common.cuh"
+#include "tc_gemm_pairs.cuh"
 
 namespace agb {
 
@@ -897,11 +897,13 @@ static bool cand_plan_fits(const CandPlan& p) {
 }
 
 // cand: the caption index of every entry; eoff: CSR entry offsets of the images, or nullptr for K entries per image.
-// m_out[v] is written for every entry v.
+// m_out[v] is written for every entry v.  v16 / rowst != nullptr (pair training forward): the pair kernels also save
+// the normalised context vectors and row statistics of every packed word row for agb_damsm_pairs_bwd.
 template <typename T16>
 static int run_cand(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
                     const int32_t* cap_lens, int Bc, const int32_t* cand, const int32_t* eoff, int Bi, int K, int T,
-                    int R, float gamma1, float gamma2, float* m_out, char* ws, const CandPlan& pl, cudaStream_t st) {
+                    int R, float gamma1, float gamma2, float* m_out, char* ws, const CandPlan& pl, cudaStream_t st,
+                    void* v16 = nullptr, float4* rowst = nullptr) {
   const bool bf = std::is_same<T16, __nv_bfloat16>::value;
   const int U = pl.split ? 64 : kTileN;
   T16* Wh = (T16*)(ws + pl.off_Wh);
@@ -948,7 +950,7 @@ static int run_cand(const float* img, const float* words, int64_t ws_b, int64_t 
   p.scale_log2 = kLog2e / sqrtf((float)kD);
   p.g1_log2 = gamma1 * kLog2e;
   p.gamma2 = gamma2;
-  p.v16 = nullptr; p.rowst = nullptr; p.Ntot = 0;
+  p.v16 = v16; p.rowst = rowst; p.Ntot = 0;
   p.tile_img = timg;
   p.wh = Wh;
   const int grid = (int)std::min<long long>(num_sms(), pl.items_max);
@@ -965,7 +967,7 @@ static int run_cand(const float* img, const float* words, int64_t ws_b, int64_t 
       FwdXCandParams xp;
       xp.f = p; xp.unit_first = ifirst; xp.unit_ncap = incap; xp.nunits = nunits;
       xp.tile_img = timg; xp.wh = Wh; xp.wl = Wl;
-      auto kx = damsm_fwd2x_kernel<false, true>;
+      auto kx = v16 ? damsm_fwd2x_kernel<true, true> : damsm_fwd2x_kernel<false, true>;
       AGB_CUDA(cudaFuncSetAttribute(kx, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes2));
       const int slot = prof_begin(PROF_DAMSM_CAND, st);
       kx<<<grid, kThreads, kSmemBytes2, st>>>(mapWh, mapWl, mapCt, mapCtl, mapCk, mapCkl, xp);
@@ -977,7 +979,7 @@ static int run_cand(const float* img, const float* words, int64_t ws_b, int64_t 
   }
   CUtensorMap mapW;
   if (int rc = make_tmap_2d(&mapW, Wh, (uint64_t)pl.nt_max * kTileN, kD, 128, bf)) return rc;
-  auto kern = damsm_fwd2_kernel<T16, false, true>;
+  auto kern = v16 ? damsm_fwd2_kernel<T16, true, true> : damsm_fwd2_kernel<T16, false, true>;
   AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes2));
   const int slot = prof_begin(PROF_DAMSM_CAND, st);
   kern<<<grid, kThreads, kSmemBytes2, st>>>(mapW, mapCt, mapCk, p);
@@ -991,7 +993,7 @@ template <typename T16>
 static int run_pairs(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
                      const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap, int P,
                      int T, int R, float gamma1, float gamma2, float* m_out, char* ws, const CandPlan& pl,
-                     cudaStream_t st) {
+                     cudaStream_t st, void* v16 = nullptr, float4* rowst = nullptr) {
   int32_t* keyA = (int32_t*)(ws + pl.off_keyA);
   int32_t* valA = (int32_t*)(ws + pl.off_valA);
   int32_t* keyB = (int32_t*)(ws + pl.off_keyB);
@@ -1016,7 +1018,7 @@ static int run_pairs(const float* img, const float* words, int64_t ws_b, int64_t
   pair_offsets_kernel<<<(unsigned)((std::max(P, Bi + 1) + 255LL) / 256), 256, 0, st>>>(keyB, valB, pair_cap, P, Bi, eoff, capS);
   if (int rc = check_launch("pair_offsets_kernel")) return rc;
   if (int rc = run_cand<T16>(img, words, ws_b, ws_d, ws_t, cap_lens, Bc, capS, eoff, Bi, 0, T, R, gamma1, gamma2, mS,
-                             ws, pl, st))
+                             ws, pl, st, v16, rowst))
     return rc;
   pair_scatter_m_kernel<<<(unsigned)((P + 255LL) / 256), 256, 0, st>>>(mS, valB, eoff, Bi, P, m_out);
   return check_launch("pair_scatter_m_kernel");
@@ -1025,6 +1027,7 @@ static int run_pairs(const float* img, const float* words, int64_t ws_b, int64_t
 #include "damsm_tc_bwd2.inc"
 #include "damsm_tc_bwd3.inc"
 #include "damsm_tc_bwd2_host.inc"
+#include "damsm_tc_pairs_bwd.inc"
 
 }  // namespace tc
 
@@ -1149,6 +1152,89 @@ int damsm_tc_pairs_fwd(const float* img, const float* words, int64_t ws_b, int64
   if (side)
     if (int rj = tc::side_join(side, st)) return rc ? rc : rj;
   return rc;
+}
+
+// 0 when the shapes are outside the pair path's range (the caller has checked T, D, R and math)
+size_t damsm_tc_pairs_train_workspace_bytes(int Bi, int Bc, long long P, int T, int math) {
+  if (Bi <= 0 || Bi > 65535 || Bc <= 0 || P < 0 || P >= (long long)INT32_MAX) return 0;
+  const tc::PairTrainPlan pl = tc::make_pairs_train_plan(Bi, Bc, P, T, math == AGB_MATH_TC_F16X2);
+  return tc::cand_plan_fits(pl.c) ? pl.total : 0;
+}
+
+static int pairs_train_check(int Bi, int Bc, long long P, float gamma1, int math) {
+  if (Bc <= 0 || Bi <= 0 || P < 0) return fail_arg("non-positive size");
+  if (Bi > 65535) return fail_unsupported("Bi=%d > 65535", Bi);
+  if (P >= (long long)INT32_MAX) return fail_unsupported("P=%lld >= 2^31", P);
+  if (math != AGB_MATH_TC_BF16 && gamma1 > 11.f) return fail_unsupported("gamma1=%g overflows fp16 (use bf16 math)", gamma1);
+  return 0;
+}
+
+int damsm_tc_pairs_train_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                             const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap,
+                             long long P, int T, int R, float gamma1, float gamma2, float* m_out, void* workspace,
+                             size_t workspace_bytes, int math, cudaStream_t st) {
+  if (int rc = pairs_train_check(Bi, Bc, P, gamma1, math)) return rc;
+  const tc::PairTrainPlan pl = tc::make_pairs_train_plan(Bi, Bc, P, T, math == AGB_MATH_TC_F16X2);
+  if (!tc::cand_plan_fits(pl.c)) return fail_unsupported("Bi=%d P=%lld: %lld word tiles exceed the int32 cost prefix", Bi, P, pl.c.nt_max);
+  if (P == 0) return 0;
+  if (workspace_bytes < pl.total) {
+    set_error("workspace too small: %zu < %zu", workspace_bytes, pl.total);
+    return AGB_E_WORKSPACE;
+  }
+  char* ws = (char*)workspace;
+  void* v16 = ws + pl.off_v16;
+  float4* rowst = (float4*)(ws + pl.off_rowst);
+  if (math == AGB_MATH_TC_BF16)
+    return tc::run_pairs<__nv_bfloat16>(img, words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, pair_img, pair_cap, (int)P, T, R,
+                                        gamma1, gamma2, m_out, ws, pl.c, st, v16, rowst);
+  return tc::run_pairs<__half>(img, words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, pair_img, pair_cap, (int)P, T, R, gamma1,
+                               gamma2, m_out, ws, pl.c, st, v16, rowst);
+}
+
+int damsm_tc_pairs_bwd(const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t, const int32_t* cap_lens, int Bi,
+                       int Bc, long long P, int T, int R, float gamma1, float gamma2, const float* dm, float* dimg,
+                       float* dwords, void* workspace, size_t workspace_bytes, int math, cudaStream_t st) {
+  if (int rc = pairs_train_check(Bi, Bc, P, gamma1, math)) return rc;
+  const tc::PairTrainPlan pl = tc::make_pairs_train_plan(Bi, Bc, P, T, math == AGB_MATH_TC_F16X2);
+  if (!tc::cand_plan_fits(pl.c)) return fail_unsupported("Bi=%d P=%lld: %lld word tiles exceed the int32 cost prefix", Bi, P, pl.c.nt_max);
+  if (P == 0) {   // no pair: every gradient is zero
+    if (dimg) AGB_CUDA(cudaMemsetAsync(dimg, 0, (size_t)Bi * tc::kD * R * sizeof(float), st));
+    if (dwords) AGB_CUDA(cudaMemsetAsync(dwords, 0, (size_t)Bc * T * tc::kD * sizeof(float), st));
+    return 0;
+  }
+  if (workspace_bytes < pl.total) {
+    set_error("workspace too small: %zu < %zu", workspace_bytes, pl.total);
+    return AGB_E_WORKSPACE;
+  }
+  if (math == AGB_MATH_TC_BF16)
+    return tc::run_pairs_bwd<__nv_bfloat16>(words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, (int)P, T, R, gamma1, gamma2, dm,
+                                            dimg, dwords, (char*)workspace, pl, st);
+  return tc::run_pairs_bwd<__half>(words, ws_b, ws_d, ws_t, cap_lens, Bi, Bc, (int)P, T, R, gamma1, gamma2, dm, dimg,
+                                   dwords, (char*)workspace, pl, st);
+}
+
+size_t sent_cos_pairs_bwd_workspace_bytes(int Bi, int Bc, long long P) {
+  if (Bi <= 0 || Bc <= 0 || P < 0 || P >= (long long)INT32_MAX) return 0;
+  return tc::make_sent_pairs_plan(Bi, Bc, P).total;
+}
+
+int sent_cos_pairs_bwd(const float* cnn, const float* rnn, int Bi, int Bc, const int32_t* pair_img,
+                       const int32_t* pair_cap, long long P, int D, float eps, const float* dscos, float* dcnn,
+                       float* drnn, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  if (Bi <= 0 || Bc <= 0 || D <= 0 || P < 0) return fail_arg("non-positive size");
+  if (P >= (long long)INT32_MAX) return fail_unsupported("P=%lld >= 2^31", P);
+  if (P == 0) {
+    if (dcnn) AGB_CUDA(cudaMemsetAsync(dcnn, 0, (size_t)Bi * D * sizeof(float), st));
+    if (drnn) AGB_CUDA(cudaMemsetAsync(drnn, 0, (size_t)Bc * D * sizeof(float), st));
+    return 0;
+  }
+  const tc::SentPairsPlan pl = tc::make_sent_pairs_plan(Bi, Bc, P);
+  if (workspace_bytes < pl.total) {
+    set_error("workspace too small: %zu < %zu", workspace_bytes, pl.total);
+    return AGB_E_WORKSPACE;
+  }
+  return tc::run_sent_pairs_bwd(cnn, rnn, Bi, Bc, pair_img, pair_cap, (int)P, D, eps, dscos, dcnn, drnn,
+                                (char*)workspace, pl, st);
 }
 
 int damsm_tc_bwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,

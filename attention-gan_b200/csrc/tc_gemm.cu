@@ -13,7 +13,7 @@
 #include <algorithm>
 #include <atomic>
 
-#include "tc_common.cuh"
+#include "tc_gemm_pairs.cuh"
 
 namespace agb {
 namespace tc {
@@ -34,10 +34,10 @@ __device__ __forceinline__ uint64_t make_desc_sw128_mn(uint32_t smem_addr, uint3
   return d;
 }
 
-__global__ void __launch_bounds__(192)
-tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
-               const __grid_constant__ CUtensorMap mapA2, const __grid_constant__ CUtensorMap mapB2,
-               const TcGemmArgs g) {
+// kPairs: the per-batch K range / B operand of TcGemmPairArgs (all of it under if constexpr)
+template <bool kPairs, typename Args>
+__device__ __forceinline__ void tc_gemm_body(const CUtensorMap& mapA, const CUtensorMap& mapB, const CUtensorMap& mapA2,
+                                             const CUtensorMap& mapB2, const Args& g) {
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* smem = (unsigned char*)(((uintptr_t)smem_dyn + 1023) & ~(uintptr_t)1023);
   __shared__ uint64_t full[kGemmStages], empty[kGemmStages], done;
@@ -54,6 +54,18 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
   if (g.split_kb) {
     kb_begin = z * g.KB;
     kb_count = max(0, min(g.KB, g.kb_total - kb_begin));
+  }
+  int krow0 = 0, zbB = zb;                             // kPairs: first K row of batch z, batch of the B operand
+  if constexpr (kPairs) {
+    if (g.koff) {
+      const int lo = min(max(g.koff[z], g.kt0), g.kt0 + g.kct), hi = min(max(g.koff[z + 1], g.kt0), g.kt0 + g.kct);
+      kchunks = max(0, hi - lo) * 2;
+      krow0 = (lo - g.kt0) * 128;
+    }
+    if (g.bsel) {
+      if (g.dyn_t0 + z >= g.dyn_tiles[0]) return;
+      zbB = g.bsel[g.dyn_t0 + z];
+    }
   }
   int m_valid = g.M;
   if (g.dyn_dim) {
@@ -100,8 +112,12 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
         unsigned char* sb = sa + MT * kChunkBytes16;
         const int64_t azr = src ? g.a2_zrow : g.a_zrow, bzr = src ? g.b2_zrow : g.b_zrow;
         const int64_t azc = src ? g.a2_zcol : g.a_zcol, bzc = src ? g.b2_zcol : g.b_zcol;
-        const int arow = (int)(zb * azr + kb * g.a_kbrow), acol = (int)(zb * azc + kb * g.a_kbcol);
-        const int brow = (int)(zb * bzr + kb * g.b_kbrow), bcol = (int)(zb * bzc + kb * g.b_kbcol);
+        int arow = (int)(zb * azr + kb * g.a_kbrow), acol = (int)(zb * azc + kb * g.a_kbcol);
+        int brow = (int)(zbB * bzr + kb * g.b_kbrow), bcol = (int)(zbB * bzc + kb * g.b_kbcol);
+        if constexpr (kPairs) {
+          (g.a_mn ? arow : acol) += krow0;
+          (g.b_mn ? brow : bcol) += krow0;
+        }
         for (int mt = 0; mt < MT; ++mt) {
           unsigned char* sam = sa + mt * kChunkBytes16;
           const int mm = m0 + mt * 128;
@@ -235,14 +251,24 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
   if (warp == 0) tmem_dealloc(tmem, tmem_cols);
 }
 
-int tc_gemm2(const TcGemmArgs& g_in, const CUtensorMap& mapA, const CUtensorMap& mapB, const CUtensorMap& mapA2,
-             const CUtensorMap& mapB2, int batch, cudaStream_t st) {
-  TcGemmArgs g = g_in;
-  if (g.M <= 0 || g.N <= 0 || batch <= 0) return 0;
+__global__ void __launch_bounds__(192)
+tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
+               const __grid_constant__ CUtensorMap mapA2, const __grid_constant__ CUtensorMap mapB2,
+               const TcGemmArgs g) {
+  tc_gemm_body<false>(mapA, mapB, mapA2, mapB2, g);
+}
+
+__global__ void __launch_bounds__(192)
+tc_gemm_pairs_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
+                     const __grid_constant__ CUtensorMap mapA2, const __grid_constant__ CUtensorMap mapB2,
+                     const TcGemmPairArgs g) {
+  tc_gemm_body<true>(mapA, mapB, mapA2, mapB2, g);
+}
+
+// launch configuration shared by both instantiations: validates g, sets g.stages, returns grid and smem size
+template <typename Args>
+static int tc_gemm_config(Args& g, int batch, dim3* grid_out, int* smem_out) {
   if (g.K <= 0 || g.K % 64 || g.KB <= 0) return fail_arg("tc_gemm: K=%d must be a positive multiple of 64", g.K);
-  // NT = 160 (MN-major B only): two equal column tiles for N = 289...320, so that the CTAs sharing an A operand run
-  // in lockstep and the second read of A hits the L2 (a 192 + 128 split drifts apart: 24 GB instead of 17 GB of DRAM
-  // reads per d img launch, profiles/r2_ncu_attention_and_gemm_metrics.txt)
   if (g.NT != 64 && g.NT != 128 && g.NT != 192 && g.NT != 256 && !(g.NT == 160 && g.b_mn))
     return fail_arg("tc_gemm: NT=%d", g.NT);
   if (g.NT0 && (g.NT0 % 64 || g.NT0 > 256 || !g.b_mn)) return fail_arg("tc_gemm: NT0=%d", g.NT0);
@@ -250,6 +276,49 @@ int tc_gemm2(const TcGemmArgs& g_in, const CUtensorMap& mapA, const CUtensorMap&
   const int nt_max = std::max(g.NT, g.NT0);
   if (g.MT * nt_max > 512) return fail_arg("tc_gemm: MT*NT=%d exceeds TMEM", g.MT * nt_max);
   if (g.nsrc != 2) g.nsrc = 1;
+  dim3 grid(g.NT0 ? 1 + cdiv(std::max(0, g.N - g.NT0), g.NT) : cdiv(g.N, g.NT), cdiv(g.M, 128 * g.MT), batch);
+  if (grid.y > 65535 || grid.z > 65535) return fail_unsupported("tc_gemm grid too large");
+  const int stage_bytes = g.MT * kChunkBytes16 + (nt_max + 63) / 64 * 64 * 128;
+  const long long chunks = (long long)g.nsrc * g.KB * (g.K / 64);
+  const int max_stages = std::min(kGemmStages, (kGemmSmem - 1024) / stage_bytes);
+  g.stages = (int)std::min<long long>(max_stages, std::max<long long>(2, chunks));
+  *grid_out = grid;
+  *smem_out = std::max(g.stages * stage_bytes, 128 * (nt_max + 1) * 4) + 1024;
+  return 0;
+}
+
+int tc_gemm_pairs(const TcGemmPairArgs& g_in, const CUtensorMap& mapA, const CUtensorMap& mapB, const CUtensorMap& mapA2,
+                  const CUtensorMap& mapB2, int batch, cudaStream_t st) {
+  TcGemmPairArgs g = g_in;
+  if (g.M <= 0 || g.N <= 0 || batch <= 0) return 0;
+  dim3 grid;
+  int smem_bytes = 0;
+  if (int rc = tc_gemm_config(g, batch, &grid, &smem_bytes)) return rc;
+  {   // per device, once
+    static std::atomic<bool> attr_set[64];
+    int dev = 0;
+    AGB_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64 || !attr_set[dev].load(std::memory_order_relaxed)) {
+      AGB_CUDA(cudaFuncSetAttribute(tc_gemm_pairs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kGemmSmem));
+      if (dev >= 0 && dev < 64) attr_set[dev].store(true, std::memory_order_relaxed);
+    }
+  }
+  const int slot = prof_begin(g.prof_tag ? g.prof_tag : PROF_DAMSM_TC_BWD, st);
+  tc_gemm_pairs_kernel<<<grid, 192, smem_bytes, st>>>(mapA, mapB, mapA2, mapB2, g);
+  prof_end(slot, st);
+  return check_launch("tc_gemm_pairs_kernel");
+}
+
+int tc_gemm2(const TcGemmArgs& g_in, const CUtensorMap& mapA, const CUtensorMap& mapB, const CUtensorMap& mapA2,
+             const CUtensorMap& mapB2, int batch, cudaStream_t st) {
+  TcGemmArgs g = g_in;
+  if (g.M <= 0 || g.N <= 0 || batch <= 0) return 0;
+  // NT = 160 (MN-major B only): two equal column tiles for N = 289...320, so that the CTAs sharing an A operand run
+  // in lockstep and the second read of A hits the L2 (a 192 + 128 split drifts apart: 24 GB instead of 17 GB of DRAM
+  // reads per d img launch, profiles/r2_ncu_attention_and_gemm_metrics.txt)
+  dim3 grid;
+  int smem_bytes = 0;
+  if (int rc = tc_gemm_config(g, batch, &grid, &smem_bytes)) return rc;
   {   // per device, once
     static std::atomic<bool> attr_set[64];
     int dev = 0;
@@ -259,15 +328,6 @@ int tc_gemm2(const TcGemmArgs& g_in, const CUtensorMap& mapA, const CUtensorMap&
       if (dev >= 0 && dev < 64) attr_set[dev].store(true, std::memory_order_relaxed);
     }
   }
-  dim3 grid(g.NT0 ? 1 + cdiv(std::max(0, g.N - g.NT0), g.NT) : cdiv(g.N, g.NT), cdiv(g.M, 128 * g.MT), batch);
-  if (grid.y > 65535 || grid.z > 65535) return fail_unsupported("tc_gemm grid too large");
-  // ring depth: as deep as ~192 KB allows; short reductions get a short ring so that several CTAs
-  // share an SM and hide each other's prologue
-  const int stage_bytes = g.MT * kChunkBytes16 + (nt_max + 63) / 64 * 64 * 128;
-  const long long chunks = (long long)g.nsrc * g.KB * (g.K / 64);
-  const int max_stages = std::min(kGemmStages, (kGemmSmem - 1024) / stage_bytes);
-  g.stages = (int)std::min<long long>(max_stages, std::max<long long>(2, chunks));
-  const int smem_bytes = std::max(g.stages * stage_bytes, 128 * (nt_max + 1) * 4) + 1024;
   const int slot = prof_begin(g.prof_tag ? g.prof_tag : PROF_DAMSM_TC_BWD, st);
   tc_gemm_kernel<<<grid, 192, smem_bytes, st>>>(mapA, mapB, mapA2, mapB2, g);
   prof_end(slot, st);

@@ -27,7 +27,7 @@ import numpy as np
 import torch
 
 from ..agb_native import native, ops, torch_ops
-from ..losses.damsm_core import as_device_i32
+from ..losses.damsm_core import as_device_i32, chunk_pairs, pair_index
 
 _CAND_MATH = ("f16", "bf16", "f16x2")
 
@@ -72,29 +72,11 @@ class DAMSMScorer:
 
     def _chunk_pairs(self, N: int, Nc: int, P: int, T: int, D: int, R: int, ws_bytes) -> int:
         """the most pairs whose workspace fits workspace_bytes (the size grows with the pair count)"""
-        if ws_bytes(N, Nc, 1, T, D, R, self.math) == 0:
-            raise native.NativeError(f"pair DAMSM shape N={N} Nc={Nc} T={T} D={D} R={R} is unsupported")
-        lo, hi = 0, P
-        while lo < hi:
-            mid = (lo + hi + 1) // 2
-            nb = ws_bytes(N, Nc, mid, T, D, R, self.math)
-            if 0 < nb <= self.workspace_bytes:
-                lo = mid
-            else:
-                hi = mid - 1
-        if lo == 0:
-            need = ws_bytes(N, Nc, 1, T, D, R, self.math)
-            raise native.NativeError(f"workspace_bytes={self.workspace_bytes} is below the {need} bytes one pair "
-                                     f"against {N} images needs")
-        return lo
+        return chunk_pairs(N, Nc, P, T, D, R, self.math, ws_bytes, self.workspace_bytes)
 
     @staticmethod
     def _pairs(image_idx, caption_idx, device):
-        pi = as_device_i32(image_idx, device).reshape(-1)
-        pc = as_device_i32(caption_idx, device).reshape(-1)
-        if pi.shape[0] != pc.shape[0]:
-            raise ValueError(f"image_idx has {pi.shape[0]} entries, caption_idx {pc.shape[0]}")
-        return pi, pc
+        return pair_index(image_idx, caption_idx, device)
 
     @staticmethod
     def _by_caption(candidates, Nc: int, device):

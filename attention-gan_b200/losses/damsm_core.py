@@ -346,3 +346,31 @@ def _side_stream(device) -> "torch.cuda.Stream":
     if s is None:
         s = _SIDE_STREAMS[key] = torch.cuda.Stream(device=device)
     return s
+
+
+def pair_index(image_idx, caption_idx, device):
+    """image_idx, caption_idx [P] (numpy, int64 or int32) -> two contiguous int32 device tensors"""
+    pi = as_device_i32(image_idx, device).reshape(-1)
+    pc = as_device_i32(caption_idx, device).reshape(-1)
+    if pi.shape[0] != pc.shape[0]:
+        raise ValueError(f"image_idx has {pi.shape[0]} entries, caption_idx {pc.shape[0]}")
+    return pi, pc
+
+
+def chunk_pairs(N: int, Nc: int, P: int, T: int, D: int, R: int, math: int, ws_bytes, budget: int) -> int:
+    """the most pairs of a list whose workspace ws_bytes(N, Nc, pairs, T, D, R, math) fits budget (the size grows
+    with the pair count); long lists run in contiguous chunks of that many pairs"""
+    if ws_bytes(N, Nc, 1, T, D, R, math) == 0:
+        raise native.NativeError(f"pair DAMSM shape N={N} Nc={Nc} T={T} D={D} R={R} is unsupported")
+    lo, hi = 0, P
+    while lo < hi:
+        mid = (lo + hi + 1) // 2
+        nb = ws_bytes(N, Nc, mid, T, D, R, math)
+        if 0 < nb <= budget:
+            lo = mid
+        else:
+            hi = mid - 1
+    if lo == 0:
+        need = ws_bytes(N, Nc, 1, T, D, R, math)
+        raise native.NativeError(f"workspace_bytes={budget} is below the {need} bytes one pair against {N} images needs")
+    return lo

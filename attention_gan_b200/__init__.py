@@ -29,6 +29,7 @@ from .losses.words_loss import WordsLoss  # noqa: E402,F401
 from .losses.sentence_loss import SentenceLoss  # noqa: E402,F401
 from .losses.damsm_loss import DAMSMLoss  # noqa: E402,F401
 from .evaluation import DAMSMScorer, mismatched_candidates, r_precision  # noqa: E402,F401
+from .losses.pair_scores import sentence_pair_scores, words_pair_scores  # noqa: E402,F401
 
 # reference module -> (native module, names it provides)
 _REPLACED = {

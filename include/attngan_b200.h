@@ -306,6 +306,40 @@ int agb_damsm_pairs_fwd(const float* img, const float* words, int64_t ws_b, int6
 int agb_sent_cos_pairs_fwd(const float* cnn, const float* rnn, int Bi, int Bc, const int32_t* pair_img,
                            const int32_t* pair_cap, long long P, int D, float eps, float* scos_out, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Training on a pair list: gradients of the pair scores m (agb_damsm_pairs_fwd) and of the pair cosines
+ * (agb_sent_cos_pairs_fwd), so that a loss over a chosen set of pairs costs only those pairs
+ *   agb_damsm_pairs_train_fwd: the arguments of agb_damsm_pairs_fwd without the maps; writes m_out [P] (bit for bit
+ *     agb_damsm_pairs_fwd's m) and leaves in the workspace what agb_damsm_pairs_bwd reads: the sorted list, the
+ *     packed tiles, the normalised context vectors and the row statistics of every packed word row
+ *   agb_damsm_pairs_bwd: the same inputs, the same list and the workspace of the matching train forward, untouched
+ *     in between; dm [P] = dLoss/dm in list order
+ *     dimg   [Bi,D,R] fp32 contiguous (or NULL), every element written
+ *     dwords [Bc,T,D] fp32 contiguous (word-major, as agb_damsm_bwd writes it) or NULL, every element written
+ *     A pair with an invalid index or a caption of length 0 contributes nothing, whatever its dm.  An image or
+ *     caption in no valid pair and the padded word slots t >= cap_lens get exactly 0.  The reductions have a fixed
+ *     order (a stable integer sort of the entries by caption): the gradients are bit-reproducible.  fp16 operands
+ *     (bf16 in AGB_MATH_TC_BF16) scaled by the dense backward's power-of-two gradient scale, fp32 accumulation.
+ *   agb_sent_cos_pairs_bwd: dscos [P] -> dcnn [Bi,D], drnn [Bc,D] (either may be NULL), fp32 contiguous, with a
+ *     workspace of its own; per image and per caption the pairs are summed in list order
+ *   The workspace sizes depend on shapes only (no device query).  P = 0 is a no-op; the backward calls then write
+ *   zero gradients.  Limits as agb_damsm_pairs_fwd (Bi <= 65535, P < 2^31).  No host synchronisation, nothing
+ *   allocated: forward and backward can be captured in a CUDA graph.
+ * ---------------------------------------------------------------------------------------------- */
+size_t agb_damsm_pairs_train_workspace_bytes(int Bi, int Bc, long long P, int T, int D, int R, int math);
+int agb_damsm_pairs_train_fwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                              const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap,
+                              long long P, int T, int D, int R, float gamma1, float gamma2, float* m_out,
+                              void* workspace, size_t workspace_bytes, int math, void* stream);
+int agb_damsm_pairs_bwd(const float* img, const float* words, int64_t ws_b, int64_t ws_d, int64_t ws_t,
+                        const int32_t* cap_lens, int Bi, int Bc, const int32_t* pair_img, const int32_t* pair_cap,
+                        long long P, int T, int D, int R, float gamma1, float gamma2, const float* dm, float* dimg,
+                        float* dwords, void* workspace, size_t workspace_bytes, int math, void* stream);
+size_t agb_sent_cos_pairs_bwd_workspace_bytes(int Bi, int Bc, long long P, int D);
+int agb_sent_cos_pairs_bwd(const float* cnn, const float* rnn, int Bi, int Bc, const int32_t* pair_img,
+                           const int32_t* pair_cap, long long P, int D, float eps, const float* dscos, float* dcnn,
+                           float* drnn, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
