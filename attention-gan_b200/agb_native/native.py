@@ -37,6 +37,13 @@ SIGNATURES = {
                                   c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_void_p, c_size_t, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                   c_void_p]),
+    "agb_word_attn_fwd_nhwc": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p,
+                                       c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
+                                       c_int, c_int, c_int, c_void_p]),
+    "agb_word_attn_bwd_nhwc": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p,
+                                       c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p,
+                                       c_void_p, c_size_t, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                       c_void_p]),
     "agb_damsm_supported": (c_int, [c_int, c_int, c_int, c_int]),
     "agb_damsm_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int]),
     "agb_damsm_fwd": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int,

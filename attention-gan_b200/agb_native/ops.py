@@ -38,24 +38,61 @@ def _ws(nbytes: int, device) -> torch.Tensor:
 # ------------------------------------------------------------------------------------------------
 # generator word-context attention                       reference networks/attention.py:25-79
 # ------------------------------------------------------------------------------------------------
+def attn_layout_nhwc(images: torch.Tensor) -> bool:
+    """The layout the attention kernels take `images` in: False for contiguous NCHW (also when the tensor is
+    channels_last-contiguous too, e.g. C = 1 or H = W = 1), True for channels_last (NHWC).  Anything else raises.
+    The reference's `.view(B, -1, H*W)` (attention.py:55) accepts both."""
+    if images.is_contiguous():
+        return False
+    if images.is_contiguous(memory_format=torch.channels_last):
+        return True
+    raise RuntimeError("images must be contiguous NCHW or channels_last (torch.channels_last); "
+                       f"got strides {tuple(images.stride())} for shape {tuple(images.shape)}")
+
+
+def attn_memory_format(images: torch.Tensor) -> torch.memory_format:
+    """the memory format of every [B, *, H, W] output and gradient the attention produces for `images`"""
+    return torch.channels_last if attn_layout_nhwc(images) else torch.contiguous_format
+
+
+def _nhwc_pixel_stride(t: torch.Tensor) -> Optional[int]:
+    """pixel stride of a [B, C, H, W] view whose channels are contiguous and whose pixels are evenly spaced
+    (channels_last, or its channel slice [:, C0:C1]); None otherwise"""
+    _, C, H, W = t.shape
+    ps = t.stride(3) if W > 1 else t.stride(2)
+    if (C > 1 and t.stride(1) != 1) or (H > 1 and t.stride(2) != W * ps) or ps < C:
+        return None
+    return ps
+
+
 def word_attn_fwd(images: torch.Tensor, words: torch.Tensor, weight: torch.Tensor, mask: torch.Tensor,
                   scaled: bool, want_attn: bool = True, ctx_out: Optional[torch.Tensor] = None
                   ) -> Tuple[torch.Tensor, Optional[torch.Tensor], torch.Tensor]:
-    """images [B,C,H,W] contiguous (f32/bf16/f16), words [B,E,T] fp32 any strides, weight [C,E] fp32,
-    mask [B,T] int64.  Returns (ctx [B,C,H,W], attn [B,T,H,W] or None, we [B,C,T] fp32).
-    ctx_out: optional pre-allocated destination whose batch stride may exceed C*H*W (a channel
-    slice of a concat buffer, generator_submodules.py:116)."""
+    """images [B,C,H,W] contiguous NCHW or channels_last (f32/bf16/f16), words [B,E,T] fp32 any strides,
+    weight [C,E] fp32, mask [B,T] int64.  Returns (ctx [B,C,H,W], attn [B,T,H,W] or None, we [B,C,T] fp32);
+    ctx and attn have the memory format of `images`.
+    ctx_out: optional pre-allocated destination whose batch stride may exceed C*H*W (a channel slice of a
+    concat buffer, generator_submodules.py:116); for channels_last images its pixel stride may exceed C."""
     require_cuda(images, words, weight, mask)
     B, C, H, W = images.shape
     E, T = words.shape[1], words.shape[2]
     HW = H * W
-    if not images.is_contiguous():
-        raise RuntimeError("images must be contiguous NCHW (the reference .view()s it, attention.py:55)")
-    ctx = ctx_out if ctx_out is not None else torch.empty_like(images)
+    nhwc = attn_layout_nhwc(images)
+    fmt = torch.channels_last if nhwc else torch.contiguous_format
+    ctx = ctx_out if ctx_out is not None else torch.empty_like(images, memory_format=fmt)
+    attn = torch.empty((B, T, H, W), dtype=images.dtype, device=images.device, memory_format=fmt) if want_attn else None
+    we = torch.empty((B, C, T), dtype=torch.float32, device=images.device)
+    if nhwc:
+        ps = _nhwc_pixel_stride(ctx)
+        if ps is None:
+            raise RuntimeError("ctx_out must be channels_last (channels contiguous) for channels_last images")
+        rc = N.lib().agb_word_attn_fwd_nhwc(_p(images), _p(words), words.stride(0), words.stride(1), words.stride(2),
+                                            _p(weight), _p(mask), _p(ctx), ctx.stride(0), ps, _p(attn), _p(we),
+                                            B, C, HW, E, T, _IO[images.dtype], int(bool(scaled)), _stream(images))
+        N.check(rc, "agb_word_attn_fwd_nhwc")
+        return ctx, attn, we
     if ctx.stride(1) != HW or ctx.stride(3) != 1 or ctx.stride(2) != W:
         raise RuntimeError("ctx_out must be channel-contiguous NCHW")
-    attn = torch.empty((B, T, H, W), dtype=images.dtype, device=images.device) if want_attn else None
-    we = torch.empty((B, C, T), dtype=torch.float32, device=images.device)
     rc = N.lib().agb_word_attn_fwd(_p(images), _p(words), words.stride(0), words.stride(1), words.stride(2),
                                    _p(weight), _p(mask), _p(ctx), ctx.stride(0), _p(attn), _p(we),
                                    B, C, HW, E, T, _IO[images.dtype], int(bool(scaled)), _stream(images))
@@ -65,20 +102,38 @@ def word_attn_fwd(images: torch.Tensor, words: torch.Tensor, weight: torch.Tenso
 
 def word_attn_bwd(images, words, weight, mask, we, dctx, dattn, scaled: bool, need_dwords: bool,
                   need_dweight: bool):
-    """Returns (dimages, dwords [B,E,T] fp32 or None, dweight [C,E] fp32 or None)."""
+    """Returns (dimages, dwords [B,E,T] fp32 or None, dweight [C,E] fp32 or None); dimages has the memory format
+    of `images`.  A dctx / dattn in the other layout is converted once; in the images' layout it is read in place
+    (dctx may be a channel slice of a concat buffer's gradient)."""
     require_cuda(images, words, weight, mask, we, dctx, dattn)
     B, C, H, W = images.shape
     E, T = words.shape[1], words.shape[2]
     HW = H * W
-    if dctx.stride(1) != HW or dctx.stride(3) != 1 or dctx.stride(2) != W:
-        dctx = dctx.contiguous()
-    if dattn is not None:
-        dattn = dattn.contiguous()
-    dimages = torch.empty_like(images)
+    nhwc = attn_layout_nhwc(images)
+    if nhwc:
+        ps = _nhwc_pixel_stride(dctx)
+        if ps is None:
+            dctx = dctx.contiguous(memory_format=torch.channels_last)
+            ps = C
+        if dattn is not None:
+            dattn = dattn.contiguous(memory_format=torch.channels_last)
+    else:
+        if dctx.stride(1) != HW or dctx.stride(3) != 1 or dctx.stride(2) != W:
+            dctx = dctx.contiguous()
+        if dattn is not None:
+            dattn = dattn.contiguous()
+    dimages = torch.empty_like(images, memory_format=torch.channels_last if nhwc else torch.contiguous_format)
     dwords = torch.empty((B, E, T), dtype=torch.float32, device=images.device) if need_dwords else None
     dweight = torch.empty((C, E), dtype=torch.float32, device=images.device) if need_dweight else None
     nbytes = N.lib().agb_word_attn_bwd_workspace_bytes(B, C, HW, E, T)
     ws = _ws(nbytes, images.device)
+    if nhwc:
+        rc = N.lib().agb_word_attn_bwd_nhwc(_p(images), _p(words), words.stride(0), words.stride(1), words.stride(2),
+                                            _p(weight), _p(mask), _p(we), _p(dctx), dctx.stride(0), ps, _p(dattn),
+                                            _p(dimages), _p(dwords), _p(dweight), _p(ws), ws.numel(),
+                                            B, C, HW, E, T, _IO[images.dtype], int(bool(scaled)), _stream(images))
+        N.check(rc, "agb_word_attn_bwd_nhwc")
+        return dimages, dwords, dweight
     rc = N.lib().agb_word_attn_bwd(_p(images), _p(words), words.stride(0), words.stride(1), words.stride(2),
                                    _p(weight), _p(mask), _p(we), _p(dctx), dctx.stride(0), _p(dattn),
                                    _p(dimages), _p(dwords), _p(dweight), _p(ws), ws.numel(),

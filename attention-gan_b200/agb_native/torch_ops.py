@@ -59,18 +59,26 @@ def host_query(name: str, *args) -> int:
 @_op("word_attn_fwd")
 def word_attn_fwd(images: Tensor, words: Tensor, weight: Tensor, mask: Tensor, scaled: bool,
                   want_attn: bool) -> Tuple[Tensor, Tensor, Tensor]:
-    """images [B,C,H,W] contiguous, words [B,E,T] fp32, weight [C,E] fp32 contiguous, mask [B,T] int64 ->
-    (ctx [B,C,H,W], attn [B,T,H,W] (empty unless want_attn), we [B,C,T] fp32)"""
+    """images [B,C,H,W] contiguous or channels_last, words [B,E,T] fp32, weight [C,E] fp32 contiguous, mask [B,T]
+    int64 -> (ctx [B,C,H,W], attn [B,T,H,W] (empty unless want_attn), we [B,C,T] fp32); ctx and attn in the
+    memory format of images"""
     ctx, attn, we = ops.word_attn_fwd(images, words, weight, mask, scaled, want_attn)
     return ctx, _none(attn, images.device), we
+
+
+def _maps_like(images: Tensor, channels: int) -> Tensor:
+    """a [B, channels, H, W] tensor in the memory format of the attention's images"""
+    B, _, H, W = images.shape
+    return torch.empty((B, channels, H, W), dtype=images.dtype, device=images.device,
+                       memory_format=ops.attn_memory_format(images))
 
 
 @word_attn_fwd.register_fake
 def _(images, words, weight, mask, scaled, want_attn):
     B, C, H, W = images.shape
     T = words.shape[2]
-    attn = images.new_empty((B, T, H, W)) if want_attn else images.new_empty((0,), dtype=torch.float32)
-    return torch.empty_like(images), attn, images.new_empty((B, C, T), dtype=torch.float32)
+    attn = _maps_like(images, T) if want_attn else images.new_empty((0,), dtype=torch.float32)
+    return _maps_like(images, C), attn, images.new_empty((B, C, T), dtype=torch.float32)
 
 
 @_op("word_attn_cat")
@@ -78,8 +86,8 @@ def word_attn_cat(images: Tensor, words: Tensor, weight: Tensor, mask: Tensor, s
                   want_attn: bool) -> Tuple[Tensor, Tensor, Tensor]:
     """word_attn_fwd writing cat((images, ctx), 1): (out [B,2C,H,W], attn or empty, we); the kernel writes the
     context at channel offset C of the fresh buffer (AttentionModule.forward_into)"""
-    B, C, H, W = images.shape
-    out = images.new_empty((B, 2 * C, H, W))
+    C = images.shape[1]
+    out = _maps_like(images, 2 * C)
     out[:, :C].copy_(images)
     _, attn, we = ops.word_attn_fwd(images, words, weight, mask, scaled, want_attn, ctx_out=out[:, C:])
     return out, _none(attn, images.device), we
@@ -89,8 +97,8 @@ def word_attn_cat(images: Tensor, words: Tensor, weight: Tensor, mask: Tensor, s
 def _(images, words, weight, mask, scaled, want_attn):
     B, C, H, W = images.shape
     T = words.shape[2]
-    attn = images.new_empty((B, T, H, W)) if want_attn else images.new_empty((0,), dtype=torch.float32)
-    return images.new_empty((B, 2 * C, H, W)), attn, images.new_empty((B, C, T), dtype=torch.float32)
+    attn = _maps_like(images, T) if want_attn else images.new_empty((0,), dtype=torch.float32)
+    return _maps_like(images, 2 * C), attn, images.new_empty((B, C, T), dtype=torch.float32)
 
 
 @_op("word_attn_bwd")
@@ -107,7 +115,7 @@ def _(images, words, weight, mask, we, dctx, dattn, scaled, need_dwords, need_dw
     B, C = images.shape[:2]
     E, T = words.shape[1], words.shape[2]
     f32 = dict(dtype=torch.float32)
-    return (torch.empty_like(images), images.new_empty((B, E, T) if need_dwords else (0,), **f32),
+    return (_maps_like(images, C), images.new_empty((B, E, T) if need_dwords else (0,), **f32),
             images.new_empty((C, E) if need_dweight else (0,), **f32))
 
 
@@ -138,8 +146,8 @@ def _word_attn_cat_backward(ctx, dout, dattn, _dwe):
     if dout is None:
         return None, None, None, None, None, None
     C = images.shape[1]
-    dout = dout.to(images.dtype).contiguous()
-    # d context is the second channel half of d out, read in place through its batch stride
+    dout = dout.to(images.dtype).contiguous(memory_format=ops.attn_memory_format(images))
+    # d context is the second channel half of d out, read in place through its batch (and pixel) stride
     di, dw, dwt = torch.ops.agb.word_attn_bwd(images, words, weight, mask, we, dout[:, C:],
                                               None if dattn is None else dattn.to(images.dtype), ctx.scaled,
                                               need_words, need_w)

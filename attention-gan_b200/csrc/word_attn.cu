@@ -21,6 +21,16 @@ int word_attn_fwd_tc(const void* images, const float* we, const int64_t* mask, v
                      int B, int C, int HW, int T, int io_dtype, float qscale, cudaStream_t st);
 int word_attn_bwd_tc_supported(const void* images, const void* dctx, int64_t dctx_bs, const void* dattn, int C, int HW,
                                int T, int io_dtype);
+int word_attn_tc_supported_nhwc(const void* images, const void* ctx, int64_t ctx_bs, int64_t ctx_ps, const void* attn,
+                                int C, int HW, int T, int io_dtype);
+int word_attn_fwd_tc_nhwc(const void* images, const float* we, const int64_t* mask, void* ctx, int64_t ctx_bs,
+                          int64_t ctx_ps, void* attn, int B, int C, int HW, int T, int io_dtype, float qscale,
+                          cudaStream_t st);
+int word_attn_bwd_tc_supported_nhwc(const void* images, const void* dctx, int64_t dctx_bs, int64_t dctx_ps,
+                                    const void* dattn, int C, int HW, int T, int io_dtype);
+int word_attn_bwd_tc_nhwc(const void* images, const float* we, const int64_t* mask, const void* dctx, int64_t dctx_bs,
+                          int64_t dctx_ps, const void* dattn, void* dimages, float* part, int part_slots, int B, int C,
+                          int HW, int T, int io_dtype, float scale, cudaStream_t st);
 int word_attn_bwd_tc_ctas(int B, int HW, int T);
 int word_attn_bwd_tc_grid(int B, int HW, int T);
 int word_attn_bwd_tc(const void* images, const float* we, const int64_t* mask, const void* dctx, int64_t dctx_bs,
@@ -84,10 +94,40 @@ __device__ __forceinline__ int stage_word_tile(const float* __restrict__ we, con
   return nv;
 }
 
+constexpr int kChanVec = 8;  // NHWC: channels one thread loads per access (pixel_scores' CU)
+constexpr int kStoreVec = 4; // NHWC: channels one thread stores per access (fewer live accumulators)
+
+// NHWC: V pixels x CU channels from pixel-major rows (pixel stride ps): per pixel, CU consecutive channels in
+// one access when `vec` (C % CU == 0 and aligned), else one by one; pixels v >= n read as zero
+template <typename IO, int CU, int V>
+__device__ __forceinline__ void load_pixel_chans(const IO* __restrict__ p, int64_t ps, int nc, bool vec, int n,
+                                                 float (&out)[CU][V]) {
+#pragma unroll
+  for (int v = 0; v < V; ++v) {
+    float t[CU];
+    if (v < n) load_vec<IO, CU>(p + (int64_t)v * ps, vec, nc, t);
+#pragma unroll
+    for (int u = 0; u < CU; ++u) out[u][v] = v < n ? t[u] : 0.f;
+  }
+}
+template <typename IO, int CU, int V>
+__device__ __forceinline__ void store_pixel_chans(IO* __restrict__ p, int64_t ps, int nc, bool vec, int n,
+                                                  const float (&in)[CU][V]) {
+#pragma unroll
+  for (int v = 0; v < V; ++v) {
+    float t[CU];
+#pragma unroll
+    for (int u = 0; u < CU; ++u) t[u] = in[u][v];
+    if (v < n) store_vec<IO, CU>(p + (int64_t)v * ps, vec, nc, t);
+  }
+}
+
 // scores for V pixels against the nv compacted words:  s[j][v] = sum_c h[c][p+v] * we_s[c][j]
-template <typename IO, int TMAX, int V>
+// kNHWC: hb points at pixel p0 of a pixel-major map with pixel stride ps (HW unused); `vec` then means
+// channel vectors of kChanVec.  The arithmetic (and its order) is the same for both layouts.
+template <typename IO, int TMAX, int V, bool kNHWC = false>
 __device__ __forceinline__ void pixel_scores(const IO* __restrict__ hb, int HW, int C, bool vec, int n,
-                                             const float* we_s, int nv, float (&s)[TMAX][V]) {
+                                             const float* we_s, int nv, float (&s)[TMAX][V], int64_t ps = 0) {
 #pragma unroll
   for (int j = 0; j < TMAX; ++j)
 #pragma unroll
@@ -95,9 +135,13 @@ __device__ __forceinline__ void pixel_scores(const IO* __restrict__ hb, int HW, 
   constexpr int CU = 8;  // channels fetched per batch: CU independent wide loads in flight
   for (int c0 = 0; c0 < C; c0 += CU) {
     float hv[CU][V];
+    if constexpr (kNHWC) {
+      load_pixel_chans<IO, CU, V>(hb + c0, ps, min(CU, C - c0), vec, n, hv);
+    } else {
 #pragma unroll
-    for (int u = 0; u < CU; ++u) {
-      if (c0 + u < C) load_vec<IO, V>(hb + (size_t)(c0 + u) * HW, vec, n, hv[u]);
+      for (int u = 0; u < CU; ++u) {
+        if (c0 + u < C) load_vec<IO, V>(hb + (size_t)(c0 + u) * HW, vec, n, hv[u]);
+      }
     }
 #pragma unroll
     for (int u = 0; u < CU; ++u) {
@@ -148,11 +192,15 @@ __device__ __forceinline__ void softmax_words(float (&s)[TMAX][V], int nv, float
 // ---------------------------------------------------------------------------------------------
 // forward                                                               attention.py:55-79
 // ---------------------------------------------------------------------------------------------
-template <typename IO, int TMAX, int V>
+// kNHWC: images / ctx / attn are pixel-major (channels_last); thread = V consecutive pixels as in NCHW, each
+// moving its pixels' channel vectors.  ctx_bs is the batch stride of ctx and ctx_ps its pixel stride (C, or 2C
+// for a channel slice of a concat buffer); vec_ok then says every channel vector is kChanVec-wide and aligned.
+template <typename IO, int TMAX, int V, bool kNHWC = false>
 __global__ void __launch_bounds__(kAttnThreads)
 word_attn_fwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
                      const int64_t* __restrict__ mask, IO* __restrict__ ctx, int64_t ctx_bs,
-                     IO* __restrict__ attn, int C, int HW, int T, float qscale, int use_tma, int vec_ok) {
+                     IO* __restrict__ attn, int C, int HW, int T, float qscale, int use_tma, int vec_ok,
+                     int64_t ctx_ps) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* we_raw = reinterpret_cast<float*>(smem_raw);
   float* we_s = we_raw + ((C * T + 3) & ~3);
@@ -165,6 +213,57 @@ word_attn_fwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
   if (p0 >= HW) return;
   const int n = min(V, HW - p0);
   const bool vec = vec_ok != 0;
+  if constexpr (kNHWC) {
+    const IO* hb = h + ((size_t)b * HW + p0) * C;
+    IO* cb = ctx + (size_t)b * ctx_bs + (size_t)p0 * ctx_ps;
+    IO* ab = attn ? attn + ((size_t)b * HW + p0) * T : nullptr;
+    const IO qnan = from_f32<IO>(__int_as_float(0x7fc00000));
+    if (nv == 0) {  // every word masked: the reference's softmax over all -inf gives NaN
+      for (int v = 0; v < n; ++v) {
+        for (int c = 0; c < C; ++c) cb[(size_t)v * ctx_ps + c] = qnan;
+        if (ab)
+          for (int t = 0; t < T; ++t) ab[(size_t)v * T + t] = qnan;
+      }
+      return;
+    }
+    float s[TMAX][V];
+    pixel_scores<IO, TMAX, V, true>(hb, HW, C, vec, n, we_s, nv, s, C);
+    softmax_words<TMAX, V>(s, nv, qscale);
+    // context = sum_j attn_j * we[:, j], kChanVec channels at a time              attention.py:73
+    for (int c0 = 0; c0 < C; c0 += kStoreVec) {
+      float acc[kStoreVec][V];
+#pragma unroll
+      for (int u = 0; u < kStoreVec; ++u) {
+#pragma unroll
+        for (int v = 0; v < V; ++v) acc[u][v] = 0.f;
+        if (c0 + u < C) {
+          const float4* w4 = reinterpret_cast<const float4*>(we_s + (c0 + u) * TMAX);
+#pragma unroll
+          for (int j4 = 0; j4 < TMAX / 4; ++j4) {
+            if (j4 * 4 < nv) {
+              const float4 w = w4[j4];
+#pragma unroll
+              for (int v = 0; v < V; ++v) {
+                acc[u][v] = fmaf(s[j4 * 4 + 0][v], w.x, acc[u][v]);
+                acc[u][v] = fmaf(s[j4 * 4 + 1][v], w.y, acc[u][v]);
+                acc[u][v] = fmaf(s[j4 * 4 + 2][v], w.z, acc[u][v]);
+                acc[u][v] = fmaf(s[j4 * 4 + 3][v], w.w, acc[u][v]);
+              }
+            }
+          }
+        }
+      }
+      store_pixel_chans<IO, kStoreVec, V>(cb + c0, ctx_ps, min(kStoreVec, C - c0), vec, n, acc);
+    }
+    if (ab) {  // a pixel's T probabilities are one contiguous row
+      for (int v = 0; v < n; ++v) {
+#pragma unroll
+        for (int j = 0; j < TMAX; ++j)
+          if (j < nv) ab[(size_t)v * T + s_idx[j]] = from_f32<IO>(s[j][v]);
+        for (int k = 0; k < T - nv; ++k) ab[(size_t)v * T + s_midx[k]] = from_f32<IO>(0.f);
+      }
+    }
+  } else {
   const IO* hb = h + (size_t)b * C * HW + p0;
   IO* cb = ctx + (size_t)b * ctx_bs + p0;
 
@@ -213,6 +312,7 @@ word_attn_fwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
     for (int v = 0; v < V; ++v) z[v] = 0.f;
     for (int k = 0; k < T - nv; ++k) store_vec<IO, V>(ab + (size_t)s_midx[k] * HW, vec, n, z);
   }
+  }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -222,12 +322,13 @@ word_attn_fwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
 // Phase 1 is thread-per-pixel like the forward; a and ds of the tile are parked in shared memory
 // and phase 2 re-maps threads to (channel, word-group) to contract over the tile's pixels.
 // ---------------------------------------------------------------------------------------------
-template <typename IO, int TMAX, int V>
+// kNHWC: images / dctx / dattn / dh pixel-major (dctx with pixel stride dctx_ps); vec_ok as in the forward
+template <typename IO, int TMAX, int V, bool kNHWC = false>
 __global__ void __launch_bounds__(kAttnThreads)
 word_attn_bwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
                      const int64_t* __restrict__ mask, const IO* __restrict__ dctx, int64_t dctx_bs,
                      const IO* __restrict__ dattn, IO* __restrict__ dh, float* __restrict__ part,
-                     int C, int HW, int T, float scale, int use_tma, int vec_ok, int vec4_ok) {
+                     int C, int HW, int T, float scale, int use_tma, int vec_ok, int vec4_ok, int64_t dctx_ps) {
   constexpr int PT = kAttnThreads * V;  // pixels per tile
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* we_raw = reinterpret_cast<float*>(smem_raw);
@@ -243,15 +344,20 @@ word_attn_bwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
   const int p0 = tile0 + tid * V;
   const int n = max(0, min(V, HW - p0));
   const bool vec = vec_ok != 0;
-  const IO* hb = h + (size_t)b * C * HW + p0;
-  const IO* db = dctx + (size_t)b * dctx_bs + p0;
+  const IO* hb = kNHWC ? h + ((size_t)b * HW + p0) * C : h + (size_t)b * C * HW + p0;
+  const IO* db = kNHWC ? dctx + (size_t)b * dctx_bs + (size_t)p0 * dctx_ps : dctx + (size_t)b * dctx_bs + p0;
 
   if (nv == 0) {  // NaN forward: propagate NaN like autograd would
     float nanv[V];
 #pragma unroll
     for (int v = 0; v < V; ++v) nanv[v] = __int_as_float(0x7fc00000);
+    if constexpr (kNHWC) {
+      for (int v = 0; v < n; ++v)
+        for (int c = 0; c < C; ++c) dh[((size_t)b * HW + p0 + v) * C + c] = from_f32<IO>(nanv[0]);
+    } else {
     if (n > 0)
       for (int c = 0; c < C; ++c) store_vec<IO, V>(dh + (size_t)b * C * HW + (size_t)c * HW + p0, vec, n, nanv);
+    }
     float* pp = part + ((size_t)b * gridDim.x + blockIdx.x) * C * T;
     for (int i = tid; i < C * T; i += kAttnThreads) pp[i] = __int_as_float(0x7fc00000);
     return;
@@ -259,7 +365,7 @@ word_attn_bwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
 
   if (n > 0) {
     float a[TMAX][V];
-    pixel_scores<IO, TMAX, V>(hb, HW, C, vec, n, we_s, nv, a);
+    pixel_scores<IO, TMAX, V, kNHWC>(hb, HW, C, vec, n, we_s, nv, a, C);
     softmax_words<TMAX, V>(a, nv, qscale);
     float g[TMAX][V];
 #pragma unroll
@@ -267,8 +373,18 @@ word_attn_bwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
 #pragma unroll
       for (int v = 0; v < V; ++v) g[j][v] = 0.f;
     // g[j] = sum_c we[c][j] * dctx[c]
-    pixel_scores<IO, TMAX, V>(db, HW, C, vec, n, we_s, nv, g);
-    if (dattn) {
+    pixel_scores<IO, TMAX, V, kNHWC>(db, HW, C, vec, n, we_s, nv, g, dctx_ps);
+    if constexpr (kNHWC) {
+      if (dattn) {  // a pixel's T gradients are one contiguous row
+        const IO* ab = dattn + ((size_t)b * HW + p0) * T;
+#pragma unroll
+        for (int j = 0; j < TMAX; ++j)
+          if (j < nv) {
+#pragma unroll
+            for (int v = 0; v < V; ++v) g[j][v] += v < n ? to_f32(ab[(size_t)v * T + s_idx[j]]) : 0.f;
+          }
+      }
+    } else if (dattn) {
       const IO* ab = dattn + (size_t)b * T * HW + p0;
 #pragma unroll
       for (int j = 0; j < TMAX; ++j)
@@ -290,6 +406,36 @@ word_attn_bwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
         if (j < nv) g[j][v] = a[j][v] * (g[j][v] - dot);  // g now holds ds
     }
     // dh[c] = scale * sum_j we[c][j] ds[j]
+    if constexpr (kNHWC) {
+      IO* ob = dh + ((size_t)b * HW + p0) * C;
+      for (int c0 = 0; c0 < C; c0 += kStoreVec) {
+        float acc[kStoreVec][V];
+#pragma unroll
+        for (int u = 0; u < kStoreVec; ++u) {
+#pragma unroll
+          for (int v = 0; v < V; ++v) acc[u][v] = 0.f;
+          if (c0 + u < C) {
+            const float4* w4 = reinterpret_cast<const float4*>(we_s + (c0 + u) * TMAX);
+#pragma unroll
+            for (int j4 = 0; j4 < TMAX / 4; ++j4) {
+              if (j4 * 4 < nv) {
+                const float4 w = w4[j4];
+#pragma unroll
+                for (int v = 0; v < V; ++v) {
+                  acc[u][v] = fmaf(g[j4 * 4 + 0][v], w.x, acc[u][v]);
+                  acc[u][v] = fmaf(g[j4 * 4 + 1][v], w.y, acc[u][v]);
+                  acc[u][v] = fmaf(g[j4 * 4 + 2][v], w.z, acc[u][v]);
+                  acc[u][v] = fmaf(g[j4 * 4 + 3][v], w.w, acc[u][v]);
+                }
+              }
+            }
+#pragma unroll
+            for (int v = 0; v < V; ++v) acc[u][v] *= scale;
+          }
+        }
+        store_pixel_chans<IO, kStoreVec, V>(ob + c0, C, min(kStoreVec, C - c0), vec, n, acc);
+      }
+    } else {
     IO* ob = dh + (size_t)b * C * HW + p0;
     for (int c = 0; c < C; ++c) {
       float acc[V];
@@ -312,6 +458,7 @@ word_attn_bwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
 #pragma unroll
       for (int v = 0; v < V; ++v) acc[v] *= scale;
       store_vec<IO, V>(ob + (size_t)c * HW, vec, n, acc);
+    }
     }
     // park a and ds (pixels beyond HW contribute zero)
 #pragma unroll
@@ -348,8 +495,18 @@ word_attn_bwd_kernel(const IO* __restrict__ h, const float* __restrict__ we,
     for (int p = 0; p < tile_pix; p += 4) {
       float h4[4], d4[4];
       const int nn = min(4, tile_pix - p);
-      load_vec<IO, 4>(hr + p, vec4_ok != 0, nn, h4);
-      load_vec<IO, 4>(dr + p, vec4_ok != 0, nn, d4);
+      if constexpr (kNHWC) {   // one channel of 4 pixels: strided
+        const IO* hq = h + ((size_t)b * HW + tile0 + p) * C + c;
+        const IO* dq = dctx + (size_t)b * dctx_bs + (size_t)(tile0 + p) * dctx_ps + c;
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          h4[i] = i < nn ? to_f32(hq[(size_t)i * C]) : 0.f;
+          d4[i] = i < nn ? to_f32(dq[(size_t)i * dctx_ps]) : 0.f;
+        }
+      } else {
+        load_vec<IO, 4>(hr + p, vec4_ok != 0, nn, h4);
+        load_vec<IO, 4>(dr + p, vec4_ok != 0, nn, d4);
+      }
 #pragma unroll
       for (int k = 0; k < JPT; ++k) {
         const int j = jg + 4 * k;
@@ -552,34 +709,44 @@ static int pick_tmax(int T) {
 static int fwd_v(int tmax) { return tmax <= 24 ? 4 : (tmax <= 32 ? 2 : 1); }
 static int bwd_v(int tmax) { return tmax <= 24 ? 2 : 1; }
 
-template <typename IO, int TMAX, int V>
+// NHWC: every channel vector of kChanVec elements starts aligned (pixel and batch strides included)
+template <typename IO>
+static bool chan_vec_ok(int C, int64_t ps, int64_t bs, const void* a, const void* b, const void* c) {
+  const uintptr_t w = sizeof(IO) * kChanVec;
+  return C % kChanVec == 0 && ps % kChanVec == 0 && bs % kChanVec == 0 && (uintptr_t)a % w == 0 &&
+         (uintptr_t)b % w == 0 && (uintptr_t)c % w == 0;
+}
+
+template <typename IO, int TMAX, int V, bool kNHWC>
 static int launch_fwd(const void* images, const float* we, const int64_t* mask, void* ctx,
-                      int64_t ctx_bs, void* attn, int B, int C, int HW, int T, float qscale,
+                      int64_t ctx_bs, int64_t ctx_ps, void* attn, int B, int C, int HW, int T, float qscale,
                       int use_tma, cudaStream_t st) {
   const size_t smem = (size_t)(((C * T + 3) & ~3) + C * TMAX) * sizeof(float);
-  const int vec_ok = (HW % V == 0) && (ctx_bs % V == 0) &&
-                     ((uintptr_t)images % (sizeof(IO) * V) == 0) && ((uintptr_t)ctx % (sizeof(IO) * V) == 0) &&
-                     (attn == nullptr || (uintptr_t)attn % (sizeof(IO) * V) == 0);
+  const int vec_ok = kNHWC ? chan_vec_ok<IO>(C, ctx_ps, ctx_bs, images, ctx, images)
+                           : (HW % V == 0) && (ctx_bs % V == 0) &&
+                             ((uintptr_t)images % (sizeof(IO) * V) == 0) && ((uintptr_t)ctx % (sizeof(IO) * V) == 0) &&
+                             (attn == nullptr || (uintptr_t)attn % (sizeof(IO) * V) == 0);
   dim3 grid(cdiv(HW, kAttnThreads * V), B);
   const int slot = prof_begin(PROF_ATTN_FWD, st);
-  word_attn_fwd_kernel<IO, TMAX, V><<<grid, kAttnThreads, smem, st>>>(
-      (const IO*)images, we, mask, (IO*)ctx, ctx_bs, (IO*)attn, C, HW, T, qscale, use_tma, vec_ok);
+  word_attn_fwd_kernel<IO, TMAX, V, kNHWC><<<grid, kAttnThreads, smem, st>>>(
+      (const IO*)images, we, mask, (IO*)ctx, ctx_bs, (IO*)attn, C, HW, T, qscale, use_tma, vec_ok, ctx_ps);
   prof_end(slot, st);
   return check_launch("word_attn_fwd_kernel");
 }
 
+constexpr size_t kBwdStaticSmem = 1024;   // bound on word_attn_bwd_kernel's static shared memory (barrier, word lists)
 template <typename IO, int TMAX, int V>
 static size_t bwd_smem(int C, int T) {
   return (size_t)(((C * T + 3) & ~3) + C * TMAX + 2 * TMAX * kAttnThreads * V) * sizeof(float);
 }
 
-template <typename IO, int TMAX, int V>
+template <typename IO, int TMAX, int V, bool kNHWC>
 static int launch_bwd(const void* images, const float* we, const int64_t* mask, const void* dctx,
-                      int64_t dctx_bs, const void* dattn, void* dimages, float* part, int B, int C,
+                      int64_t dctx_bs, int64_t dctx_ps, const void* dattn, void* dimages, float* part, int B, int C,
                       int HW, int T, float scale, int use_tma, cudaStream_t st) {
   const size_t smem = bwd_smem<IO, TMAX, V>(C, T);
-  auto kern = word_attn_bwd_kernel<IO, TMAX, V>;
-  if (smem > 48 * 1024)
+  auto kern = word_attn_bwd_kernel<IO, TMAX, V, kNHWC>;
+  if (smem + kBwdStaticSmem > 48 * 1024)   // the opt-in counts the kernel's static shared memory too
     AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   auto ok = [&](int w) {
     return (HW % w == 0) && (dctx_bs % w == 0) && ((uintptr_t)images % (sizeof(IO) * w) == 0) &&
@@ -588,9 +755,10 @@ static int launch_bwd(const void* images, const float* we, const int64_t* mask, 
   };
   dim3 grid(cdiv(HW, kAttnThreads * V), B);
   const int slot = prof_begin(PROF_ATTN_BWD, st);
+  const int vec_ok = kNHWC ? chan_vec_ok<IO>(C, dctx_ps, dctx_bs, images, dctx, dimages) : ok(V);
   kern<<<grid, kAttnThreads, smem, st>>>((const IO*)images, we, mask, (const IO*)dctx, dctx_bs,
                                         (const IO*)dattn, (IO*)dimages, part, C, HW, T, scale,
-                                        use_tma, ok(V) ? 1 : 0, ok(4) ? 1 : 0);
+                                        use_tma, vec_ok ? 1 : 0, ok(4) ? 1 : 0, dctx_ps);
   prof_end(slot, st);
   return check_launch("word_attn_bwd_kernel");
 }
@@ -618,12 +786,16 @@ static int check_common(int B, int C, int HW, int E, int T, int io_dtype) {
 
 using namespace agb;
 
-extern "C" int agb_word_attn_fwd(const void* images, const float* words, int64_t ws_b, int64_t ws_e,
-                                 int64_t ws_t, const float* conv_w, const int64_t* mask, void* ctx,
-                                 int64_t ctx_bs, void* attn, float* we, int B, int C, int HW, int E,
-                                 int T, int io_dtype, int scaled, void* stream) {
+// both layouts: nhwc = images / ctx / attn pixel-major, ctx with pixel stride ctx_ps
+static int word_attn_fwd_impl(bool nhwc, const void* images, const float* words, int64_t ws_b, int64_t ws_e,
+                              int64_t ws_t, const float* conv_w, const int64_t* mask, void* ctx, int64_t ctx_bs,
+                              int64_t ctx_ps, void* attn, float* we, int B, int C, int HW, int E, int T, int io_dtype,
+                              int scaled, void* stream) {
   if (int rc = check_common(B, C, HW, E, T, io_dtype)) return rc;
   if (!images || !words || !conv_w || !mask || !ctx || !we) return fail_arg("null pointer");
+  if (nhwc && (ctx_ps < C || ctx_bs < (int64_t)HW * ctx_ps))
+    return fail_arg("ctx strides overlap: pixel stride %lld < C=%d or batch stride %lld < HW * pixel stride",
+                    (long long)ctx_ps, C, (long long)ctx_bs);
   cudaStream_t st = (cudaStream_t)stream;
   // we[b][c,t] = sum_e W[c,e] words[b][e,t]                     (attention.py:50-52, conv1 1x1)
   {
@@ -641,18 +813,41 @@ extern "C" int agb_word_attn_fwd(const void* images, const float* words, int64_t
   const float qscale = (scaled ? 1.f / sqrtf((float)C) : 1.f) * kLog2e;
   // 16-bit feature maps: both contractions on tcgen05 (word_attn_tc.cu); fp32 maps and odd shapes:
   // CUDA cores.  Both are native sm_100a kernels of this library.
-  if (tc::word_attn_tc_supported(images, C, HW, T, io_dtype))
+  if (nhwc) {
+    if (tc::word_attn_tc_supported_nhwc(images, ctx, ctx_bs, ctx_ps, attn, C, HW, T, io_dtype))
+      return tc::word_attn_fwd_tc_nhwc(images, we, mask, ctx, ctx_bs, ctx_ps, attn, B, C, HW, T, io_dtype, qscale, st);
+  } else if (tc::word_attn_tc_supported(images, C, HW, T, io_dtype)) {
     return tc::word_attn_fwd_tc(images, we, mask, ctx, ctx_bs, attn, B, C, HW, T, io_dtype, qscale, st);
+  }
   const int use_tma = ((C * T) % 4 == 0) && ((uintptr_t)we % 16 == 0);
   const int tm = pick_tmax(T);
   int rc = 0;
-  AGB_DISPATCH_TMAX(tm, {
-    constexpr int V = TMAX <= 24 ? 4 : (TMAX <= 32 ? 2 : 1);
-    if (io_dtype == AGB_F32) rc = launch_fwd<float, TMAX, V>(images, we, mask, ctx, ctx_bs, attn, B, C, HW, T, qscale, use_tma, st);
-    else if (io_dtype == AGB_BF16) rc = launch_fwd<__nv_bfloat16, TMAX, V>(images, we, mask, ctx, ctx_bs, attn, B, C, HW, T, qscale, use_tma, st);
-    else rc = launch_fwd<__half, TMAX, V>(images, we, mask, ctx, ctx_bs, attn, B, C, HW, T, qscale, use_tma, st);
-  });
+#define AGB_FWD_LAYOUT(L)                                                                                                   \
+  AGB_DISPATCH_TMAX(tm, {                                                                                                   \
+    constexpr int V = TMAX <= 24 ? 4 : (TMAX <= 32 ? 2 : 1);                                                                \
+    if (io_dtype == AGB_F32) rc = launch_fwd<float, TMAX, V, L>(images, we, mask, ctx, ctx_bs, ctx_ps, attn, B, C, HW, T, qscale, use_tma, st); \
+    else if (io_dtype == AGB_BF16) rc = launch_fwd<__nv_bfloat16, TMAX, V, L>(images, we, mask, ctx, ctx_bs, ctx_ps, attn, B, C, HW, T, qscale, use_tma, st); \
+    else rc = launch_fwd<__half, TMAX, V, L>(images, we, mask, ctx, ctx_bs, ctx_ps, attn, B, C, HW, T, qscale, use_tma, st); \
+  })
+  if (nhwc) AGB_FWD_LAYOUT(true) else AGB_FWD_LAYOUT(false)
+#undef AGB_FWD_LAYOUT
   return rc;
+}
+
+extern "C" int agb_word_attn_fwd(const void* images, const float* words, int64_t ws_b, int64_t ws_e,
+                                 int64_t ws_t, const float* conv_w, const int64_t* mask, void* ctx,
+                                 int64_t ctx_bs, void* attn, float* we, int B, int C, int HW, int E,
+                                 int T, int io_dtype, int scaled, void* stream) {
+  return word_attn_fwd_impl(false, images, words, ws_b, ws_e, ws_t, conv_w, mask, ctx, ctx_bs, 0, attn, we, B, C, HW,
+                            E, T, io_dtype, scaled, stream);
+}
+
+extern "C" int agb_word_attn_fwd_nhwc(const void* images, const float* words, int64_t ws_b, int64_t ws_e,
+                                      int64_t ws_t, const float* conv_w, const int64_t* mask, void* ctx,
+                                      int64_t ctx_bs, int64_t ctx_ps, void* attn, float* we, int B, int C, int HW,
+                                      int E, int T, int io_dtype, int scaled, void* stream) {
+  return word_attn_fwd_impl(true, images, words, ws_b, ws_e, ws_t, conv_w, mask, ctx, ctx_bs, ctx_ps, attn, we, B, C,
+                            HW, E, T, io_dtype, scaled, stream);
 }
 
 static int dw_splits(int B) {
@@ -668,14 +863,16 @@ extern "C" size_t agb_word_attn_bwd_workspace_bytes(int B, int C, int HW, int E,
   return (((size_t)B * ntiles + (size_t)B) * C * T + (size_t)B * C * E) * sizeof(float);
 }
 
-extern "C" int agb_word_attn_bwd(const void* images, const float* words, int64_t ws_b, int64_t ws_e,
-                                 int64_t ws_t, const float* conv_w, const int64_t* mask,
-                                 const float* we, const void* dctx, int64_t dctx_bs, const void* dattn,
-                                 void* dimages, float* dwords, float* dconv_w, void* workspace,
-                                 size_t workspace_bytes, int B, int C, int HW, int E, int T,
-                                 int io_dtype, int scaled, void* stream) {
+static int word_attn_bwd_impl(bool nhwc, const void* images, const float* words, int64_t ws_b, int64_t ws_e,
+                              int64_t ws_t, const float* conv_w, const int64_t* mask, const float* we,
+                              const void* dctx, int64_t dctx_bs, int64_t dctx_ps, const void* dattn, void* dimages,
+                              float* dwords, float* dconv_w, void* workspace, size_t workspace_bytes, int B, int C,
+                              int HW, int E, int T, int io_dtype, int scaled, void* stream) {
   if (int rc = check_common(B, C, HW, E, T, io_dtype)) return rc;
   if (!images || !words || !conv_w || !mask || !we || !dctx || !dimages || !workspace) return fail_arg("null pointer");
+  if (nhwc && (dctx_ps < C || dctx_bs < (int64_t)HW * dctx_ps))
+    return fail_arg("dctx strides overlap: pixel stride %lld < C=%d or batch stride %lld < HW * pixel stride",
+                    (long long)dctx_ps, C, (long long)dctx_bs);
   if (workspace_bytes < agb_word_attn_bwd_workspace_bytes(B, C, HW, E, T)) {
     set_error("workspace too small: %zu < %zu", workspace_bytes, agb_word_attn_bwd_workspace_bytes(B, C, HW, E, T));
     return AGB_E_WORKSPACE;
@@ -688,21 +885,28 @@ extern "C" int agb_word_attn_bwd(const void* images, const float* words, int64_t
   int ntiles = cdiv(HW, kAttnThreads * V);
   float* part = (float*)workspace;
   int rc = 0;
-  const bool use_tc = tc::word_attn_bwd_tc_supported(images, dctx, dctx_bs, dattn, C, HW, T, io_dtype) != 0;
+  const bool use_tc = (nhwc ? tc::word_attn_bwd_tc_supported_nhwc(images, dctx, dctx_bs, dctx_ps, dattn, C, HW, T, io_dtype)
+                            : tc::word_attn_bwd_tc_supported(images, dctx, dctx_bs, dattn, C, HW, T, io_dtype)) != 0;
   if (use_tc) ntiles = tc::word_attn_bwd_tc_ctas(B, HW, T);
   float* dwe = part + (size_t)B * ntiles * C * T;
   int G = 0;                                      // 0: every partial slot is valid
   if (use_tc) {
     G = tc::word_attn_bwd_tc_grid(B, HW, T);
-    rc = tc::word_attn_bwd_tc(images, we, mask, dctx, dctx_bs, dattn, dimages, part, ntiles, nullptr, B, C, HW, T, io_dtype, scale, st);
+    rc = nhwc ? tc::word_attn_bwd_tc_nhwc(images, we, mask, dctx, dctx_bs, dctx_ps, dattn, dimages, part, ntiles, B, C,
+                                          HW, T, io_dtype, scale, st)
+              : tc::word_attn_bwd_tc(images, we, mask, dctx, dctx_bs, dattn, dimages, part, ntiles, nullptr, B, C, HW, T,
+                                     io_dtype, scale, st);
     if (rc) return rc;
   } else {
-    AGB_DISPATCH_TMAX(tm, {
-      constexpr int VV = TMAX <= 24 ? 2 : 1;
-      if (io_dtype == AGB_F32) rc = launch_bwd<float, TMAX, VV>(images, we, mask, dctx, dctx_bs, dattn, dimages, part, B, C, HW, T, scale, use_tma, st);
-      else if (io_dtype == AGB_BF16) rc = launch_bwd<__nv_bfloat16, TMAX, VV>(images, we, mask, dctx, dctx_bs, dattn, dimages, part, B, C, HW, T, scale, use_tma, st);
-      else rc = launch_bwd<__half, TMAX, VV>(images, we, mask, dctx, dctx_bs, dattn, dimages, part, B, C, HW, T, scale, use_tma, st);
-    });
+#define AGB_BWD_LAYOUT(L)                                                                                                   \
+    AGB_DISPATCH_TMAX(tm, {                                                                                                 \
+      constexpr int VV = TMAX <= 24 ? 2 : 1;                                                                                \
+      if (io_dtype == AGB_F32) rc = launch_bwd<float, TMAX, VV, L>(images, we, mask, dctx, dctx_bs, dctx_ps, dattn, dimages, part, B, C, HW, T, scale, use_tma, st); \
+      else if (io_dtype == AGB_BF16) rc = launch_bwd<__nv_bfloat16, TMAX, VV, L>(images, we, mask, dctx, dctx_bs, dctx_ps, dattn, dimages, part, B, C, HW, T, scale, use_tma, st); \
+      else rc = launch_bwd<__half, TMAX, VV, L>(images, we, mask, dctx, dctx_bs, dctx_ps, dattn, dimages, part, B, C, HW, T, scale, use_tma, st); \
+    })
+    if (nhwc) AGB_BWD_LAYOUT(true) else AGB_BWD_LAYOUT(false)
+#undef AGB_BWD_LAYOUT
     if (rc) return rc;
   }
   // one CTA per sample: dwe[b] = sum of the partial slots; dwords[b][e,t] = sum_c W[c,e] dwe[b][c,t];
@@ -723,4 +927,25 @@ extern "C" int agb_word_attn_bwd(const void* images, const float* words, int64_t
     if ((rc = check_launch("sum_partials_kernel"))) return rc;
   }
   return 0;
+}
+
+extern "C" int agb_word_attn_bwd(const void* images, const float* words, int64_t ws_b, int64_t ws_e,
+                                 int64_t ws_t, const float* conv_w, const int64_t* mask,
+                                 const float* we, const void* dctx, int64_t dctx_bs, const void* dattn,
+                                 void* dimages, float* dwords, float* dconv_w, void* workspace,
+                                 size_t workspace_bytes, int B, int C, int HW, int E, int T,
+                                 int io_dtype, int scaled, void* stream) {
+  return word_attn_bwd_impl(false, images, words, ws_b, ws_e, ws_t, conv_w, mask, we, dctx, dctx_bs, 0, dattn, dimages,
+                            dwords, dconv_w, workspace, workspace_bytes, B, C, HW, E, T, io_dtype, scaled, stream);
+}
+
+extern "C" int agb_word_attn_bwd_nhwc(const void* images, const float* words, int64_t ws_b, int64_t ws_e,
+                                      int64_t ws_t, const float* conv_w, const int64_t* mask,
+                                      const float* we, const void* dctx, int64_t dctx_bs, int64_t dctx_ps,
+                                      const void* dattn, void* dimages, float* dwords, float* dconv_w,
+                                      void* workspace, size_t workspace_bytes, int B, int C, int HW, int E, int T,
+                                      int io_dtype, int scaled, void* stream) {
+  return word_attn_bwd_impl(true, images, words, ws_b, ws_e, ws_t, conv_w, mask, we, dctx, dctx_bs, dctx_ps, dattn,
+                            dimages, dwords, dconv_w, workspace, workspace_bytes, B, C, HW, E, T, io_dtype, scaled,
+                            stream);
 }

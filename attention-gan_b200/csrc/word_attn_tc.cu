@@ -45,6 +45,30 @@ __device__ __forceinline__ uint64_t make_desc_sw128_mn_lbo(uint32_t smem_addr, u
   return d;
 }
 
+// ---- channels_last (NHWC) tiles ----
+// A tile of 128 pixels x C channels is C/16 slabs of [128 px][16 ch] (32-byte rows, SWIZZLE_32B, 4 KB each),
+// loaded by a 3-D TMA over (channel, pixel, sample), so pixels past the end of a sample read as zeros.
+// Slab k holds channels 16k..16k+15: for a GEMM that contracts over channels it is the K-major operand of one
+// K = 16 step; for a GEMM that contracts over pixels the slabs side by side are an MN-major operand (16
+// channels per 32-byte row, 8-pixel groups 256 B apart, next 16 channels one slab = 4 KB further).
+constexpr int kSlabBytes = 128 * 32;
+__device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1,
+                                            int c2) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+      ::"r"(smem_u32(smem_dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
+      : "memory");
+}
+__device__ __forceinline__ uint64_t make_desc_sw32(uint32_t smem_addr, uint32_t lbo_bytes) {
+  uint64_t d = 0;
+  d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
+  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;   // MN-major: next 16 MN elements (K-major: ignored)
+  d |= (uint64_t)(256 >> 4) << 32;                     // next group of 8 rows
+  d |= (uint64_t)1 << 46;
+  d |= (uint64_t)6 << 61;                              // SWIZZLE_32B
+  return d;
+}
+
 template <typename T16> __device__ __forceinline__ T16 f2h(float v);
 template <> __device__ __forceinline__ __half f2h<__half>(float v) { return __float2half_rn(v); }
 template <> __device__ __forceinline__ __nv_bfloat16 f2h<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
@@ -67,6 +91,7 @@ struct AttnFwdParams {
   int tiles, ctas_per_sample;
   int stages;             // h-tile ring depth of the forward kernel
   int dbg;                // ablation switches for tuning (AGB_ATTN_DEBUG): 1 = no ctx stores, 2 = no attn stores
+  int64_t ctx_ps;         // NHWC: pixel stride of ctx
 };
 
 constexpr int kAttnStages = 3;
@@ -183,7 +208,9 @@ __device__ __forceinline__ Segment next_segment(long long g, long long g1, int t
   return s;
 }
 
-template <typename IO, int NT, int TL, int CT>
+// kNHWC: channels_last maps.  The h tile is C/16 K-major slabs (see kSlabBytes), and the output warps read
+// ctx and the packed attention maps thread = pixel and store each pixel's contiguous C-vector and T-row.
+template <typename IO, int NT, int TL, int CT, bool kNHWC = false>
 __global__ void __launch_bounds__(kFwdThreads, (fwd_min_ctas<NT, CT>()))
 word_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const AttnFwdParams p) {
   constexpr int KB = TL / 8;
@@ -255,8 +282,14 @@ word_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const AttnFwdP
           const int s = it % nst, use = it / nst;
           mbar_wait(&h_empty[s], (use & 1) ^ 1);
           mbar_expect_tx(&h_full[s], (uint32_t)stage_bytes);
-          tma_load_2d(sH + s * stage_bytes, &mapH, &h_full[s], (sg.tile0 + i) * 128, sg.b * C);
-          tma_load_2d(sH + s * stage_bytes + box_bytes, &mapH, &h_full[s], (sg.tile0 + i) * 128 + 64, sg.b * C);
+          if constexpr (kNHWC) {
+#pragma unroll
+            for (int k = 0; k < C / 16; ++k)
+              tma_load_3d(sH + s * stage_bytes + k * kSlabBytes, &mapH, &h_full[s], 16 * k, (sg.tile0 + i) * 128, sg.b);
+          } else {
+            tma_load_2d(sH + s * stage_bytes, &mapH, &h_full[s], (sg.tile0 + i) * 128, sg.b * C);
+            tma_load_2d(sH + s * stage_bytes + box_bytes, &mapH, &h_full[s], (sg.tile0 + i) * 128 + 64, sg.b * C);
+          }
         }
         g += sg.n;
       }
@@ -323,9 +356,16 @@ word_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const AttnFwdP
               umma_f16(tmem + u * bufc, d_ones, d_bias, idesc1, 0u);            // S = 0 / -inf per word
 #pragma unroll
               for (int kk = 0; kk < ks1; ++kk) {
+                if constexpr (kNHWC) {
+                  constexpr uint32_t idesc1k = make_idesc(128, NT, fmt_io);                // A K-major (channels contiguous)
+                  const uint64_t da = make_desc_sw32(a0 + kk * kSlabBytes, 0u);
+                  umma_f16(tmem + u * bufc, da, make_desc_sw128(smem_u32(sB1hi)) + 2 * kk, idesc1k, 1u);
+                  umma_f16(tmem + u * bufc, da, make_desc_sw128(smem_u32(sB1lo)) + 2 * kk, idesc1k, 1u);
+                } else {
                 const uint64_t da = make_desc_sw128_mn_lbo(a0 + kk * 2048, (uint32_t)box_bytes);
                 umma_f16(tmem + u * bufc, da, make_desc_sw128(smem_u32(sB1hi)) + 2 * kk, idesc1, 1u);
                 umma_f16(tmem + u * bufc, da, make_desc_sw128(smem_u32(sB1lo)) + 2 * kk, idesc1, 1u);
+                }
               }
               umma_commit(&h_empty[s]);
               umma_commit(&s_full[u]);
@@ -418,6 +458,61 @@ word_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const AttnFwdP
             if (lane == 0) mbar_arrive(&c_empty[u]);
             continue;
           }
+          if constexpr (kNHWC) {
+            // thread = pixel: its C context values and its T probabilities go to this warp's staging rows
+            // ([32 px][C] and [32 px][T], 16-bit), TMEM read 16 columns at a time so the live set fits the 64
+            // registers of three CTAs per SM; the warp then copies its 32 pixels out with 16-byte accesses on
+            // consecutive addresses (a warp's maps are one contiguous block, its contexts C-vectors ctx_ps apart)
+            unsigned char* wc = sStC + q * (32 * C * 2);
+            unsigned char* wa = sStA + q * (32 * TL * 2);
+#pragma unroll
+            for (int c0 = 0; c0 < C; c0 += 16) {
+              float cv[16];
+              tmem_ld16(tmem + lane0 + u * bufc + NT + c0, cv);
+              tmem_ld_wait();
+#pragma unroll
+              for (int c = 0; c < 16; c += 8)
+                *reinterpret_cast<uint4*>(wc + (lane * C + c0 + c) * 2) =
+                    make_uint4(pack2<IO>(cv[c], cv[c + 1]), pack2<IO>(cv[c + 2], cv[c + 3]),
+                               pack2<IO>(cv[c + 4], cv[c + 5]), pack2<IO>(cv[c + 6], cv[c + 7]));
+            }
+            if (attn != nullptr) {
+              float pv[TL / 2];
+              tmem_ld_n<TL / 2>(tmem + lane0 + u * bufc + kAttnCol, pv);
+              tmem_ld_wait();
+              unsigned char* row = wa + lane * p.T * 2;
+              if ((p.T & 1) == 0) {
+#pragma unroll
+                for (int t = 0; t < TL; t += 2)
+                  if (t < p.T) *reinterpret_cast<uint32_t*>(row + t * 2) = __float_as_uint(pv[t / 2]);
+              } else {           // odd T: rows are 2-byte aligned only
+#pragma unroll
+                for (int t = 0; t < TL; t += 2) {
+                  const uint32_t pr = __float_as_uint(pv[t / 2]);
+                  if (t < p.T) *reinterpret_cast<uint16_t*>(row + t * 2) = (uint16_t)(pr & 0xffffu);
+                  if (t + 1 < p.T) *reinterpret_cast<uint16_t*>(row + t * 2 + 2) = (uint16_t)(pr >> 16);
+                }
+              }
+            }
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&c_empty[u]);
+            const int pix0 = (sg.tile0 + j) * 128 + q * 32;
+            const int nvp = max(0, min(32, p.HW - pix0));         // a multiple of 8 (HW % 8 == 0)
+            if (!AGB_ABL(p, 1)) {
+              for (int i = lane; i < nvp * (C / 8); i += 32) {
+                const int px = i / (C / 8), part = i - px * (C / 8);
+                *reinterpret_cast<uint4*>(ctx + (size_t)(pix0 + px) * p.ctx_ps + part * 8) =
+                    *reinterpret_cast<const uint4*>(wc + i * 16);
+              }
+            }
+            if (attn != nullptr && !AGB_ABL(p, 2)) {
+              uint4* dst = reinterpret_cast<uint4*>(attn + (size_t)pix0 * p.T);   // 16-byte aligned: pix0 % 8 == 0
+              for (int i = lane; i < nvp * p.T / 8; i += 32) dst[i] = *reinterpret_cast<const uint4*>(wa + i * 16);
+            }
+            __syncwarp();
+            continue;
+          }
           float w[2][4 * (C / 8)];
           uint32_t pa[2][2 * KB];
           tmem_ld_frag<C / 8>(tmem + lane0 + u * bufc + NT, w[0]);
@@ -476,7 +571,36 @@ word_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const AttnFwdP
   if (warp == 0) tmem_dealloc(tmem, tmem_cols);
 }
 
-template <typename IO, int CT>
+// 3-D map of a channels_last 16-bit tensor: element (c, p, b) at base + (c + p*ps + b*bs) elements; box =
+// one [128 px][16 ch] slab, SWIZZLE_32B; pixels p >= HW (the tail of a sample's last tile) read as zeros
+static int make_tmap_nhwc(CUtensorMap* map, const void* base, int C, int HW, int B, int64_t ps, int64_t bs, bool bf16) {
+  static EncodeTiledFn encode = nullptr;
+  if (!encode) {
+    void* fn = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
+    if (e != cudaSuccess || fn == nullptr) {
+      set_error("cuTensorMapEncodeTiled entry point unavailable: %s", cudaGetErrorString(e));
+      return e != cudaSuccess ? (int)e : (int)cudaErrorUnknown;
+    }
+    encode = (EncodeTiledFn)fn;
+  }
+  const cuuint64_t gdim[3] = {(cuuint64_t)C, (cuuint64_t)HW, (cuuint64_t)B};
+  const cuuint64_t gstride[2] = {(cuuint64_t)ps * 2, (cuuint64_t)bs * 2};
+  const cuuint32_t box[3] = {16, 128, 1};
+  const cuuint32_t estr[3] = {1, 1, 1};
+  CUresult r = encode(map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3,
+                      const_cast<void*>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                      CU_TENSOR_MAP_SWIZZLE_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_error("cuTensorMapEncodeTiled (NHWC) failed with CUresult %d (C=%d HW=%d B=%d ps=%lld bs=%lld)", (int)r, C, HW,
+              B, (long long)ps, (long long)bs);
+    return (int)cudaErrorInvalidValue;
+  }
+  return 0;
+}
+
+template <typename IO, int CT, bool kNHWC>
 static int launch_attn_fwd_tc_c(const CUtensorMap& mapH, const AttnFwdParams& p_in, int sms, cudaStream_t st) {
   const int NT = p_in.T <= 32 ? 32 : 64;
   const int TL = (p_in.T + 7) / 8 * 8;
@@ -494,7 +618,7 @@ static int launch_attn_fwd_tc_c(const CUtensorMap& mapH, const AttnFwdParams& p_
     grid = (int)std::min<long long>(options().attn_fwd_ctas, (long long)p.B * p.tiles);
 #define AGB_ATTN_FWD_CASE(NTV, TLV)                                                              \
   {                                                                                               \
-    auto kern = word_attn_fwd_tc_kernel<IO, NTV, TLV, CT>;                                        \
+    auto kern = word_attn_fwd_tc_kernel<IO, NTV, TLV, CT, kNHWC>;                                 \
     AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));      \
     kern<<<grid, kFwdThreads, smem, st>>>(mapH, p);                                               \
   }
@@ -512,20 +636,22 @@ static int launch_attn_fwd_tc_c(const CUtensorMap& mapH, const AttnFwdParams& p_
   return 0;
 }
 
-template <typename IO>
+template <typename IO, bool kNHWC = false>
 static int launch_attn_fwd_tc(const void* images, const AttnFwdParams& p, cudaStream_t st) {
   CUtensorMap mapH;
-  if (int rc = make_tmap_2d(&mapH, images, (uint64_t)p.B * p.C, (uint64_t)p.HW, (uint32_t)p.C,
-                            std::is_same<IO, __nv_bfloat16>::value))
+  if (int rc = kNHWC ? make_tmap_nhwc(&mapH, images, p.C, p.HW, p.B, p.C, (int64_t)p.HW * p.C,
+                                      std::is_same<IO, __nv_bfloat16>::value)
+                     : make_tmap_2d(&mapH, images, (uint64_t)p.B * p.C, (uint64_t)p.HW, (uint32_t)p.C,
+                                    std::is_same<IO, __nv_bfloat16>::value))
     return rc;
   const int sms = device_sms();
   const int slot = prof_begin(PROF_ATTN_FWD, st);
   int rc = 0;
   switch (p.C) {
-    case 16: rc = launch_attn_fwd_tc_c<IO, 16>(mapH, p, sms, st); break;
-    case 32: rc = launch_attn_fwd_tc_c<IO, 32>(mapH, p, sms, st); break;
-    case 48: rc = launch_attn_fwd_tc_c<IO, 48>(mapH, p, sms, st); break;
-    default: rc = launch_attn_fwd_tc_c<IO, 64>(mapH, p, sms, st); break;
+    case 16: rc = launch_attn_fwd_tc_c<IO, 16, kNHWC>(mapH, p, sms, st); break;
+    case 32: rc = launch_attn_fwd_tc_c<IO, 32, kNHWC>(mapH, p, sms, st); break;
+    case 48: rc = launch_attn_fwd_tc_c<IO, 48, kNHWC>(mapH, p, sms, st); break;
+    default: rc = launch_attn_fwd_tc_c<IO, 64, kNHWC>(mapH, p, sms, st); break;
   }
   if (rc) return rc;
   prof_end(slot, st);
@@ -576,7 +702,10 @@ constexpr int kMaxBwdStages = 4;
 // TMEM columns per tile buffer u (UB = 2 NT + 32):  [0,NT) S -> ds hi | ds lo (bf16 pairs, NT/2 columns each),
 // [NT,2NT) G -> a (pairs, TL/2 columns) | ds in fp16 (fp16 maps, at NT + NT/2), [2NT, 2NT+32) dh;  the d(W.e)
 // accumulator [a part | ds part] (2 TL columns) follows the two buffers at 2 UB.
-template <typename IO, int NT, int TL, int CT>
+// kNHWC: channels_last maps.  A stage is [dctx slabs | h slabs] (see kSlabBytes): K-major A operands of GEMM1,
+// and side by side the MN-major A operand [dctx channels; h channels] x pixels of GEMM4.  dattn rows and dh
+// are read / written thread = pixel.
+template <typename IO, int NT, int TL, int CT, bool kNHWC = false>
 __global__ void __launch_bounds__(kBwdThreads, NT <= 32 ? 2 : 1)
 word_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const __grid_constant__ CUtensorMap mapD,
                         const AttnBwdParams p) {
@@ -655,10 +784,18 @@ word_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const __grid_c
           mbar_wait(&in_empty[s], (use & 1) ^ 1);
           mbar_expect_tx(&in_full[s], (uint32_t)stage_bytes);
           unsigned char* st = sIn + s * stage_bytes;
+          if constexpr (kNHWC) {
+#pragma unroll
+            for (int k = 0; k < C / 16; ++k) {
+              tma_load_3d(st + k * kSlabBytes, &mapD, &in_full[s], 16 * k, px0, sg.b);
+              tma_load_3d(st + (C / 16 + k) * kSlabBytes, &mapH, &in_full[s], 16 * k, px0, sg.b);
+            }
+          } else {
           tma_load_2d(st, &mapD, &in_full[s], px0, sg.b * p.d_rows);
           tma_load_2d(st + box, &mapH, &in_full[s], px0, sg.b * C);
           tma_load_2d(st + 2 * box, &mapD, &in_full[s], px0 + 64, sg.b * p.d_rows);
           tma_load_2d(st + 3 * box, &mapH, &in_full[s], px0 + 64, sg.b * C);
+          }
         }
         g += sg.n;
       }
@@ -718,12 +855,22 @@ word_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const __grid_c
               umma_f16(tmem + u * UB, d_ones, d_bias, idesc1, 0u);        // S = 0 / -inf per word
 #pragma unroll
               for (int kk = 0; kk < ks1; ++kk) {
+                if constexpr (kNHWC) {
+                  constexpr uint32_t idesc1k = make_idesc(128, NT, fmt_io);                          // A K-major
+                  const uint64_t dh_ = make_desc_sw32(st + (C / 16 + kk) * kSlabBytes, 0u);           // h
+                  const uint64_t dd_ = make_desc_sw32(st + kk * kSlabBytes, 0u);                      // dctx
+                  umma_f16(tmem + u * UB, dh_, make_desc_sw128(smem_u32(sB1s)) + 2 * kk, idesc1k, 1u);
+                  umma_f16(tmem + u * UB, dh_, make_desc_sw128(smem_u32(sB1s + NT * 128)) + 2 * kk, idesc1k, 1u);
+                  umma_f16(tmem + u * UB + NT, dd_, make_desc_sw128(smem_u32(sB1u)) + 2 * kk, idesc1k, kk ? 1u : 0u);
+                  umma_f16(tmem + u * UB + NT, dd_, make_desc_sw128(smem_u32(sB1u + NT * 128)) + 2 * kk, idesc1k, 1u);
+                } else {
                 const uint64_t dh_ = make_desc_sw128_mn_lbo(st + box + kk * 2048, (uint32_t)(2 * box));    // h
                 const uint64_t dd_ = make_desc_sw128_mn_lbo(st + kk * 2048, (uint32_t)(2 * box));          // dctx
                 umma_f16(tmem + u * UB, dh_, make_desc_sw128(smem_u32(sB1s)) + 2 * kk, idesc1, 1u);
                 umma_f16(tmem + u * UB, dh_, make_desc_sw128(smem_u32(sB1s + NT * 128)) + 2 * kk, idesc1, 1u);
                 umma_f16(tmem + u * UB + NT, dd_, make_desc_sw128(smem_u32(sB1u)) + 2 * kk, idesc1, kk ? 1u : 0u);
                 umma_f16(tmem + u * UB + NT, dd_, make_desc_sw128(smem_u32(sB1u + NT * 128)) + 2 * kk, idesc1, 1u);
+                }
               }
               umma_commit(&s_full[u]);
               ++j1;
@@ -747,9 +894,17 @@ word_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const __grid_c
 #pragma unroll
               for (int j = 0; j < 2; ++j)                  // two chunks of 64 pixels
 #pragma unroll
-                for (int kk = 0; kk < 4; ++kk)
+                for (int kk = 0; kk < 4; ++kk) {
+                  if constexpr (kNHWC) {
+                    // [dctx; h] channels x 16 pixels: MN-major over the slabs (rows 2C..127 of M are not read back)
+                    constexpr uint32_t idesc4m = make_idesc(128, 2 * TL, fmt_io) | (1u << 15);
+                    umma_f16(tmem + kAccCol, make_desc_sw32(st + (4 * j + kk) * 512, (uint32_t)kSlabBytes),
+                             make_desc_sw128(bt + j * bt_box) + 2 * kk, idesc4m, (j2 | j | kk) ? 1u : 0u);
+                  } else {
                   umma_f16(tmem + kAccCol, make_desc_sw128(st + j * 2 * box) + 2 * kk,
                            make_desc_sw128(bt + j * bt_box) + 2 * kk, idesc4, (j2 | j | kk) ? 1u : 0u);
+                  }
+                }
               umma_commit(&in_empty[s]);
               ++j2;
             }
@@ -786,7 +941,7 @@ word_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const __grid_c
               const int pix = (sg.tile0 + j) * 128 + q * 32 + lane;
 #pragma unroll
               for (int t = 0; t < TL; ++t)
-                if (t < p.T && pix < p.HW) g[t] += to_f32(dattn[(size_t)t * p.HW + pix]);
+                if (t < p.T && pix < p.HW) g[t] += to_f32(dattn[kNHWC ? (size_t)pix * p.T + t : (size_t)t * p.HW + pix]);
             }
             float d4[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
@@ -855,7 +1010,8 @@ word_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const __grid_c
 #pragma unroll
               for (int t = 0; t < 16; ++t) {
                 if (c0 + t < TL) {
-                  if (dattn != nullptr && c0 + t < p.T && pix < p.HW) g[t] += to_f32(dattn[(size_t)(c0 + t) * p.HW + pix]);
+                  if (dattn != nullptr && c0 + t < p.T && pix < p.HW)
+                    g[t] += to_f32(dattn[kNHWC ? (size_t)pix * p.T + c0 + t : (size_t)(c0 + t) * p.HW + pix]);
                   s[c0 + t] *= inv;
                   d4[t & 3] = fmaf(s[c0 + t], g[t], d4[t & 3]);
                 }
@@ -875,8 +1031,9 @@ word_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const __grid_c
                   if (c0 + t < TL) {
                     float g0 = g[t], g1 = g[t + 1];
                     if (dattn != nullptr && pix < p.HW) {
-                      if (c0 + t < p.T) g0 += to_f32(dattn[(size_t)(c0 + t) * p.HW + pix]);
-                      if (c0 + t + 1 < p.T) g1 += to_f32(dattn[(size_t)(c0 + t + 1) * p.HW + pix]);
+                      if (c0 + t < p.T) g0 += to_f32(dattn[kNHWC ? (size_t)pix * p.T + c0 + t : (size_t)(c0 + t) * p.HW + pix]);
+                      if (c0 + t + 1 < p.T)
+                        g1 += to_f32(dattn[kNHWC ? (size_t)pix * p.T + c0 + t + 1 : (size_t)(c0 + t + 1) * p.HW + pix]);
                     }
                     const float d0 = s[c0 + t] * (g0 - dot), d1 = s[c0 + t + 1] * (g1 - dot);
                     const uint32_t h2 = pack2<__nv_bfloat16>(d0, d1);
@@ -928,6 +1085,31 @@ word_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapH, const __grid_c
           const int it = it0 + j, u = it & 1, k = it >> 1;
           mbar_wait(&dh_full[u], k & 1);
           tc_fence_after();
+          if constexpr (kNHWC) {
+            // thread = pixel: its C gradient values go to this warp's staging rows [32 px][C], then the warp
+            // copies its 32 pixels (one contiguous block of d images) out with 16-byte accesses
+            unsigned char* wd = sStD + (px >> 5) * (32 * C * 2);
+#pragma unroll
+            for (int c0 = 0; c0 < C; c0 += 16) {
+              float dv[16];
+              tmem_ld16(tmem + lane0 + u * UB + 2 * NT + c0, dv);
+              tmem_ld_wait();
+#pragma unroll
+              for (int c = 0; c < 16; c += 8)
+                *reinterpret_cast<uint4*>(wd + (lane * C + c0 + c) * 2) =
+                    make_uint4(pack2<IO>(dv[c], dv[c + 1]), pack2<IO>(dv[c + 2], dv[c + 3]),
+                               pack2<IO>(dv[c + 4], dv[c + 5]), pack2<IO>(dv[c + 6], dv[c + 7]));
+            }
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&dh_empty[u]);
+            const int pix0 = (sg.tile0 + j) * 128 + (px & ~31);
+            const int nvp = max(0, min(32, p.HW - pix0));
+            uint4* dst = reinterpret_cast<uint4*>((IO*)p.dh + ((size_t)b * p.HW + pix0) * C);
+            for (int i = lane; i < nvp * C / 8; i += 32) dst[i] = *reinterpret_cast<const uint4*>(wd + i * 16);
+            __syncwarp();
+            continue;
+          }
           float w[2][4 * (C / 8)];
           tmem_ld_frag<C / 8>(tmem + lane0 + u * UB + 2 * NT, w[0]);
           tmem_ld_frag<C / 8>(tmem + lane0 + kHalfLanes + u * UB + 2 * NT, w[1]);
@@ -1038,14 +1220,21 @@ __global__ void sum_range_partials_kernel(const float* __restrict__ part, int sl
   out[(size_t)b * n + i] = acc;
 }
 
-int word_attn_bwd_tc(const void* images, const float* we, const int64_t* mask, const void* dctx, int64_t dctx_bs,
-                     const void* dattn, void* dimages, float* part, int part_slots, float* dwe, int B, int C, int HW, int T, int io_dtype,
-                     float scale, cudaStream_t st) {
+// nhwc: channels_last maps, dctx with pixel stride dctx_ps
+static int word_attn_bwd_tc_run(bool nhwc, const void* images, const float* we, const int64_t* mask, const void* dctx,
+                                int64_t dctx_bs, int64_t dctx_ps, const void* dattn, void* dimages, float* part,
+                                int part_slots, float* dwe, int B, int C, int HW, int T, int io_dtype, float scale,
+                                cudaStream_t st) {
   const bool bf = io_dtype == AGB_BF16;
   CUtensorMap mapH, mapD;
-  if (int rc = make_tmap_2d(&mapH, images, (uint64_t)B * C, (uint64_t)HW, (uint32_t)C, bf)) return rc;
-  const int d_rows = (int)(dctx_bs / HW);
-  if (int rc = make_tmap_2d(&mapD, dctx, (uint64_t)(B - 1) * d_rows + C, (uint64_t)HW, (uint32_t)C, bf)) return rc;
+  const int d_rows = nhwc ? 0 : (int)(dctx_bs / HW);
+  if (nhwc) {
+    if (int rc = make_tmap_nhwc(&mapH, images, C, HW, B, C, (int64_t)HW * C, bf)) return rc;
+    if (int rc = make_tmap_nhwc(&mapD, dctx, C, HW, B, dctx_ps, dctx_bs, bf)) return rc;
+  } else {
+    if (int rc = make_tmap_2d(&mapH, images, (uint64_t)B * C, (uint64_t)HW, (uint32_t)C, bf)) return rc;
+    if (int rc = make_tmap_2d(&mapD, dctx, (uint64_t)(B - 1) * d_rows + C, (uint64_t)HW, (uint32_t)C, bf)) return rc;
+  }
   AttnBwdParams p;
   p.we = we; p.mask = mask; p.dattn = dattn; p.dh = dimages; p.part = part;
   p.B = B; p.C = C; p.HW = HW; p.T = T; p.scale = scale;
@@ -1065,12 +1254,14 @@ int word_attn_bwd_tc(const void* images, const float* we, const int64_t* mask, c
   const int smem = stages * 4 * C * 128 + fixed;
   const int grid = word_attn_bwd_tc_grid(B, HW, T);
   const int slot = prof_begin(PROF_ATTN_BWD, st);
-#define AGB_ATTN_BWD_LAUNCH(IOT, NTV, TLV, CTV)                                                    \
+#define AGB_ATTN_BWD_LAUNCH_L(IOT, NTV, TLV, CTV, L)                                              \
   {                                                                                               \
-    auto kern = word_attn_bwd_tc_kernel<IOT, NTV, TLV, CTV>;                                      \
+    auto kern = word_attn_bwd_tc_kernel<IOT, NTV, TLV, CTV, L>;                                   \
     AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));      \
     kern<<<grid, kBwdThreads, smem, st>>>(mapH, mapD, p);                                         \
   }
+#define AGB_ATTN_BWD_LAUNCH(IOT, NTV, TLV, CTV)                                                    \
+  if (nhwc) AGB_ATTN_BWD_LAUNCH_L(IOT, NTV, TLV, CTV, true) else AGB_ATTN_BWD_LAUNCH_L(IOT, NTV, TLV, CTV, false)
 #define AGB_ATTN_BWD_CASE2(TLV, CTV)                                                              \
   if (bf) AGB_ATTN_BWD_LAUNCH(__nv_bfloat16, 32, TLV, CTV) else AGB_ATTN_BWD_LAUNCH(__half, 32, TLV, CTV)
 #define AGB_ATTN_BWD_CASE(TLV)        \
@@ -1093,6 +1284,7 @@ int word_attn_bwd_tc(const void* images, const float* we, const int64_t* mask, c
     default: AGB_ATTN_BWD_LONG(64) break;
   }
 #undef AGB_ATTN_BWD_LAUNCH
+#undef AGB_ATTN_BWD_LAUNCH_L
 #undef AGB_ATTN_BWD_LONG
 #undef AGB_ATTN_BWD_CASE2
 #undef AGB_ATTN_BWD_CASE
@@ -1104,6 +1296,29 @@ int word_attn_bwd_tc(const void* images, const float* we, const int64_t* mask, c
   return check_launch("sum_range_partials_kernel");
 }
 
+int word_attn_bwd_tc(const void* images, const float* we, const int64_t* mask, const void* dctx, int64_t dctx_bs,
+                     const void* dattn, void* dimages, float* part, int part_slots, float* dwe, int B, int C, int HW, int T, int io_dtype,
+                     float scale, cudaStream_t st) {
+  return word_attn_bwd_tc_run(false, images, we, mask, dctx, dctx_bs, 0, dattn, dimages, part, part_slots, dwe, B, C, HW,
+                              T, io_dtype, scale, st);
+}
+
+int word_attn_bwd_tc_nhwc(const void* images, const float* we, const int64_t* mask, const void* dctx, int64_t dctx_bs,
+                          int64_t dctx_ps, const void* dattn, void* dimages, float* part, int part_slots, int B, int C,
+                          int HW, int T, int io_dtype, float scale, cudaStream_t st) {
+  return word_attn_bwd_tc_run(true, images, we, mask, dctx, dctx_bs, dctx_ps, dattn, dimages, part, part_slots, nullptr,
+                              B, C, HW, T, io_dtype, scale, st);
+}
+
+// NHWC takes the tensor-core kernels exactly where NCHW does (same dtype, C, T and HW rules, 16-byte aligned
+// images and gradient), so the two layouts give the same results; the TMA map additionally needs 16-byte pixel and
+// batch strides of dctx, which a channels_last tensor or its channel slice [:, C:] has whenever C % 16 == 0
+int word_attn_bwd_tc_supported_nhwc(const void* images, const void* dctx, int64_t dctx_bs, int64_t dctx_ps,
+                                    const void* dattn, int C, int HW, int T, int io_dtype) {
+  if (!word_attn_bwd_tc_supported(images, dctx, (int64_t)C * HW, dattn, C, HW, T, io_dtype)) return 0;
+  return dctx_ps % 8 == 0 && dctx_bs % 8 == 0;
+}
+
 // 1 when the tensor-core kernel can take this problem
 int word_attn_tc_supported(const void* images, int C, int HW, int T, int io_dtype) {
   if (io_dtype != AGB_BF16 && io_dtype != AGB_F16) return 0;
@@ -1112,10 +1327,34 @@ int word_attn_tc_supported(const void* images, int C, int HW, int T, int io_dtyp
   return 1;
 }
 
+// the forward's NHWC rule: the NCHW one, plus 16-byte aligned ctx vectors and attention maps (the epilogue copies
+// 16 bytes at a time)
+int word_attn_tc_supported_nhwc(const void* images, const void* ctx, int64_t ctx_bs, int64_t ctx_ps, const void* attn,
+                                int C, int HW, int T, int io_dtype) {
+  if (!word_attn_tc_supported(images, C, HW, T, io_dtype)) return 0;
+  return ((uintptr_t)ctx & 15) == 0 && ctx_ps % 8 == 0 && ctx_bs % 8 == 0 && ((uintptr_t)attn & 15) == 0;
+}
+
+int word_attn_fwd_tc_nhwc(const void* images, const float* we, const int64_t* mask, void* ctx, int64_t ctx_bs,
+                          int64_t ctx_ps, void* attn, int B, int C, int HW, int T, int io_dtype, float qscale,
+                          cudaStream_t st) {
+  AttnFwdParams p;
+  p.we = we; p.mask = mask; p.ctx = ctx; p.attn = attn; p.ctx_bs = ctx_bs; p.ctx_ps = ctx_ps;
+  p.B = B; p.C = C; p.HW = HW; p.T = T; p.qscale = qscale;
+  p.tiles = cdiv(HW, 128);
+  p.ctas_per_sample = 0;
+  p.dbg = 0;
+#ifdef AGB_ABLATION
+  if (const char* e = getenv("AGB_ATTN_DEBUG")) p.dbg = atoi(e);
+#endif
+  if (io_dtype == AGB_BF16) return launch_attn_fwd_tc<__nv_bfloat16, true>(images, p, st);
+  return launch_attn_fwd_tc<__half, true>(images, p, st);
+}
+
 int word_attn_fwd_tc(const void* images, const float* we, const int64_t* mask, void* ctx, int64_t ctx_bs, void* attn,
                      int B, int C, int HW, int T, int io_dtype, float qscale, cudaStream_t st) {
   AttnFwdParams p;
-  p.we = we; p.mask = mask; p.ctx = ctx; p.attn = attn; p.ctx_bs = ctx_bs;
+  p.we = we; p.mask = mask; p.ctx = ctx; p.attn = attn; p.ctx_bs = ctx_bs; p.ctx_ps = 0;
   p.B = B; p.C = C; p.HW = HW; p.T = T; p.qscale = qscale;
   p.tiles = cdiv(HW, 128);
   p.ctas_per_sample = 0;   // the forward kernel is persistent over all samples

@@ -58,16 +58,27 @@ class _WordAttention(torch.autograd.Function):
         return (dimages if need_img else None), dwords, dweight, None, None
 
 
+def _check_cat_out(images, out):
+    """`out` of forward_into: [B, 2C, H, W], the images' dtype and memory format (contiguous or channels_last)"""
+    B, C, H, W = images.shape
+    fmt = ops.attn_memory_format(images)
+    if out.shape != (B, 2 * C, H, W) or out.dtype != images.dtype or not out.is_contiguous(memory_format=fmt):
+        if fmt == torch.channels_last:
+            raise RuntimeError("forward_into: `out` must be a channels_last [B, 2*C, H, W] tensor of the images' "
+                               "dtype (the images are channels_last)")
+        raise RuntimeError("forward_into: `out` must be a contiguous [B, 2*C, H, W] tensor of the images' dtype")
+
+
 class _WordAttentionInto(torch.autograd.Function):
     """the same fused attention, writing  cat((images, context), 1)  into a caller-owned [B, 2C, H, W] buffer:
-    the context leaves the kernel at channel offset C (ctx batch stride 2C*H*W in the C ABI), so GenNextStage's
-    torch.cat (generator_submodules.py:116) costs one copy of `images` instead of re-reading and re-writing both"""
+    the context leaves the kernel at channel offset C (ctx batch stride 2C*H*W in the C ABI; for channels_last maps
+    also pixel stride 2C), so GenNextStage's torch.cat (generator_submodules.py:116) costs one copy of `images`
+    instead of re-reading and re-writing both"""
 
     @staticmethod
     def forward(ctx, images, words, weight, mask, scaled, out, want_attn):
         B, C, H, W = images.shape
-        if out.shape != (B, 2 * C, H, W) or out.dtype != images.dtype or not out.is_contiguous():
-            raise RuntimeError("forward_into: `out` must be a contiguous [B, 2*C, H, W] tensor of the images' dtype")
+        _check_cat_out(images, out)
         w32 = words if words.dtype == torch.float32 else words.float()
         wt = weight.reshape(weight.shape[0], -1)
         wt32 = (wt if wt.dtype == torch.float32 else wt.float()).contiguous()
@@ -93,9 +104,10 @@ class _WordAttentionInto(torch.autograd.Function):
         if dout is None:
             return None, None, None, None, None, None, None
         dout = dout.to(images.dtype)
-        if not dout.is_contiguous():
-            dout = dout.contiguous()
-        # d context is the second channel half of d out, read in place through its batch stride
+        fmt = ops.attn_memory_format(images)
+        if not dout.is_contiguous(memory_format=fmt):
+            dout = dout.contiguous(memory_format=fmt)
+        # d context is the second channel half of d out, read in place through its batch (and pixel) stride
         dimages, dwords, dweight = ops.word_attn_bwd(images, w32, wt32, m64, we, dout[:, C:],
                                                      None if dattn is None else dattn.to(images.dtype),
                                                      ctx.scaled, need_words, need_w)
@@ -132,7 +144,8 @@ class AttentionModule(nn.Module):
 
     def forward(self, images, words, scaled=True):
         """images [B, nc_in, H, W], words [B, emb_dim, T] -> (context [B, nc_in, H, W],
-        attn [B, T, H, W])."""
+        attn [B, T, H, W]).  images may be contiguous NCHW or channels_last; the outputs (and the gradient of
+        images) take its memory format."""
         if self.mask is None:
             # the reference dereferences self.mask unconditionally (attention.py:47,65)
             raise AttributeError("AttentionModule.forward called before apply_mask(mask)")
@@ -144,7 +157,8 @@ class AttentionModule(nn.Module):
         return _WordAttention.apply(images, words, self.conv1.weight, self.mask, bool(scaled))
 
     def forward_into(self, images, words, out, scaled=True, want_attn=True):
-        """images [B, C, H, W], words [B, E, T], out [B, 2C, H, W] (pre-allocated, contiguous) ->
+        """images [B, C, H, W], words [B, E, T], out [B, 2C, H, W] (pre-allocated, in the memory format of images:
+        contiguous, or channels_last for channels_last images) ->
         (out, attn [B, T, H, W] or None) with  out == torch.cat((images, context), 1)  -- what GenNextStage builds
         right after the attention call (generator_submodules.py:113-116).  Not part of the reference API."""
         if self.mask is None:
@@ -152,9 +166,7 @@ class AttentionModule(nn.Module):
         ops.require_cuda(images, words, self.conv1.weight, out)
         if torch.compiler.is_compiling():
             # the op returns a fresh buffer (custom ops do not write into their inputs' storage): one extra copy
-            B, C, H, W = images.shape
-            if out.shape != (B, 2 * C, H, W) or out.dtype != images.dtype or not out.is_contiguous():
-                raise RuntimeError("forward_into: `out` must be a contiguous [B, 2*C, H, W] tensor of the images' dtype")
+            _check_cat_out(images, out)
             res, attn = self.forward_cat(images, words, scaled, want_attn)
             return out.copy_(res), attn
         res, attn = _WordAttentionInto.apply(images, words, self.conv1.weight, self.mask, bool(scaled), out,
@@ -173,7 +185,8 @@ class AttentionModule(nn.Module):
             out, attn, _ = torch.ops.agb.word_attn_cat(images, w32, wt32, m64, bool(scaled), bool(want_attn))
             return out, (attn if want_attn else None)
         B, C, H, W = images.shape
-        out = torch.empty((B, 2 * C, H, W), dtype=images.dtype, device=images.device)
+        out = torch.empty((B, 2 * C, H, W), dtype=images.dtype, device=images.device,
+                          memory_format=ops.attn_memory_format(images))
         return self.forward_into(images, words, out, scaled, want_attn)
 
 

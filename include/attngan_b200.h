@@ -340,6 +340,30 @@ int agb_sent_cos_pairs_bwd(const float* cnn, const float* rnn, int Bi, int Bc, c
                            const int32_t* pair_cap, long long P, int D, float eps, const float* dscos, float* dcnn,
                            float* drnn, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Generator word-context attention on channels_last (NHWC) feature maps
+ *   agb_word_attn_fwd_nhwc / agb_word_attn_bwd_nhwc take the arguments of agb_word_attn_fwd /
+ *   agb_word_attn_bwd plus the pixel stride of ctx (ctx_ps) / of dctx (dctx_ps), in elements:
+ *     images  [B,HW,C]  io dtype, dense (a channels_last [B,C,h,w] tensor)
+ *     ctx     [B,HW,C]  element (b, p, c) at b*ctx_bs + p*ctx_ps + c; ctx_ps = C, or 2C for the channel slice
+ *                       [:, C:] of a channels_last [B,2C,h,w] concat buffer; ctx_bs >= HW*ctx_ps
+ *     attn    [B,HW,T]  io dtype, dense (a channels_last [B,T,h,w] tensor), or NULL
+ *     dctx    [B,HW,C]  as ctx, strides dctx_bs / dctx_ps;  dattn [B,HW,T] dense or NULL
+ *     dimages [B,HW,C]  dense out
+ *   Everything else (words, conv_w, mask, we, workspace, dwords, dconv_w), the limits and the behaviour are those
+ *   of the NCHW entries, and for the same inputs the results are bit for bit the same.  The bwd workspace size is
+ *   agb_word_attn_bwd_workspace_bytes.
+ * ---------------------------------------------------------------------------------------------- */
+int agb_word_attn_fwd_nhwc(const void* images, const float* words, int64_t ws_b, int64_t ws_e,
+                           int64_t ws_t, const float* conv_w, const int64_t* mask, void* ctx,
+                           int64_t ctx_bs, int64_t ctx_ps, void* attn, float* we, int B, int C, int HW, int E,
+                           int T, int io_dtype, int scaled, void* stream);
+int agb_word_attn_bwd_nhwc(const void* images, const float* words, int64_t ws_b, int64_t ws_e,
+                           int64_t ws_t, const float* conv_w, const int64_t* mask, const float* we,
+                           const void* dctx, int64_t dctx_bs, int64_t dctx_ps, const void* dattn, void* dimages,
+                           float* dwords, float* dconv_w, void* workspace, size_t workspace_bytes, int B,
+                           int C, int HW, int E, int T, int io_dtype, int scaled, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
