@@ -6,6 +6,13 @@ compiled call computes what the eager call computes, bit for bit.  The drop-ins 
 ``torch.compiler.is_compiling()``; eager calls keep going through their ``torch.autograd.Function``s and never
 enter the dispatcher (DESIGN.md §1).
 
+Each differentiable primitive (word attention, func_attention, the region head, the pair scores) has its op body
+(the impl) as a plain function of this module and its gradient formula as one ``*_setup`` / ``*_backward`` pair.
+The setup stores the backward kernel on ``ctx`` and the backward calls ``ctx.bwd``: the op's registered autograd
+binds it to ``torch.ops.agb.<bwd op>``, the eager ``autograd.Function``s bind it to the plain backward impl.  The
+kernel cannot be chosen with ``torch.compiler.is_compiling()`` inside the backward: AOTAutograd traces a registered
+backward after Dynamo has finished, where that returns False.
+
 * Schemas take tensors and scalars only; an optional output that is not asked for comes back as an empty tensor.
 * Every op has a fake kernel (shapes, dtypes, strides).  Workspace outputs are sized with the library's host
   queries, which are pure host code; registering the ops loads nothing (the library is opened at the first query).
@@ -19,6 +26,7 @@ enter the dispatcher (DESIGN.md §1).
 """
 from __future__ import annotations
 
+from functools import partial
 from typing import Optional, Tuple
 
 import torch
@@ -30,8 +38,9 @@ from . import ops
 _LIB = "agb"
 
 
-def _op(name: str, mutates_args=()):
-    return torch.library.custom_op(f"{_LIB}::{name}", mutates_args=mutates_args, device_types="cuda")
+def _op(name: str, fn=None, mutates_args=()):
+    """register fn as agb::<name> (a decorator without fn); the impl stays callable without the dispatcher"""
+    return torch.library.custom_op(f"{_LIB}::{name}", fn, mutates_args=mutates_args, device_types="cuda")
 
 
 def _none(t: Optional[Tensor], dev) -> Tensor:
@@ -56,7 +65,6 @@ def host_query(name: str, *args) -> int:
 # ------------------------------------------------------------------------------------------------
 # generator word-context attention
 # ------------------------------------------------------------------------------------------------
-@_op("word_attn_fwd")
 def word_attn_fwd(images: Tensor, words: Tensor, weight: Tensor, mask: Tensor, scaled: bool,
                   want_attn: bool) -> Tuple[Tensor, Tensor, Tensor]:
     """images [B,C,H,W] contiguous or channels_last, words [B,E,T] fp32, weight [C,E] fp32 contiguous, mask [B,T]
@@ -66,6 +74,9 @@ def word_attn_fwd(images: Tensor, words: Tensor, weight: Tensor, mask: Tensor, s
     return ctx, _none(attn, images.device), we
 
 
+_word_attn_fwd = _op("word_attn_fwd", word_attn_fwd)
+
+
 def _maps_like(images: Tensor, channels: int) -> Tensor:
     """a [B, channels, H, W] tensor in the memory format of the attention's images"""
     B, _, H, W = images.shape
@@ -73,7 +84,7 @@ def _maps_like(images: Tensor, channels: int) -> Tensor:
                        memory_format=ops.attn_memory_format(images))
 
 
-@word_attn_fwd.register_fake
+@_word_attn_fwd.register_fake
 def _(images, words, weight, mask, scaled, want_attn):
     B, C, H, W = images.shape
     T = words.shape[2]
@@ -81,19 +92,26 @@ def _(images, words, weight, mask, scaled, want_attn):
     return _maps_like(images, C), attn, images.new_empty((B, C, T), dtype=torch.float32)
 
 
-@_op("word_attn_cat")
-def word_attn_cat(images: Tensor, words: Tensor, weight: Tensor, mask: Tensor, scaled: bool,
-                  want_attn: bool) -> Tuple[Tensor, Tensor, Tensor]:
-    """word_attn_fwd writing cat((images, ctx), 1): (out [B,2C,H,W], attn or empty, we); the kernel writes the
-    context at channel offset C of the fresh buffer (AttentionModule.forward_into)"""
+def word_attn_into(out: Tensor, images: Tensor, words: Tensor, weight: Tensor, mask: Tensor, scaled: bool,
+                   want_attn: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """word_attn_fwd writing cat((images, ctx), 1) into out [B,2C,H,W] (the images' dtype and memory format):
+    (out, attn or empty, we); the kernel writes the context at channel offset C"""
     C = images.shape[1]
-    out = _maps_like(images, 2 * C)
     out[:, :C].copy_(images)
     _, attn, we = ops.word_attn_fwd(images, words, weight, mask, scaled, want_attn, ctx_out=out[:, C:])
     return out, _none(attn, images.device), we
 
 
-@word_attn_cat.register_fake
+def word_attn_cat(images: Tensor, words: Tensor, weight: Tensor, mask: Tensor, scaled: bool,
+                  want_attn: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """word_attn_into a fresh buffer (AttentionModule.forward_cat)"""
+    return word_attn_into(_maps_like(images, 2 * images.shape[1]), images, words, weight, mask, scaled, want_attn)
+
+
+_word_attn_cat = _op("word_attn_cat", word_attn_cat)
+
+
+@_word_attn_cat.register_fake
 def _(images, words, weight, mask, scaled, want_attn):
     B, C, H, W = images.shape
     T = words.shape[2]
@@ -101,7 +119,6 @@ def _(images, words, weight, mask, scaled, want_attn):
     return _maps_like(images, 2 * C), attn, images.new_empty((B, C, T), dtype=torch.float32)
 
 
-@_op("word_attn_bwd")
 def word_attn_bwd(images: Tensor, words: Tensor, weight: Tensor, mask: Tensor, we: Tensor, dctx: Tensor,
                   dattn: Optional[Tensor], scaled: bool, need_dwords: bool,
                   need_dweight: bool) -> Tuple[Tensor, Tensor, Tensor]:
@@ -110,7 +127,10 @@ def word_attn_bwd(images: Tensor, words: Tensor, weight: Tensor, mask: Tensor, w
     return di, _none(dw, images.device), _none(dwt, images.device)
 
 
-@word_attn_bwd.register_fake
+_word_attn_bwd = _op("word_attn_bwd", word_attn_bwd)
+
+
+@_word_attn_bwd.register_fake
 def _(images, words, weight, mask, we, dctx, dattn, scaled, need_dwords, need_dweight):
     B, C = images.shape[:2]
     E, T = words.shape[1], words.shape[2]
@@ -119,44 +139,49 @@ def _(images, words, weight, mask, we, dctx, dattn, scaled, need_dwords, need_dw
             images.new_empty((C, E) if need_dweight else (0,), **f32))
 
 
-def _word_attn_setup(ctx, inputs, output):
+def word_attn_setup(ctx, inputs, output, bwd):
+    """word_attn_fwd / word_attn_cat: inputs and output as the op's, bwd the word_attn_bwd to call"""
     images, words, weight, mask, scaled, want_attn = inputs
     ctx.save_for_backward(images, words, weight, mask, output[2])
     ctx.scaled = scaled
+    ctx.bwd = bwd
     ctx.mark_non_differentiable(output[2])
     if not want_attn:
         ctx.mark_non_differentiable(output[1])
     ctx.set_materialize_grads(False)
 
 
-def _word_attn_backward(ctx, dctx, dattn, _dwe):
+def word_attn_backward(ctx, dctx, dattn, _dwe):
     images, words, weight, mask, we = ctx.saved_tensors
     need_img, need_words, need_w = ctx.needs_input_grad[:3]
     if dctx is None:
         dctx = torch.zeros_like(images)
-    di, dw, dwt = torch.ops.agb.word_attn_bwd(images, words, weight, mask, we, dctx.to(images.dtype),
-                                              None if dattn is None else dattn.to(images.dtype), ctx.scaled,
-                                              need_words, need_w)
+    di, dw, dwt = ctx.bwd(images, words, weight, mask, we, dctx.to(images.dtype),
+                          None if dattn is None else dattn.to(images.dtype), ctx.scaled, need_words, need_w)
     return (di if need_img else None), (dw if need_words else None), (dwt if need_w else None), None, None, None
 
 
-def _word_attn_cat_backward(ctx, dout, dattn, _dwe):
+def word_attn_cat_backward(ctx, dout, dattn, _dwe):
     images, words, weight, mask, we = ctx.saved_tensors
     need_img, need_words, need_w = ctx.needs_input_grad[:3]
     if dout is None:
         return None, None, None, None, None, None
     C = images.shape[1]
-    dout = dout.to(images.dtype).contiguous(memory_format=ops.attn_memory_format(images))
+    dout = dout.to(images.dtype)
+    fmt = ops.attn_memory_format(images)
+    if not dout.is_contiguous(memory_format=fmt):
+        dout = dout.contiguous(memory_format=fmt)
     # d context is the second channel half of d out, read in place through its batch (and pixel) stride
-    di, dw, dwt = torch.ops.agb.word_attn_bwd(images, words, weight, mask, we, dout[:, C:],
-                                              None if dattn is None else dattn.to(images.dtype), ctx.scaled,
-                                              need_words, need_w)
-    di = di + dout[:, :C] if need_img else None                  # the identity half of the concatenation
-    return di, (dw if need_words else None), (dwt if need_w else None), None, None, None
+    di, dw, dwt = ctx.bwd(images, words, weight, mask, we, dout[:, C:],
+                          None if dattn is None else dattn.to(images.dtype), ctx.scaled, need_words, need_w)
+    if need_img:
+        di += dout[:, :C]                                        # the identity half of the concatenation
+    return (di if need_img else None), (dw if need_words else None), (dwt if need_w else None), None, None, None
 
 
-word_attn_fwd.register_autograd(_word_attn_backward, setup_context=_word_attn_setup)
-word_attn_cat.register_autograd(_word_attn_cat_backward, setup_context=_word_attn_setup)
+_word_attn_setup_op = partial(word_attn_setup, bwd=torch.ops.agb.word_attn_bwd)
+_word_attn_fwd.register_autograd(word_attn_backward, setup_context=_word_attn_setup_op)
+_word_attn_cat.register_autograd(word_attn_cat_backward, setup_context=_word_attn_setup_op)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -377,14 +402,16 @@ def _(cnn, rnn, pair_img, pair_cap, eps):
 
 # the differentiable pair scores (losses/pair_scores.py): the training forward returns its workspace, which the
 # backward reads and overwrites with its staging
-@_op("damsm_pairs_train_fwd")
 def damsm_pairs_train_fwd(img: Tensor, words: Tensor, cap_lens: Tensor, pair_img: Tensor, pair_cap: Tensor,
                           gamma1: float, gamma2: float, math: int) -> Tuple[Tensor, Tensor]:
     """(m [P], ws uint8) of the pair list (ops.damsm_pairs_train_fwd)"""
     return ops.damsm_pairs_train_fwd(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math)
 
 
-@damsm_pairs_train_fwd.register_fake
+_damsm_pairs_train_fwd = _op("damsm_pairs_train_fwd", damsm_pairs_train_fwd)
+
+
+@_damsm_pairs_train_fwd.register_fake
 def _(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math):
     Bi, D, R = img.shape
     Bc, _, T = words.shape
@@ -397,7 +424,6 @@ def _(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math):
     return img.new_empty((P,), dtype=torch.float32), _ws_like(nbytes, img)
 
 
-@_op("damsm_pairs_bwd", mutates_args=("ws",))
 def damsm_pairs_bwd(img: Tensor, words: Tensor, cap_lens: Tensor, pair_img: Tensor, pair_cap: Tensor, gamma1: float,
                     gamma2: float, math: int, dm: Tensor, ws: Tensor, need_dimg: bool,
                     need_dwords: bool) -> Tuple[Tensor, Tensor]:
@@ -408,56 +434,66 @@ def damsm_pairs_bwd(img: Tensor, words: Tensor, cap_lens: Tensor, pair_img: Tens
     return _none(dimg, img.device), _none(dwords, img.device)
 
 
-@damsm_pairs_bwd.register_fake
+_damsm_pairs_bwd = _op("damsm_pairs_bwd", damsm_pairs_bwd, mutates_args=("ws",))
+
+
+@_damsm_pairs_bwd.register_fake
 def _(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math, dm, ws, need_dimg, need_dwords):
     Bc, D, T = words.shape
     e = img.new_empty((0,), dtype=torch.float32)
     return (torch.empty_like(img) if need_dimg else e), (img.new_empty((Bc, T, D)) if need_dwords else e.clone())
 
 
-def _damsm_pairs_setup(ctx, inputs, output):
+_SECOND_BACKWARD = ("a second backward through the same pair scores is not supported (the first one released the "
+                   "training workspace); compute the scores again")
+
+
+def damsm_pairs_setup(ctx, inputs, output, bwd):
+    """damsm_pairs_train_fwd: inputs and output as the op's, bwd the damsm_pairs_bwd to call"""
     img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math = inputs
     ctx.save_for_backward(img, words, cap_lens, pair_img, pair_cap)
     ctx.ws = output[1]
     ctx.cfg = (gamma1, gamma2, math)
+    ctx.bwd = bwd
     ctx.mark_non_differentiable(output[1])
     ctx.set_materialize_grads(False)
 
 
-def _damsm_pairs_backward(ctx, dm, _dws):
+def damsm_pairs_backward(ctx, dm, _dws):
     img, words, cap_lens, pair_img, pair_cap = ctx.saved_tensors
     gamma1, gamma2, math = ctx.cfg
     need_img, need_words = ctx.needs_input_grad[:2]
     dimg = dwords = None
     if dm is not None and (need_img or need_words):
         if ctx.ws is None:
-            raise RuntimeError("agb::damsm_pairs_train_fwd: a second backward is not supported (the first one "
-                               "released the training workspace)")
-        di, dw = torch.ops.agb.damsm_pairs_bwd(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math,
-                                               dm.contiguous(), ctx.ws, need_img, need_words)
+            raise RuntimeError(_SECOND_BACKWARD)
+        di, dw = ctx.bwd(img, words, cap_lens, pair_img, pair_cap, gamma1, gamma2, math, dm.float().contiguous(),
+                         ctx.ws, need_img, need_words)
         dimg = di if need_img else None
         dwords = dw.transpose(1, 2) if need_words else None           # [Bc,D,T] view like words
-    ctx.ws = None
+    ctx.ws = None                                 # the saved vectors are not needed again: free them now
     return dimg, dwords, None, None, None, None, None, None
 
 
-damsm_pairs_train_fwd.register_autograd(_damsm_pairs_backward, setup_context=_damsm_pairs_setup)
+_damsm_pairs_train_fwd.register_autograd(damsm_pairs_backward,
+                                         setup_context=partial(damsm_pairs_setup, bwd=torch.ops.agb.damsm_pairs_bwd))
 
 
-@_op("sent_cos_pairs_train_fwd")
 def sent_cos_pairs_train_fwd(cnn: Tensor, rnn: Tensor, pair_img: Tensor, pair_cap: Tensor, eps: float) -> Tensor:
     """cosine [P] of the pair list, the values of sent_cos_pairs_fwd, with a registered backward"""
     return ops.sent_cos_pairs_fwd(cnn, rnn, pair_img, pair_cap, eps)
 
 
-@sent_cos_pairs_train_fwd.register_fake
+_sent_cos_pairs_train_fwd = _op("sent_cos_pairs_train_fwd", sent_cos_pairs_train_fwd)
+
+
+@_sent_cos_pairs_train_fwd.register_fake
 def _(cnn, rnn, pair_img, pair_cap, eps):
     if pair_cap.shape[0] != pair_img.shape[0]:
         raise RuntimeError(f"pair_img has {pair_img.shape[0]} entries, pair_cap {pair_cap.shape[0]}")
     return cnn.new_empty((pair_img.shape[0],), dtype=torch.float32)
 
 
-@_op("sent_cos_pairs_bwd")
 def sent_cos_pairs_bwd(cnn: Tensor, rnn: Tensor, pair_img: Tensor, pair_cap: Tensor, eps: float, dscos: Tensor,
                        need_dcnn: bool, need_drnn: bool) -> Tuple[Tensor, Tensor]:
     """(dcnn or empty, drnn or empty)"""
@@ -465,46 +501,52 @@ def sent_cos_pairs_bwd(cnn: Tensor, rnn: Tensor, pair_img: Tensor, pair_cap: Ten
     return _none(dcnn, cnn.device), _none(drnn, cnn.device)
 
 
-@sent_cos_pairs_bwd.register_fake
+_sent_cos_pairs_bwd = _op("sent_cos_pairs_bwd", sent_cos_pairs_bwd)
+
+
+@_sent_cos_pairs_bwd.register_fake
 def _(cnn, rnn, pair_img, pair_cap, eps, dscos, need_dcnn, need_drnn):
     e = cnn.new_empty((0,), dtype=torch.float32)
     return (torch.empty_like(cnn) if need_dcnn else e), (torch.empty_like(rnn) if need_drnn else e.clone())
 
 
-def _sent_cos_pairs_setup(ctx, inputs, output):
+def sent_cos_pairs_setup(ctx, inputs, output, bwd):
+    """sent_cos_pairs_train_fwd: inputs and output as the op's, bwd the sent_cos_pairs_bwd to call"""
     cnn, rnn, pair_img, pair_cap, eps = inputs
     ctx.save_for_backward(cnn, rnn, pair_img, pair_cap)
     ctx.eps = eps
+    ctx.bwd = bwd
 
 
-def _sent_cos_pairs_backward(ctx, dscos):
+def sent_cos_pairs_backward(ctx, dscos):
     cnn, rnn, pair_img, pair_cap = ctx.saved_tensors
     need_c, need_r = ctx.needs_input_grad[:2]
-    dc, dr = torch.ops.agb.sent_cos_pairs_bwd(cnn, rnn, pair_img, pair_cap, ctx.eps, dscos.contiguous(), need_c,
-                                              need_r)
+    dc, dr = ctx.bwd(cnn, rnn, pair_img, pair_cap, ctx.eps, dscos.float().contiguous(), need_c, need_r)
     return (dc if need_c else None), (dr if need_r else None), None, None, None
 
 
-sent_cos_pairs_train_fwd.register_autograd(_sent_cos_pairs_backward, setup_context=_sent_cos_pairs_setup)
+_sent_cos_pairs_train_fwd.register_autograd(
+    sent_cos_pairs_backward, setup_context=partial(sent_cos_pairs_setup, bwd=torch.ops.agb.sent_cos_pairs_bwd))
 
 
 # ------------------------------------------------------------------------------------------------
 # functional region-word attention
 # ------------------------------------------------------------------------------------------------
-@_op("func_attention_fwd")
 def func_attention_fwd(query: Tensor, context: Tensor, gamma1: float, scaled: bool) -> Tuple[Tensor, Tensor]:
     """query [B,D,L] fp32, context [B,D,R] fp32 contiguous -> (wc [B,D,L], attn [B,L,R])"""
     return ops.func_attention_fwd(query, context, gamma1, scaled)
 
 
-@func_attention_fwd.register_fake
+_func_attention_fwd = _op("func_attention_fwd", func_attention_fwd)
+
+
+@_func_attention_fwd.register_fake
 def _(query, context, gamma1, scaled):
     B, D, L = query.shape
     return query.new_empty((B, D, L), dtype=torch.float32), query.new_empty((B, L, context.shape[2]),
                                                                             dtype=torch.float32)
 
 
-@_op("func_attention_bwd")
 def func_attention_bwd(query: Tensor, context: Tensor, gamma1: float, scaled: bool, dwc: Tensor,
                        dattn: Optional[Tensor], need_dquery: bool, need_dcontext: bool) -> Tuple[Tensor, Tensor]:
     """(dquery [B,D,L] or empty, dcontext [B,D,R] or empty)"""
@@ -512,7 +554,10 @@ def func_attention_bwd(query: Tensor, context: Tensor, gamma1: float, scaled: bo
     return _none(dq, query.device), _none(dc, query.device)
 
 
-@func_attention_bwd.register_fake
+_func_attention_bwd = _op("func_attention_bwd", func_attention_bwd)
+
+
+@_func_attention_bwd.register_fake
 def _(query, context, gamma1, scaled, dwc, dattn, need_dquery, need_dcontext):
     B, D, L = query.shape
     f32 = dict(dtype=torch.float32)
@@ -520,24 +565,27 @@ def _(query, context, gamma1, scaled, dwc, dattn, need_dquery, need_dcontext):
             query.new_empty((B, D, context.shape[2]) if need_dcontext else (0,), **f32))
 
 
-def _func_attention_setup(ctx, inputs, output):
+def func_attention_setup(ctx, inputs, output, bwd):
+    """func_attention_fwd: inputs and output as the op's, bwd the func_attention_bwd to call"""
     query, context, gamma1, scaled = inputs
     ctx.save_for_backward(query, context)
     ctx.cfg = (gamma1, scaled)
+    ctx.bwd = bwd
     ctx.set_materialize_grads(False)
 
 
-def _func_attention_backward(ctx, dwc, dattn):
+def func_attention_backward(ctx, dwc, dattn):
     query, context = ctx.saved_tensors
     gamma1, scaled = ctx.cfg
     need_q, need_c = ctx.needs_input_grad[:2]
     dwc = torch.zeros_like(query) if dwc is None else dwc
-    dq, dc = torch.ops.agb.func_attention_bwd(query, context, gamma1, scaled, dwc.contiguous(),
-                                              None if dattn is None else dattn.contiguous(), need_q, need_c)
+    dq, dc = ctx.bwd(query, context, gamma1, scaled, dwc.contiguous(), None if dattn is None else dattn.contiguous(),
+                     need_q, need_c)
     return (dq if need_q else None), (dc if need_c else None), None, None
 
 
-func_attention_fwd.register_autograd(_func_attention_backward, setup_context=_func_attention_setup)
+_func_attention_fwd.register_autograd(
+    func_attention_backward, setup_context=partial(func_attention_setup, bwd=torch.ops.agb.func_attention_bwd))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -547,14 +595,16 @@ def region_head_workspace_bytes(B: int, Cin: int, Cout: int, R: int) -> int:
     return int(N.lib().agb_region_head_workspace_bytes(B, Cin, Cout, R))
 
 
-@_op("region_head_fwd")
 def region_head_fwd(x: Tensor, weight: Tensor) -> Tuple[Tensor, Tensor]:
     """x [B,Cin,R] fp32 contiguous, weight [Cout,Cin] fp32 -> (feat [B,Cout,R] fp32, ws uint8 holding the 16-bit
     operand copies region_head_bwd reuses)"""
     return ops.region_head_fwd(x, weight, keep_ws=True)
 
 
-@region_head_fwd.register_fake
+_region_head_fwd = _op("region_head_fwd", region_head_fwd)
+
+
+@_region_head_fwd.register_fake
 def _(x, weight):
     B, Cin, R = x.shape
     Cout = weight.shape[0]
@@ -564,7 +614,6 @@ def _(x, weight):
     return x.new_empty((B, Cout, R), dtype=torch.float32), _ws_like(nbytes, x)
 
 
-@_op("region_head_bwd", mutates_args=("ws",))
 def region_head_bwd(x: Tensor, weight: Tensor, dfeat: Tensor, need_dw: bool, need_dx: bool,
                     ws: Optional[Tensor]) -> Tuple[Tensor, Tensor]:
     """(dweight [Cout,Cin] or empty, dx [B,Cin,R] or empty); ws: the workspace region_head_fwd returned, which
@@ -573,27 +622,35 @@ def region_head_bwd(x: Tensor, weight: Tensor, dfeat: Tensor, need_dw: bool, nee
     return _none(dw, x.device), _none(dx, x.device)
 
 
-@region_head_bwd.register_fake
+_region_head_bwd = _op("region_head_bwd", region_head_bwd, mutates_args=("ws",))
+
+
+@_region_head_bwd.register_fake
 def _(x, weight, dfeat, need_dw, need_dx, ws):
     f32 = dict(dtype=torch.float32)
     return (x.new_empty(tuple(weight.shape) if need_dw else (0,), **f32),
             x.new_empty(tuple(x.shape) if need_dx else (0,), **f32))
 
 
-def _region_head_setup(ctx, inputs, output):
+def region_head_setup(ctx, inputs, output, bwd):
+    """region_head_fwd: inputs and output as the op's, bwd the region_head_bwd to call"""
     x, weight = inputs
-    ctx.save_for_backward(x, weight, output[1])
+    ctx.save_for_backward(x, weight)
+    ctx.ws = output[1] if any(ctx.needs_input_grad) else None      # 16-bit copies of x and W, reused by backward
+    ctx.bwd = bwd
     ctx.mark_non_differentiable(output[1])
 
 
-def _region_head_backward(ctx, dfeat, _dws):
-    x, weight, ws = ctx.saved_tensors
+def region_head_backward(ctx, dfeat, _dws):
+    x, weight = ctx.saved_tensors
     need_x, need_w = ctx.needs_input_grad[:2]
-    dw, dx = torch.ops.agb.region_head_bwd(x, weight, dfeat.contiguous(), need_w, need_x, ws)
+    dw, dx = ctx.bwd(x, weight, dfeat.contiguous(), need_w, need_x, ctx.ws)
+    ctx.ws = None                                                   # the backward wrote its staging over it
     return (dx if need_x else None), (dw if need_w else None)
 
 
-region_head_fwd.register_autograd(_region_head_backward, setup_context=_region_head_setup)
+_region_head_fwd.register_autograd(
+    region_head_backward, setup_context=partial(region_head_setup, bwd=torch.ops.agb.region_head_bwd))
 
 OPS = ("word_attn_fwd", "word_attn_cat", "word_attn_bwd", "damsm_fwd", "damsm_bwd", "contrastive", "sent_cos_fwd",
        "sent_cos_bwd", "func_attention_fwd", "func_attention_bwd", "region_head_fwd", "region_head_bwd",

@@ -137,13 +137,28 @@ class _Exchange:
         self.lens, self.cls, self.labels = lens, cls, labels.contiguous()
 
 
+def _words_operands(img, words):
+    """img_features [Bl,D,h,w] or [Bl,D,R], words_emb [Bl,D,T] -> the kernels' fp32 operands img3 [Bl,D,R], w32"""
+    return img.float().reshape(img.shape[0], img.shape[1], -1).contiguous(), words.float()
+
+
+def _words_forward_mode(cfg: DamsmConfig, img3, w32, train: bool, supported):
+    """(math, save) of the DAMSM forward.  cfg.math was resolved from the LOCAL caption padding: if the T the kernels
+    get (agreed by all ranks after the exchange) leaves the tensor-core range, all ranks fall back to the fp32 kernels
+    together.  supported(T, D, R, math): the library's query, None for an injected backend without one."""
+    math = cfg.math
+    if math != native.AGB_MATH_FP32 and supported is not None and \
+            not supported(int(w32.shape[2]), int(img3.shape[1]), int(img3.shape[2]), math):
+        math = native.AGB_MATH_FP32
+    return math, math != native.AGB_MATH_FP32 and train
+
+
 class _WordsLossFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, img, words, cfg: DamsmConfig, ex: _Exchange, cnn, rnn):
         o = cfg.ops
-        Bl, D = img.shape[0], img.shape[1]
-        img3 = img.detach().float().reshape(Bl, D, -1).contiguous()
-        w32 = words.detach().float()
+        Bl = img.shape[0]
+        img3, w32 = _words_operands(img.detach(), words.detach())
         T_local = w32.shape[2]
         if ex.W > 1:
             T_all = _agree_on_words(T_local, cfg, w32.device)
@@ -157,14 +172,9 @@ class _WordsLossFn(torch.autograd.Function):
             rnn32 = rnn.detach().float().reshape(rnn.shape[-2], -1).contiguous()
             if ex.W > 1:
                 rnn32 = _gather_cat(rnn32, cfg.group)
-        # the math mode was resolved from the LOCAL caption padding; after the exchange every rank sees the agreed T:
-        # if that leaves the tensor-core range, all ranks fall back to the fp32 kernels together
-        math = cfg.math
-        if math != native.AGB_MATH_FP32 and hasattr(o, "damsm_supported") and \
-                not o.damsm_supported(int(w32.shape[2]), D, int(img3.shape[2]), math):
-            math = native.AGB_MATH_FP32
+        math, save = _words_forward_mode(cfg, img3, w32, any(ctx.needs_input_grad[:2]),
+                                         getattr(o, "damsm_supported", None))
         ctx.math = math
-        save = math != native.AGB_MATH_FP32 and any(ctx.needs_input_grad[:2])       # training forward
         m, att, scos, ws = o.damsm_fwd(img3, w32, ex.lens, cfg.gamma1, cfg.gamma2, cfg.eps, ex.row0, cfg.want_att,
                                        math, cnn32 if fuse_sent else None, rnn32 if fuse_sent else None, True,
                                        save)
@@ -244,7 +254,10 @@ class _SentLossFn(torch.autograd.Function):
 
 
 # ------------------------------------------------------------------------------------------------
-# the same losses while torch.compile traces: the agb:: ops (agb_native/torch_ops.py), single process only
+# the same losses while torch.compile traces: the agb:: ops (agb_native/torch_ops.py), single process only.
+# These stay apart from _WordsLossFn / _SentLossFn on purpose: eagerly, the contrastive backward is fused into the
+# DAMSM and cosine backwards through gscale (one launch less in a launch-bound step), and the Functions carry the
+# sharded exchange; the ops keep the contrastive loss as a differentiable op of its own.
 # ------------------------------------------------------------------------------------------------
 def _op_path(*cfgs: DamsmConfig) -> bool:
     """trace the agb:: ops: compiling, the native kernels (not an injected backend) and no process group (the
@@ -254,18 +267,17 @@ def _op_path(*cfgs: DamsmConfig) -> bool:
 
 def _words_loss_op(img, words, cfg: DamsmConfig, ex: _Exchange):
     """_WordsLossFn of a single process as agb:: ops: (loss, packed att [Bl,T,R] or empty)"""
-    Bl, D = img.shape[0], img.shape[1]
-    img3 = img.float().reshape(Bl, D, -1).contiguous()
-    w32 = words.float()
-    math = cfg.math
-    if math != native.AGB_MATH_FP32 and \
-            not torch_ops.host_query("agb_damsm_supported", int(w32.shape[2]), D, int(img3.shape[2]), math):
-        math = native.AGB_MATH_FP32
-    save = math != native.AGB_MATH_FP32 and torch.is_grad_enabled() and (img.requires_grad or words.requires_grad)
+    img3, w32 = _words_operands(img, words)
+    train = torch.is_grad_enabled() and (img.requires_grad or words.requires_grad)
+    math, save = _words_forward_mode(cfg, img3, w32, train, _traced_damsm_supported)
     m, att, _, _ = torch.ops.agb.damsm_fwd(img3, w32, ex.lens, None, None, cfg.gamma1, cfg.gamma2, cfg.eps, 0,
                                            cfg.want_att, math, save)
-    loss, _ = torch.ops.agb.contrastive(m, ex.cls, ex.labels, cfg.gamma3, cfg.lam, 0, Bl, True)
+    loss, _ = torch.ops.agb.contrastive(m, ex.cls, ex.labels, cfg.gamma3, cfg.lam, 0, img.shape[0], True)
     return loss.reshape(()), att
+
+
+def _traced_damsm_supported(*args) -> bool:
+    return bool(torch_ops.host_query("agb_damsm_supported", *args))
 
 
 def _sentence_loss_op(cnn, rnn, cfg: DamsmConfig, ex: _Exchange):

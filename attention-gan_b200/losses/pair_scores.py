@@ -11,7 +11,8 @@ N x Nc similarity matrix:
 
 Forward: agb_damsm_pairs_train_fwd / agb_sent_cos_pairs_fwd; backward: agb_damsm_pairs_bwd / agb_sent_cos_pairs_bwd
 (INTEGRATION.md §8).  Under ``torch.compile`` they go through the ``agb::damsm_pairs_train_fwd`` and
-``agb::sent_cos_pairs_train_fwd`` custom ops, whose registered backward calls the same kernels.
+``agb::sent_cos_pairs_train_fwd`` custom ops; eager calls run the same op bodies and gradient formulas
+(agb_native/torch_ops.py) as the autograd Functions below, without the dispatcher.
 """
 from __future__ import annotations
 
@@ -23,49 +24,31 @@ from .damsm_core import as_device_i32, chunk_pairs, pair_index
 _PAIR_MATH = ("f16", "bf16", "f16x2")
 
 
+# The shared setup runs inside forward rather than as a separate setup_context: with one, every apply binds its
+# arguments through inspect.signature, tens of microseconds per call.
 class _WordsPairs(torch.autograd.Function):
-    """one chunk of pairs: m [P]; the training workspace is kept for the backward"""
+    """agb::damsm_pairs_train_fwd of one chunk of pairs: (m [P], ws); the training workspace is kept for the
+    backward"""
 
     @staticmethod
-    def forward(ctx, img, words, lens, pi, pc, gamma1, gamma2, math):
-        m, ws = ops.damsm_pairs_train_fwd(img, words, lens, pi, pc, gamma1, gamma2, math)
-        ctx.save_for_backward(img, words, lens, pi, pc)
-        ctx.ws = ws
-        ctx.cfg = (gamma1, gamma2, math)
-        return m
+    def forward(ctx, *inputs):
+        out = torch_ops.damsm_pairs_train_fwd(*inputs)
+        torch_ops.damsm_pairs_setup(ctx, inputs, out, bwd=torch_ops.damsm_pairs_bwd)
+        return out
 
-    @staticmethod
-    def backward(ctx, dm):
-        img, words, lens, pi, pc = ctx.saved_tensors
-        need_img, need_words = ctx.needs_input_grad[:2]
-        dimg = dwords = None
-        if need_img or need_words:
-            if ctx.ws is None:
-                raise RuntimeError(_TWICE)
-            dimg, dw = ops.damsm_pairs_bwd(img, words, lens, pi, pc, *ctx.cfg, dm.float().contiguous(), ctx.ws,
-                                           need_dwords=need_words, need_dimg=need_img)
-            dwords = dw.transpose(1, 2) if need_words else None           # [Nc,D,T] view like words
-        ctx.ws = None                             # the saved vectors are not needed again: free them now
-        return dimg, dwords, None, None, None, None, None, None
+    backward = staticmethod(torch_ops.damsm_pairs_backward)
 
 
 class _SentencePairs(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, cnn, rnn, pi, pc, eps):
-        ctx.save_for_backward(cnn, rnn, pi, pc)
-        ctx.eps = eps
-        return ops.sent_cos_pairs_fwd(cnn, rnn, pi, pc, eps)
+    """agb::sent_cos_pairs_train_fwd"""
 
     @staticmethod
-    def backward(ctx, dcos):
-        cnn, rnn, pi, pc = ctx.saved_tensors
-        need_c, need_r = ctx.needs_input_grad[:2]
-        dc, dr = ops.sent_cos_pairs_bwd(cnn, rnn, pi, pc, ctx.eps, dcos.float().contiguous(), need_c, need_r)
-        return dc, dr, None, None, None
+    def forward(ctx, *inputs):
+        out = torch_ops.sent_cos_pairs_train_fwd(*inputs)
+        torch_ops.sent_cos_pairs_setup(ctx, inputs, out, bwd=torch_ops.sent_cos_pairs_bwd)
+        return out
 
-
-_TWICE = ("words_pair_scores: a second backward through the same scores is not supported (the first one released "
-          "the training workspace); compute the scores again")
+    backward = staticmethod(torch_ops.sent_cos_pairs_backward)
 
 
 def _traced_train_workspace_bytes(*args) -> int:
@@ -110,13 +93,12 @@ def words_pair_scores(img_features: torch.Tensor, words_emb: torch.Tensor, cap_l
         ws_bytes = _traced_score_workspace_bytes if compiling else ops.damsm_pairs_workspace_bytes
     per = chunk_pairs(N, Nc, max(P, 1), T, D, R, mt, ws_bytes, int(workspace_bytes))
     score_ws = None if train or compiling else ops._ws(ws_bytes(N, Nc, per, T, D, R, mt), img.device)
+    train_fwd = torch.ops.agb.damsm_pairs_train_fwd if compiling else _WordsPairs.apply     # both give (m, ws)
     parts = []
     for s in range(0, max(P, 1), per):
         a, b = pi[s:s + per], pc[s:s + per]
-        if train and compiling:
-            parts.append(torch.ops.agb.damsm_pairs_train_fwd(img, words, lens, a, b, g1, g2, mt)[0])
-        elif train:
-            parts.append(_WordsPairs.apply(img, words, lens, a, b, g1, g2, mt))
+        if train:
+            parts.append(train_fwd(img, words, lens, a, b, g1, g2, mt)[0])
         elif compiling:
             parts.append(torch.ops.agb.damsm_pairs_fwd(img, words, lens, a, b, g1, g2, False, mt)[0])
         else:
@@ -132,6 +114,5 @@ def sentence_pair_scores(cnn_code: torch.Tensor, sent_emb: torch.Tensor, image_i
     cnn = cnn_code.float().contiguous()
     rnn = sent_emb.float().contiguous()
     pi, pc = pair_index(image_idx, caption_idx, cnn.device)
-    if torch.compiler.is_compiling():
-        return torch.ops.agb.sent_cos_pairs_train_fwd(cnn, rnn, pi, pc, float(eps))
-    return _SentencePairs.apply(cnn, rnn, pi, pc, float(eps))
+    fwd = torch.ops.agb.sent_cos_pairs_train_fwd if torch.compiler.is_compiling() else _SentencePairs.apply
+    return fwd(cnn, rnn, pi, pc, float(eps))

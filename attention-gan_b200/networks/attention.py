@@ -18,44 +18,41 @@ import torch
 from torch import nn
 
 from ..agb_native import ops
-from ..agb_native import torch_ops  # noqa: F401  (registers torch.ops.agb, used while compiling)
+from ..agb_native import torch_ops
 
 GlobalAttention = None  # set below (BASELINE.json's name for AttentionModule)
 
 
+def _word_attn_operands(images, words, weight, mask):
+    """the operands of agb::word_attn_fwd / word_attn_cat after images: words and weight [C,E] in fp32, mask int64"""
+    wt32 = weight.reshape(weight.shape[0], -1).float().contiguous()
+    return words.float(), wt32, mask.to(device=images.device, dtype=torch.int64).contiguous()
+
+
+def _word_attn_grads(ctx, grads):
+    """the gradients of torch_ops.word_attn_backward / word_attn_cat_backward in the dtypes and shapes of words and
+    conv1.weight"""
+    di, dw, dwt = grads[:3]
+    words_dtype, weight_dtype, weight_shape = ctx.meta
+    return (di, None if dw is None else dw.to(words_dtype),
+            None if dwt is None else dwt.reshape(weight_shape).to(weight_dtype), None, None, None)
+
+
 class _WordAttention(torch.autograd.Function):
-    """fused  W.e projection -> scores -> mask -> softmax over words -> context   (fwd + bwd)"""
+    """fused  W.e projection -> scores -> mask -> softmax over words -> context   (fwd + bwd): agb::word_attn_fwd
+    without the dispatcher, with the casts of words and conv1.weight inside the one autograd node"""
 
     @staticmethod
-    def forward(ctx, images, words, weight, mask, scaled):
-        w32 = words if words.dtype == torch.float32 else words.float()
-        wt = weight.reshape(weight.shape[0], -1)
-        wt32 = (wt if wt.dtype == torch.float32 else wt.float()).contiguous()
-        m64 = mask if mask.dtype == torch.int64 else mask.to(torch.int64)
-        m64 = m64.to(images.device).contiguous()
-        out, attn, we = ops.word_attn_fwd(images.detach(), w32.detach(), wt32.detach(), m64, scaled, True)
-        ctx.save_for_backward(images, w32, wt32, m64, we)
-        ctx.scaled = scaled
-        ctx.words_dtype = words.dtype
-        ctx.weight_dtype = weight.dtype
-        ctx.weight_shape = weight.shape
-        ctx.set_materialize_grads(False)
-        return out, attn
+    def forward(ctx, images, words, weight, mask, scaled, want_attn):
+        inputs = (images, *_word_attn_operands(images, words, weight, mask), scaled, want_attn)
+        out = torch_ops.word_attn_fwd(*inputs)
+        torch_ops.word_attn_setup(ctx, inputs, out, bwd=torch_ops.word_attn_bwd)
+        ctx.meta = (words.dtype, weight.dtype, weight.shape)
+        return out[0], out[1]
 
     @staticmethod
     def backward(ctx, dctx, dattn):
-        images, w32, wt32, m64, we = ctx.saved_tensors
-        if dctx is None:
-            dctx = torch.zeros_like(images)
-        need_img, need_words, need_w = ctx.needs_input_grad[0], ctx.needs_input_grad[1], ctx.needs_input_grad[2]
-        dimages, dwords, dweight = ops.word_attn_bwd(images, w32, wt32, m64, we, dctx.to(images.dtype),
-                                                     None if dattn is None else dattn.to(images.dtype),
-                                                     ctx.scaled, need_words, need_w)
-        if dwords is not None:
-            dwords = dwords.to(ctx.words_dtype)
-        if dweight is not None:
-            dweight = dweight.reshape(ctx.weight_shape).to(ctx.weight_dtype)
-        return (dimages if need_img else None), dwords, dweight, None, None
+        return _word_attn_grads(ctx, torch_ops.word_attn_backward(ctx, dctx, dattn, None))
 
 
 def _check_cat_out(images, out):
@@ -76,57 +73,18 @@ class _WordAttentionInto(torch.autograd.Function):
     instead of re-reading and re-writing both"""
 
     @staticmethod
-    def forward(ctx, images, words, weight, mask, scaled, out, want_attn):
-        B, C, H, W = images.shape
+    def forward(ctx, images, words, weight, mask, scaled, want_attn, out):
         _check_cat_out(images, out)
-        w32 = words if words.dtype == torch.float32 else words.float()
-        wt = weight.reshape(weight.shape[0], -1)
-        wt32 = (wt if wt.dtype == torch.float32 else wt.float()).contiguous()
-        m64 = (mask if mask.dtype == torch.int64 else mask.to(torch.int64)).to(images.device).contiguous()
-        out[:, :C].copy_(images.detach())
-        _, attn, we = ops.word_attn_fwd(images.detach(), w32.detach(), wt32.detach(), m64, scaled, want_attn,
-                                        ctx_out=out[:, C:])
+        inputs = (images, *_word_attn_operands(images, words, weight, mask), scaled, want_attn)
+        res = torch_ops.word_attn_into(out, *inputs)
         ctx.mark_dirty(out)
-        ctx.save_for_backward(images, w32, wt32, m64, we)
-        ctx.scaled = scaled
-        ctx.meta = (words.dtype, weight.dtype, weight.shape, C)
-        ctx.set_materialize_grads(False)
-        if attn is None:
-            attn = torch.empty(0, device=images.device, dtype=images.dtype)
-            ctx.mark_non_differentiable(attn)
-        return out, attn
+        torch_ops.word_attn_setup(ctx, inputs, res, bwd=torch_ops.word_attn_bwd)
+        ctx.meta = (words.dtype, weight.dtype, weight.shape)
+        return res[0], res[1]
 
     @staticmethod
     def backward(ctx, dout, dattn):
-        images, w32, wt32, m64, we = ctx.saved_tensors
-        wdt, wtdt, wshape, C = ctx.meta
-        need_img, need_words, need_w = ctx.needs_input_grad[0], ctx.needs_input_grad[1], ctx.needs_input_grad[2]
-        if dout is None:
-            return None, None, None, None, None, None, None
-        dout = dout.to(images.dtype)
-        fmt = ops.attn_memory_format(images)
-        if not dout.is_contiguous(memory_format=fmt):
-            dout = dout.contiguous(memory_format=fmt)
-        # d context is the second channel half of d out, read in place through its batch (and pixel) stride
-        dimages, dwords, dweight = ops.word_attn_bwd(images, w32, wt32, m64, we, dout[:, C:],
-                                                     None if dattn is None else dattn.to(images.dtype),
-                                                     ctx.scaled, need_words, need_w)
-        if need_img:
-            dimages += dout[:, :C]                       # the identity half of the concatenation
-        if dwords is not None:
-            dwords = dwords.to(wdt)
-        if dweight is not None:
-            dweight = dweight.reshape(wshape).to(wtdt)
-        return (dimages if need_img else None), dwords, dweight, None, None, None, None
-
-
-def _word_attn_operands(images, words, weight, mask):
-    """the operands the kernels take, built like _WordAttention.forward does (traced by torch.compile)"""
-    w32 = words if words.dtype == torch.float32 else words.float()
-    wt = weight.reshape(weight.shape[0], -1)
-    wt32 = (wt if wt.dtype == torch.float32 else wt.float()).contiguous()
-    m64 = (mask if mask.dtype == torch.int64 else mask.to(torch.int64)).to(images.device).contiguous()
-    return w32, wt32, m64
+        return _word_attn_grads(ctx, torch_ops.word_attn_cat_backward(ctx, dout, dattn, None)) + (None,)
 
 
 class AttentionModule(nn.Module):
@@ -154,7 +112,7 @@ class AttentionModule(nn.Module):
             w32, wt32, m64 = _word_attn_operands(images, words, self.conv1.weight, self.mask)
             ctx, attn, _ = torch.ops.agb.word_attn_fwd(images, w32, wt32, m64, bool(scaled), True)
             return ctx, attn
-        return _WordAttention.apply(images, words, self.conv1.weight, self.mask, bool(scaled))
+        return _WordAttention.apply(images, words, self.conv1.weight, self.mask, bool(scaled), True)
 
     def forward_into(self, images, words, out, scaled=True, want_attn=True):
         """images [B, C, H, W], words [B, E, T], out [B, 2C, H, W] (pre-allocated, in the memory format of images:
@@ -169,8 +127,8 @@ class AttentionModule(nn.Module):
             _check_cat_out(images, out)
             res, attn = self.forward_cat(images, words, scaled, want_attn)
             return out.copy_(res), attn
-        res, attn = _WordAttentionInto.apply(images, words, self.conv1.weight, self.mask, bool(scaled), out,
-                                             bool(want_attn))
+        res, attn = _WordAttentionInto.apply(images, words, self.conv1.weight, self.mask, bool(scaled),
+                                             bool(want_attn), out)
         return res, (attn if want_attn else None)
 
     def forward_cat(self, images, words, scaled=True, want_attn=True):
@@ -193,35 +151,28 @@ class AttentionModule(nn.Module):
 GlobalAttention = AttentionModule
 
 
+def _func_attention_operands(query, context):
+    """query [B,D,L] and context [B,D,ih,iw] -> the operands of agb::func_attention_fwd: fp32, context [B,D,R]"""
+    return query.float(), context.float().reshape(context.shape[0], context.shape[1], -1).contiguous()
+
+
 class _FuncAttention(torch.autograd.Function):
+    """agb::func_attention_fwd without the dispatcher, with the casts and reshapes inside the one autograd node"""
+
     @staticmethod
     def forward(ctx, query, context, gamma1, scaled):
-        B, D, L = query.shape
-        ih, iw = context.shape[2], context.shape[3]
-        q32 = query if query.dtype == torch.float32 else query.float()
-        c32 = (context if context.dtype == torch.float32 else context.float()).reshape(B, D, ih * iw).contiguous()
-        wc, attn = ops.func_attention_fwd(q32.detach(), c32.detach(), gamma1, scaled)
-        ctx.save_for_backward(q32, c32)
-        ctx.cfg = (gamma1, scaled, query.dtype, context.dtype, context.shape)
-        ctx.set_materialize_grads(False)
-        return wc.to(query.dtype), attn.reshape(B, L, ih, iw).to(query.dtype)
+        inputs = (*_func_attention_operands(query, context), gamma1, scaled)
+        wc, attn = torch_ops.func_attention_fwd(*inputs)
+        torch_ops.func_attention_setup(ctx, inputs, (wc, attn), bwd=torch_ops.func_attention_bwd)
+        ctx.meta = (query.dtype, context.dtype, context.shape)
+        return wc.to(query.dtype), attn.reshape(*attn.shape[:2], *context.shape[2:]).to(query.dtype)
 
     @staticmethod
     def backward(ctx, dwc, dattn):
-        q32, c32 = ctx.saved_tensors
-        gamma1, scaled, qdt, cdt, cshape = ctx.cfg
-        if dwc is None:
-            dwc = torch.zeros_like(q32)
-        dwc = dwc.float().contiguous()
-        if dattn is not None:
-            dattn = dattn.float().reshape(q32.shape[0], q32.shape[2], -1).contiguous()
-        dq, dc = ops.func_attention_bwd(q32, c32, gamma1, scaled, dwc, dattn,
-                                        ctx.needs_input_grad[0], ctx.needs_input_grad[1])
-        if dq is not None:
-            dq = dq.to(qdt)
-        if dc is not None:
-            dc = dc.reshape(cshape).to(cdt)
-        return dq, dc, None, None
+        qdt, cdt, cshape = ctx.meta
+        dq, dc, _, _ = torch_ops.func_attention_backward(ctx, None if dwc is None else dwc.float(),
+                                                         None if dattn is None else dattn.float().flatten(2))
+        return (None if dq is None else dq.to(qdt)), (None if dc is None else dc.reshape(cshape).to(cdt)), None, None
 
 
 def func_attention(query, context, gamma1=4.0, scaled=True):
@@ -229,10 +180,7 @@ def func_attention(query, context, gamma1=4.0, scaled=True):
     (weightedContext [B, D, L], attn [B, L, ih, iw])        reference networks/attention.py:82-121"""
     ops.require_cuda(query, context)
     if torch.compiler.is_compiling():
-        B, D, L = query.shape
-        ih, iw = context.shape[2], context.shape[3]
-        q32 = query if query.dtype == torch.float32 else query.float()
-        c32 = (context if context.dtype == torch.float32 else context.float()).reshape(B, D, ih * iw).contiguous()
-        wc, attn = torch.ops.agb.func_attention_fwd(q32, c32, float(gamma1), bool(scaled))
-        return wc.to(query.dtype), attn.reshape(B, L, ih, iw).to(query.dtype)
+        wc, attn = torch.ops.agb.func_attention_fwd(*_func_attention_operands(query, context), float(gamma1),
+                                                    bool(scaled))
+        return wc.to(query.dtype), attn.reshape(*attn.shape[:2], *context.shape[2:]).to(query.dtype)
     return _FuncAttention.apply(query, context, float(gamma1), bool(scaled))

@@ -13,46 +13,41 @@ import torch
 from torch import nn
 
 from ..agb_native import ops
-from ..agb_native import torch_ops  # noqa: F401  (registers torch.ops.agb, used while compiling)
+from ..agb_native import torch_ops
+
+
+def _region_head_operands(x, weight):
+    """x [B,Cin,H,W], weight [Cout,Cin,1,1] -> the operands of agb::region_head_fwd: x [B,Cin,H*W] and weight
+    [Cout,Cin], fp32 contiguous"""
+    B, Cin = x.shape[:2]
+    return x.float().reshape(B, Cin, -1).contiguous(), weight.reshape(weight.shape[0], Cin).float().contiguous()
 
 
 class _RegionHead(torch.autograd.Function):
+    """agb::region_head_fwd without the dispatcher, with the casts and reshapes inside the one autograd node"""
+
     @staticmethod
     def forward(ctx, x, weight):
-        B, Cin, H, W = x.shape
-        x3 = (x if x.dtype == torch.float32 else x.float()).reshape(B, Cin, H * W).contiguous()
-        w2 = weight.reshape(weight.shape[0], Cin)
-        w2 = (w2 if w2.dtype == torch.float32 else w2.float()).contiguous()
-        feat, ws = ops.region_head_fwd(x3.detach(), w2.detach(), keep_ws=True)
-        ctx.save_for_backward(x3, w2)
-        ctx.ws = ws if any(ctx.needs_input_grad) else None        # bf16 copies of x and W, reused by backward
+        inputs = _region_head_operands(x, weight)
+        feat, ws = torch_ops.region_head_fwd(*inputs)
+        torch_ops.region_head_setup(ctx, inputs, (feat, ws), bwd=torch_ops.region_head_bwd)
         ctx.meta = (x.shape, x.dtype, weight.shape, weight.dtype)
-        return feat.reshape(B, weight.shape[0], H, W).to(x.dtype)
+        return feat.reshape(*feat.shape[:2], *x.shape[2:]).to(x.dtype)
 
     @staticmethod
     def backward(ctx, dfeat):
-        x3, w2 = ctx.saved_tensors
         xshape, xdt, wshape, wdt = ctx.meta
-        d3 = dfeat.float().reshape(x3.shape[0], w2.shape[0], -1).contiguous()
-        dw, dx = ops.region_head_bwd(x3, w2, d3, ctx.needs_input_grad[1], ctx.needs_input_grad[0], ctx.ws)
-        ctx.ws = None
-        if dw is not None:
-            dw = dw.reshape(wshape).to(wdt)
-        if dx is not None:
-            dx = dx.reshape(xshape).to(xdt)
-        return dx, dw
+        dx, dw = torch_ops.region_head_backward(ctx, dfeat.float().flatten(2), None)
+        return ((None if dx is None else dx.reshape(xshape).to(xdt)),
+                (None if dw is None else dw.reshape(wshape).to(wdt)))
 
 
 def region_head(x: torch.Tensor, weight: torch.Tensor) -> torch.Tensor:
     """x [B, Cin, H, W], weight [Cout, Cin, 1, 1] -> [B, Cout, H, W]: _RegionHead, or agb::region_head_fwd while
     torch.compile traces (same kernels, same operands)"""
     if torch.compiler.is_compiling():
-        B, Cin, H, W = x.shape
-        x3 = (x if x.dtype == torch.float32 else x.float()).reshape(B, Cin, H * W).contiguous()
-        w2 = weight.reshape(weight.shape[0], Cin)
-        w2 = (w2 if w2.dtype == torch.float32 else w2.float()).contiguous()
-        feat, _ = torch.ops.agb.region_head_fwd(x3, w2)
-        return feat.reshape(B, weight.shape[0], H, W).to(x.dtype)
+        feat, _ = torch.ops.agb.region_head_fwd(*_region_head_operands(x, weight))
+        return feat.reshape(*feat.shape[:2], *x.shape[2:]).to(x.dtype)
     return _RegionHead.apply(x, weight)
 
 
